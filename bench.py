@@ -35,8 +35,10 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: no __pycache__ is left in it
 
 N_TRAIN, TRIALS, SYSTEM = 2000, 100, "CP"
+DUMP_BYTES = 64_000_000  # cap of --dump-outputs; above it a seeded sample of the GPs is written
 METRIC = "batched fp64 logML+gradient evals/sec (n=2000)"
 WORKLOAD_NAMES = {"P1": "P1 simple pendulum", "P2": "P2 double pendulum", "CP": "CP cartpole noise experiment", "FB": "FB fourbar"}
 
@@ -166,6 +168,21 @@ def julia_probe():
         return "present (version probe failed)"
 
 
+def dump_outputs(out_dir, arrays):
+    """Write {name: array with one row per GP} as out_dir/<name>.npy in float64.  Above DUMP_BYTES in all, the same
+    seeded sample of GP rows is taken from every array, and gp_index.npy records which GPs they are."""
+    B = len(next(iter(arrays.values())))
+    row_bytes = sum(8 * int(np.prod(a.shape[1:], dtype=np.int64)) for a in arrays.values())
+    keep = max(1, (DUMP_BYTES - 4096 * (len(arrays) + 1)) // (row_bytes + 8))
+    if B > keep:
+        idx = np.sort(np.random.default_rng(0).choice(B, size=keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["gp_index"] = idx
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -213,7 +230,14 @@ def main():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak (default, what the driver runs): every rank owns --trials trials; strong: the SAME --trials "
                          "trials (north_star: '100 trial datasets batched across 8xB200') are split round-robin over the ranks")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned for rank 0's GPs (mll, grad, info) and "
+                         "the last timed mean+variance prediction (predict_mu, predict_var) as DIR/<name>.npy, float64, one row per GP")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -314,6 +338,7 @@ def main():
     ms_total = float(ms.item())
     sampler.stop_flag = True
     info_host = info_dev.cpu().numpy()
+    outputs = {"mll": mll_dev.cpu().numpy(), "grad": grad_dev.cpu().numpy(), "info": info_host} if args.dump_outputs else None
     info_hist = {str(int(k)): int(c) for k, c in zip(*np.unique(info_host, return_counts=True))}  # rank 0, last timed step
     value = B_total * args.steps / (ms_total * 1e-3)
 
@@ -390,9 +415,11 @@ def main():
             barrier()
             tdev, t0 = 0.0, time.perf_counter()
             for _ in range(reps):
-                batch.predict_y(Xt, var=want_var)
+                mu_var = batch.predict_y(Xt, var=want_var)
                 tdev += batch.last_predict_ms(0)
             twall = time.perf_counter() - t0
+            if want_var and outputs is not None:
+                outputs["predict_mu"], outputs["predict_var"] = mu_var
             tt = torch.tensor([tdev * 1e-3, twall], dtype=torch.float64, device=dev)
             if world > 1:
                 dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -475,6 +502,8 @@ def main():
         line["cpu_baseline"] = cpu
     if pred:
         line["predict"] = pred
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -1,6 +1,6 @@
 import os, sys, time, json
 import numpy as np
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import gpr_jl_b200 as G
 from gpr_jl_b200 import data
 trials = data.make_config("CP", trials=25, n=2000)
