@@ -87,6 +87,14 @@ static void free_batch(gprb_batch* b) {
     if (sl.t0) cudaEventDestroy(sl.t0);
     if (sl.t1) cudaEventDestroy(sl.t1);
   }
+  {
+    gprb_postcov_ws& w = b->pc;
+    cudaFree(w.T); cudaFree(w.S); cudaFree(w.L); cudaFree(w.Dinv); cudaFree(w.DinvT); cudaFree(w.logdet); cudaFree(w.Z);
+    cudaFree(w.O); cudaFree(w.bad); cudaFree(w.fail); cudaFree(w.list);
+    if (w.fail_host) cudaFreeHost(w.fail_host);
+    if (w.list_host) cudaFreeHost(w.list_host);
+    if (w.z_ready) cudaEventDestroy(w.z_ready);
+  }
   if (b->list_host) cudaFreeHost(b->list_host);
   if (b->fail_host) cudaFreeHost(b->fail_host);
   if (b->stage_host) cudaFreeHost(b->stage_host);
@@ -470,7 +478,7 @@ using namespace gprb;
 
 extern "C" {
 
-int gprb_version(void) { return 200; }
+int gprb_version(void) { return 300; }
 const char* gprb_last_error(void) { return g_err.c_str(); }
 
 int gprb_init(gprb_ctx** out, int device) {
@@ -493,7 +501,7 @@ int gprb_init(gprb_ctx** out, int device) {
   // dynamic shared-memory opt-ins are per-device function attributes: set them for THIS device (a second context on
   // another GPU of the same process gets its own)
   int rc;
-  if ((rc = configure_tile_gemm()) || (rc = configure_diag_factor())) return rc;
+  if ((rc = configure_tile_gemm()) || (rc = configure_diag_factor()) || (rc = configure_post_cov())) return rc;
   gprb_ctx* c = new (std::nothrow) gprb_ctx();
   GPRB_REQUIRE(c != nullptr, "gprb_init: out of host memory");
   c->device = device;
@@ -1160,6 +1168,261 @@ int gprb_get_Kinv(gprb_batch* b, int32_t gp, double* out) {
       out[r + c * n] = out[c + r * n] = v;
     }
   return GPRB_OK;
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------------
+// Full posterior covariance and posterior draws (gprb_predict_cov, gprb_sample_posterior) on prediction slot 0.
+// The right-hand sides T = L^-1 K* of every 128-column chunk are kept (one [B][npad][PT] block per chunk behind one tensor
+// map), computed by the launches gprb_predict uses (k_predict_cross, GEMM_FWD_ROW chains on the four stream groups,
+// k_predict_finish for mu) - always the tiled path, the GEMV path never materialises T.  The covariance tiles of a stream
+// group follow its last FWD_ROW chain on the group's stream.  Leaves Sigma in pc.S and mu in the slot's pmu; t0 recorded.
+static int postcov_enqueue(gprb_batch* b, int64_t m, const double* Xstar, int64_t xstar_stride, const double* mstar, bool add_noise) {
+  gprb_predict_slot& sl = b->ps[0];
+  gprb_postcov_ws& w = b->pc;
+  const int B = b->B, J = b->J, count = B, gp0 = 0;
+  cudaStream_t* str = b->stream;
+  cudaStream_t st = str[0];
+  const int64_t npad = b->npad, mpad = (m + NB - 1) / NB * NB;
+  const int nchunk = (int)(mpad / NB);
+  const size_t nx = (size_t)(xstar_stride ? xstar_stride * (B - 1) + m * b->d : m * b->d);
+  const size_t nout = (size_t)count * m;
+  int rc;
+  if (!sl.t0) {
+    GPRB_CUDA(cudaEventCreate(&sl.t0));
+    GPRB_CUDA(cudaEventCreate(&sl.t1));
+    GPRB_CUDA(cudaMallocHost((void**)&sl.h_mask, sizeof(int32_t) * B));
+    if ((rc = dev_alloc(&sl.mask, (size_t)B))) return rc;
+  }
+  if ((rc = ensure_dev(&sl.pX, &sl.pX_cap, nx)) || (rc = ensure_dev(&sl.pmu, &sl.pmu_cap, nout)) ||
+      (rc = ensure_dev(&sl.pmupart, &sl.pmupart_cap, (size_t)count * J * PT)) ||
+      (rc = ensure_pinned(&sl.h_in, &sl.h_in_cap, nx + (mstar ? nout : 0))) || (rc = ensure_pinned(&sl.h_out, &sl.h_out_cap, nout)) ||
+      (rc = ensure_dev(&w.T, &w.T_cap, (size_t)nchunk * count * npad * PT)) ||
+      (rc = ensure_dev(&w.S, &w.S_cap, (size_t)count * mpad * mpad)) || (rc = ensure_dev(&w.bad, &w.bad_cap, (size_t)count)))
+    return rc;
+  if (mstar && (rc = ensure_dev(&sl.pms, &sl.pms_cap, nout))) return rc;
+  // T of chunk c, GP g is block c * count + g of the map (GEMM_FWD_ROW reads it through t_gp_off = gp0 - c * count)
+  if ((rc = make_tensor_map(&w.tm_T68, w.T, PT, (uint64_t)npad, (uint64_t)nchunk * count, PT, (uint64_t)npad * PT, NB / 2 + 4, KT)))
+    return rc;
+  for (int i = 0; i < B; ++i) sl.h_mask[i] = b->state_ok[i] ? 0 : 1;
+  memcpy(sl.h_in, Xstar, sizeof(double) * nx);
+  if (mstar) memcpy(sl.h_in + nx, mstar, sizeof(double) * nout);
+  GPRB_CUDA(cudaEventRecord(sl.t0, st));
+  GPRB_CUDA(cudaMemcpyAsync(sl.mask, sl.h_mask, sizeof(int32_t) * B, cudaMemcpyHostToDevice, st));
+  GPRB_CUDA(cudaMemcpyAsync(sl.pX, sl.h_in, sizeof(double) * nx, cudaMemcpyHostToDevice, st));
+  if (mstar) GPRB_CUDA(cudaMemcpyAsync(sl.pms, sl.h_in + nx, sizeof(double) * nout, cudaMemcpyHostToDevice, st));
+  GPRB_CUDA(cudaMemsetAsync(w.bad, 0, sizeof(int32_t) * count, st));
+
+  const int nv = (int)((b->n + KT - 1) / KT * KT);
+  PostCovArgs pa{sl.pX, b->theta, sl.mask, w.S, w.bad, xstar_stride, nv, b->d, (int)m, (int)mpad, b->kind, gp0, count, 0,
+                 add_noise ? 1 : 0, w.tm_T68};
+  const int ns = std::min(4, b->nstreams);
+  const int S = (count >= 8 * ns) ? ns : 1;
+  for (int c = 0; c < nchunk; ++c) {
+    const int64_t s0 = (int64_t)c * PT;
+    PredictTileArgs ta{b->Xtptr, b->theta, b->alpha, sl.pX, mstar ? sl.pms : nullptr, w.T + (size_t)c * count * npad * PT,
+                       sl.pmupart, sl.pmu, nullptr, xstar_stride, (int)b->n, (int)b->npad, b->d, J, (int)m, b->kind,
+                       (int)s0, (int)std::min<int64_t>(PT, m - s0)};
+    ta.gp_off = gp0;
+    ta.mask = sl.mask;
+    if ((rc = launch_predict_cross(ta, count, st))) return rc;
+    b->ctx->launches++;
+    GemmArgs ga{b->Lm, b->DinvT, b->Dinv, nullptr, b->Lm, b->KinvD, nullptr, b->npad * b->npad, (int64_t)J * NB * NB,
+                (int)b->npad, J, 0, GEMM_FWD_ROW, nv};
+    ga.Tm = w.T; ga.t_stride = npad * PT; ga.ldt = PT; ga.t_gp_off = gp0 - c * count;
+    set_gemm_maps(ga, b);
+    ga.tm_T68 = w.tm_T68;
+    ga.ncols = ta.mc;
+    ga.fail = sl.mask;
+    ga.colw = (int64_t)count * ((ta.mc + 63) / 64) >= b->ctx->sm_count ? 64 : 32;
+    const int ntl = (ta.mc + ga.colw - 1) / ga.colw;
+    if (S > 1) GPRB_CUDA(cudaEventRecord(b->join[0], st));
+    for (int s = 0; s < S; ++s) {
+      const int g0 = (int)((int64_t)count * s / S), g1 = (int)((int64_t)count * (s + 1) / S);
+      cudaStream_t ss = str[s];
+      if (s > 0) GPRB_CUDA(cudaStreamWaitEvent(ss, b->join[0], 0));
+      ga.gp_off = gp0 + g0;
+      for (int i = 0; i < J; ++i) {
+        ga.step = i;
+        if ((rc = launch_tile_gemm(ga, ntl, g1 - g0, ss))) return rc;
+        b->ctx->launches++;
+      }
+      if (c == nchunk - 1) {  // every chunk of this group's GPs is solved: its covariance tiles
+        pa.g0 = g0;
+        if ((rc = launch_post_cov(pa, g1 - g0, ss))) return rc;
+        b->ctx->launches++;
+      }
+      if (s > 0) {
+        GPRB_CUDA(cudaEventRecord(b->join[s], ss));
+        GPRB_CUDA(cudaStreamWaitEvent(st, b->join[s], 0));
+      }
+    }
+    if ((rc = launch_predict_finish(ta, count, st))) return rc;
+    b->ctx->launches++;
+  }
+  return 0;
+}
+
+static int postcov_check(gprb_batch* b, int64_t m, const double* Xstar, int64_t xstar_stride) {
+  int rc = predict_check(b, 0, 0, b ? b->B : 1, m, Xstar, xstar_stride);
+  if (rc) return rc;
+  GPRB_REQUIRE(m <= POSTCOV_MAX_M, "gprb_predict_cov / gprb_sample_posterior: m must be <= 8192");
+  return 0;
+}
+
+// make_posdef! + blocked Cholesky of Sigma_f for `cnt` GPs (list = nullptr: GPs 0 .. cnt-1) on `st`: the left-looking
+// schedule of the evaluation pipeline on the per-call workspace (one k_diag_factor launch when m <= 128).
+static int postcov_factor(gprb_batch* b, int64_t m, const int32_t* list, int cnt, cudaStream_t st) {
+  gprb_postcov_ws& w = b->pc;
+  const int64_t mpad = (m + NB - 1) / NB * NB;
+  const int Jm = (int)(mpad / NB), nvm = (int)((m + KT - 1) / KT * KT);
+  const int64_t ms = mpad * mpad, dstride = (int64_t)Jm * NB * NB;
+  int rc;
+  GemmArgs ga{w.L, w.DinvT, w.Dinv, w.S, w.L, nullptr, list, ms, dstride, (int)mpad, Jm, 0, GEMM_CHOL_DIAG, nvm};
+  ga.fail = w.fail;
+  if (Jm > 1) {
+    const uint64_t B = (uint64_t)b->B;
+    if ((rc = make_tensor_map(&ga.tm_L132, w.L, mpad, mpad, B, mpad, ms, NB + 4, KT)) ||
+        (rc = make_tensor_map(&ga.tm_L68, w.L, mpad, mpad, B, mpad, ms, NB / 2 + 4, KT)) ||
+        (rc = make_tensor_map(&ga.tm_A68, w.S, mpad, mpad, B, mpad, ms, NB / 2 + 4, KT)) ||
+        (rc = make_tensor_map(&ga.tm_DT132, w.DinvT, NB, (uint64_t)Jm * NB, B, NB, dstride, NB + 4, KT)) ||
+        (rc = make_tensor_map(&ga.tm_DT68, w.DinvT, NB, (uint64_t)Jm * NB, B, NB, dstride, NB / 2 + 4, KT)) ||
+        (rc = make_tensor_map(&ga.tm_D132, w.Dinv, NB, (uint64_t)Jm * NB, B, NB, dstride, NB + 4, KT)))
+      return rc;
+    ga.tm_T68 = w.tm_T68;
+  }
+  DiagArgs da{w.S, w.L, w.Dinv, w.DinvT, w.logdet, w.fail, list, ms, dstride, (int)mpad, Jm, 0, nvm};
+  for (int j = 0; j < Jm; ++j) {
+    ga.step = j;
+    if (j > 0) {  // S(0,0) = Sigma(0,0): k_diag_factor reads block column 0 straight from the workspace
+      ga.mode = GEMM_CHOL_DIAG;
+      if ((rc = launch_tile_gemm(ga, 1, cnt, st))) return rc;
+      b->ctx->launches++;
+    }
+    da.step = j;
+    da.Src = j == 0 ? w.S : nullptr;
+    if ((rc = launch_diag_factor(da, cnt, st))) return rc;
+    b->ctx->launches++;
+    if (j + 1 < Jm) {
+      ga.mode = GEMM_CHOL_COL;
+      if ((rc = launch_tile_gemm(ga, Jm - 1 - j, cnt, st))) return rc;
+      b->ctx->launches++;
+    }
+  }
+  return 0;
+}
+
+static int postcov_finish_time(gprb_batch* b) {
+  gprb_predict_slot& sl = b->ps[0];
+  GPRB_CUDA(cudaEventSynchronize(sl.t1));
+  float ms = 0.f;
+  if (cudaEventElapsedTime(&ms, sl.t0, sl.t1) == cudaSuccess) sl.last_ms = ms;
+  return 0;
+}
+
+extern "C" {
+
+int gprb_predict_cov(gprb_batch* b, int64_t m, const double* Xstar, int64_t xstar_stride, const double* mstar, int32_t add_noise,
+                     double* mu, double* cov) {
+  GPRB_REQUIRE(b && mu && cov, "gprb_predict_cov: NULL argument");
+  int rc = postcov_check(b, m, Xstar, xstar_stride);
+  if (rc) return rc;
+  GPRB_CUDA(cudaSetDevice(b->ctx->device));
+  gprb_predict_slot& sl = b->ps[0];
+  gprb_postcov_ws& w = b->pc;
+  const int B = b->B;
+  const int64_t mpad = (m + NB - 1) / NB * NB;
+  if ((rc = ensure_dev(&w.O, &w.O_cap, (size_t)B * m * m))) return rc;
+  if ((rc = postcov_enqueue(b, m, Xstar, xstar_stride, mstar, add_noise != 0))) return rc;
+  cudaStream_t st = b->stream[0];
+  // pack Sigma [B][mpad][mpad] -> [B][m][m] on the device, so that the copy to the host is one contiguous transfer
+  cudaMemcpy3DParms p = {};
+  p.srcPtr = make_cudaPitchedPtr(w.S, sizeof(double) * mpad, sizeof(double) * mpad, mpad);
+  p.dstPtr = make_cudaPitchedPtr(w.O, sizeof(double) * m, sizeof(double) * m, m);
+  p.extent = make_cudaExtent(sizeof(double) * m, m, B);
+  p.kind = cudaMemcpyDeviceToDevice;
+  GPRB_CUDA(cudaMemcpy3DAsync(&p, st));
+  GPRB_CUDA(cudaEventRecord(sl.t1, st));  // device time: the m x m blocks' copy to the host is not part of it
+  GPRB_CUDA(cudaMemcpyAsync(sl.h_out, sl.pmu, sizeof(double) * B * m, cudaMemcpyDeviceToHost, st));
+  GPRB_CUDA(cudaMemcpyAsync(cov, w.O, sizeof(double) * B * m * m, cudaMemcpyDeviceToHost, st));
+  GPRB_CUDA(cudaStreamSynchronize(st));
+  if ((rc = postcov_finish_time(b))) return rc;
+  memcpy(mu, sl.h_out, sizeof(double) * B * m);
+  return GPRB_OK;
+}
+
+int gprb_sample_posterior(gprb_batch* b, int64_t m, const double* Xstar, int64_t xstar_stride, const double* mstar, int32_t ns,
+                          const double* Z, double* out, int32_t* info) {
+  GPRB_REQUIRE(b && Z && out && info, "gprb_sample_posterior: NULL argument");
+  GPRB_REQUIRE(ns >= 1, "gprb_sample_posterior: ns must be >= 1");
+  int rc = postcov_check(b, m, Xstar, xstar_stride);
+  if (rc) return rc;
+  GPRB_CUDA(cudaSetDevice(b->ctx->device));
+  gprb_predict_slot& sl = b->ps[0];
+  gprb_postcov_ws& w = b->pc;
+  const int B = b->B;
+  const int64_t mpad = (m + NB - 1) / NB * NB, Jm = mpad / NB;
+  const size_t nz = (size_t)B * ns * m;
+  if ((rc = ensure_dev(&w.L, &w.L_cap, (size_t)B * mpad * mpad)) || (rc = ensure_dev(&w.logdet, &w.logdet_cap, (size_t)B * Jm)) ||
+      (rc = ensure_dev(&w.Z, &w.Z_cap, nz)) || (rc = ensure_dev(&w.O, &w.O_cap, nz)) ||
+      (rc = ensure_dev(&w.fail, &w.fail_cap, (size_t)B)) || (rc = ensure_dev(&w.list, &w.list_cap, (size_t)B)))
+    return rc;
+  if (w.D_cap < (size_t)B * Jm * NB * NB) {  // k_diag_factor writes only the triangular halves: the other halves stay zero
+    if ((rc = ensure_dev(&w.Dinv, &w.D_cap, (size_t)B * Jm * NB * NB, true))) return rc;
+    cudaFree(w.DinvT);
+    w.DinvT = nullptr;
+    if ((rc = dev_alloc(&w.DinvT, w.D_cap))) { w.D_cap = 0; return rc; }
+    GPRB_CUDA(cudaMemset(w.DinvT, 0, sizeof(double) * w.D_cap));
+  }
+  if (!w.fail_host) {
+    GPRB_CUDA(cudaMallocHost((void**)&w.fail_host, sizeof(int32_t) * B));
+    GPRB_CUDA(cudaMallocHost((void**)&w.list_host, sizeof(int32_t) * B));
+    GPRB_CUDA(cudaEventCreateWithFlags(&w.z_ready, cudaEventDisableTiming));
+  }
+  if ((rc = postcov_enqueue(b, m, Xstar, xstar_stride, mstar, false))) return rc;
+  cudaStream_t st = b->stream[0];
+  // the draws' standard normals (m ns B doubles, 32 MB at m = ns = 100, B = 400) travel on the upload stream while the
+  // device solves for T; only the draws wait for them
+  GPRB_CUDA(cudaMemcpyAsync(w.Z, Z, sizeof(double) * nz, cudaMemcpyHostToDevice, b->ctx->upload));
+  GPRB_CUDA(cudaEventRecord(w.z_ready, b->ctx->upload));
+  if ((rc = launch_post_fail_init(w.fail, sl.mask, w.bad, 0, B, st))) return rc;
+  // make_posdef! ladder, like eval_pass: every attempt factorises the GPs still pending, a failed GP gets one more
+  // cumulative jitter and is re-submitted alone, at most MAX_JITTER times
+  std::vector<int32_t> tries(B, 0), pend;
+  for (int i = 0; i < B; ++i) info[i] = 0;
+  const int32_t* list = nullptr;
+  int cnt = B;
+  for (;;) {
+    if ((rc = postcov_factor(b, m, list, cnt, st))) return rc;
+    GPRB_CUDA(cudaMemcpyAsync(w.fail_host, w.fail, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, st));
+    GPRB_CUDA(cudaStreamSynchronize(st));
+    std::vector<int32_t> retry;
+    for (int k = 0; k < cnt; ++k) {
+      const int g = list ? pend[k] : k;
+      const int f = w.fail_host[g];
+      if (f == 0) info[g] = tries[g];
+      else if (f < 0) info[g] = -2;
+      else if (tries[g] >= MAX_JITTER) info[g] = -1;
+      else { ++tries[g]; retry.push_back(g); }
+    }
+    if (retry.empty()) break;
+    pend = retry;
+    cnt = (int)pend.size();
+    memcpy(w.list_host, pend.data(), sizeof(int32_t) * cnt);
+    GPRB_CUDA(cudaMemcpyAsync(w.list, w.list_host, sizeof(int32_t) * cnt, cudaMemcpyHostToDevice, st));
+    if ((rc = launch_post_jitter(w.S, w.fail, w.list, (int)m, (int)mpad, cnt, st))) return rc;
+    b->ctx->launches++;
+    list = w.list;
+  }
+  GPRB_CUDA(cudaStreamWaitEvent(st, w.z_ready, 0));
+  PostDrawArgs da{w.L, sl.pmu, w.Z, w.fail, w.O, (int)m, (int)mpad, ns};
+  if ((rc = launch_post_draws(da, B, st))) return rc;
+  b->ctx->launches++;
+  GPRB_CUDA(cudaEventRecord(sl.t1, st));
+  GPRB_CUDA(cudaMemcpyAsync(out, w.O, sizeof(double) * nz, cudaMemcpyDeviceToHost, st));
+  GPRB_CUDA(cudaStreamSynchronize(st));
+  return postcov_finish_time(b);
 }
 
 }  // extern "C"

@@ -116,6 +116,25 @@ struct gprb_predict_slot {
   double last_ms = 0.0;
 };
 
+// Workspace of gprb_predict_cov / gprb_sample_posterior (allocated on first use, grow-only; slot 0's streams, staging and
+// events run the calls).  mpad = m rounded up to NB, Jm = mpad / NB.
+struct gprb_postcov_ws {
+  double* T = nullptr;      // [chunk][B][npad][PT] right-hand sides L^-1 K* of every 128-column chunk
+  double* S = nullptr;      // [B][mpad][mpad] Sigma (identity padding); the make_posdef! jitter is added in place
+  double* L = nullptr;      // [B][mpad][mpad] lower factor of Sigma_f
+  double* Dinv = nullptr; double* DinvT = nullptr;  // [B][Jm][NB*NB]; the structural-zero halves are set at allocation
+  double* logdet = nullptr; // [B][Jm] (written by k_diag_factor, unused)
+  double* Z = nullptr;      // [B][ns][m] standard normals
+  double* O = nullptr;      // [B][m][m] packed Sigma / [B][ns][m] draws for the copy to the host
+  int32_t* bad = nullptr;   // [B] 1 = non-finite Sigma
+  int32_t* fail = nullptr;  // [B] factorisation status (LAPACK info, -2 no state / non-finite)
+  int32_t* list = nullptr;  // [B] GPs of a make_posdef! retry
+  int32_t* fail_host = nullptr; int32_t* list_host = nullptr;  // pinned [B]
+  size_t T_cap = 0, S_cap = 0, L_cap = 0, D_cap = 0, logdet_cap = 0, Z_cap = 0, O_cap = 0, bad_cap = 0, fail_cap = 0, list_cap = 0;
+  CUtensorMap tm_T68;       // T as [chunk * B + GP][npad][PT], box = 68 test columns x KT rows (GEMM_FWD_ROW and k_post_cov)
+  cudaEvent_t z_ready = nullptr;  // Z has arrived (its copy runs on the upload stream, under the T solve)
+};
+
 // Per-GP device state (structure-of-arrays over the batch), all resident in HBM:
 //   A   [B][npad*npad]  K in the lower tiles (kept); after the inverse stage the strictly-upper tile (j,i) holds the
 //                       K^-1 tile (i,j) un-transposed, and KinvD the diagonal tiles of K^-1
@@ -172,6 +191,7 @@ struct gprb_batch {
   double stage_ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};
   // prediction pipelines (scratch allocated on first use and kept, grow-only): slot s runs on stream[4s .. 4s+3]
   gprb_predict_slot ps[2];
+  gprb_postcov_ws pc;             // full covariance / posterior draws (gprb_predict_cov, gprb_sample_posterior)
   // TMA tensor maps of the tile GEMM's operands (encoded once per batch; box = padded rows x KT columns x 1 GP)
   CUtensorMap tm_L132, tm_L68;     // Lm  [B][npad][npad]
   CUtensorMap tm_A68;              // A   [B][npad][npad] (L2 prefetch of the K tiles the Cholesky modes start from)
@@ -273,6 +293,17 @@ __device__ __forceinline__ double exp_nonpos(double x) {
   p = fma(p, r, 1.0);
   const int k1 = ki >> 1, k2 = ki - k1;
   return p * __hiloint2double((k1 + 1023) << 20, 0) * __hiloint2double((k2 + 1023) << 20, 0);
+}
+
+// k(r2) of the kernel family KIND for the weighted squared distance r2 (predict.cu, postcov.cu)
+template <int KIND>
+__device__ __forceinline__ double kcross(double r2, double sf2) {
+  if (KIND == GPRB_KERNEL_SE_ARD) return sf2 * exp_nonpos(-0.5 * r2);
+  const double r = sqrt(r2);
+  if (KIND == GPRB_KERNEL_MAT12_ARD) return sf2 * exp_nonpos(-r);
+  if (KIND == GPRB_KERNEL_MAT32_ARD) { const double s = 1.7320508075688772 * r; return sf2 * (1.0 + s) * exp_nonpos(-s); }
+  const double s = 2.23606797749979 * r;
+  return sf2 * (1.0 + s + 5.0 * r2 / 3.0) * exp_nonpos(-s);
 }
 
 // D(8x8) += A(8x4, row) * B(4x8, col) in fp64 on the tensor pipe (SASS DMMA.8x8x4).

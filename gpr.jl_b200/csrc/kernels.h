@@ -160,4 +160,39 @@ struct PredictTileArgs {
 int launch_predict_cross(const PredictTileArgs& a, int count, cudaStream_t stream);
 int launch_predict_finish(const PredictTileArgs& a, int count, cudaStream_t stream);
 
+// Full posterior covariance (postcov.cu): Sigma = K** - T'T (+ exp(2 logNoise) I) from the solved right-hand sides
+// T = L^-1 K* of every 128-column chunk, one CTA per lower 128 x 128 tile of Sigma and GP, both triangles written.
+// GPs gp_off .. gp_off + count - 1; T / S / bad are indexed by the local GP index (gp - gp_off) like PredictTileArgs.
+constexpr int POSTCOV_MAX_M = 8192;
+struct PostCovArgs {
+  const double* Xstar;  // d x m (+ local gp * xstar_stride)
+  const double* theta;
+  const int32_t* mask;  // [B]: 1 = no evaluated state (Sigma rows come back NaN)
+  double* S;            // [nloc][mpad][mpad] column-major; rows / columns >= m are the identity
+  int32_t* bad;         // [nloc] or nullptr: set to 1 when the GP's Sigma holds a non-finite entry
+  int64_t xstar_stride;
+  int nv, d, m, mpad, kind;
+  int gp_off, nloc;     // nloc: GPs of the whole call (chunk c of local GP g is GP index c * nloc + g of tm_T68)
+  int g0;               // first local GP of this launch (a stream group of the call): blockIdx.y + g0 = local GP
+  int add_noise;
+  CUtensorMap tm_T68;   // the T blocks [chunk][nloc][npad][PT], box = 68 test columns x KT rows (the GEMM_FWD_ROW map)
+};
+int launch_post_cov(const PostCovArgs& a, int count, cudaStream_t stream);
+int configure_post_cov();  // per-device shared-memory opt-in (current device); called by gprb_init
+
+// make_posdef! on Sigma_f of the listed GPs: A_ii += 1e-6 tr(A)/m (i < m, fixed summation order), fail reset to 0
+int launch_post_jitter(double* S, int32_t* fail, const int32_t* list, int m, int mpad, int count, cudaStream_t stream);
+// fail[g] = -2 for GPs without state (mask[gp_off + g]) or with a non-finite Sigma (bad[g]), else 0
+int launch_post_fail_init(int32_t* fail, const int32_t* mask, const int32_t* bad, int gp_off, int count, cudaStream_t stream);
+// out[g][s][i] = mu[g][i] + sum_{k <= i} L(i,k) Z[g][s][k] (k ascending); NaN for the GPs with fail[g] != 0
+struct PostDrawArgs {
+  const double* L;     // [count][mpad][mpad] lower factor (column-major)
+  const double* mu;    // [count][m]
+  const double* Z;     // [count][ns][m]
+  const int32_t* fail;
+  double* out;         // [count][ns][m]
+  int m, mpad, ns;
+};
+int launch_post_draws(const PostDrawArgs& a, int count, cudaStream_t stream);
+
 }  // namespace gprb

@@ -12,16 +12,6 @@ namespace gprb {
 
 constexpr int PRED_THREADS = 256;
 
-template <int KIND>
-__device__ __forceinline__ double kcross(double r2, double sf2) {
-  if (KIND == GPRB_KERNEL_SE_ARD) return sf2 * exp_nonpos(-0.5 * r2);
-  const double r = sqrt(r2);
-  if (KIND == GPRB_KERNEL_MAT12_ARD) return sf2 * exp_nonpos(-r);
-  if (KIND == GPRB_KERNEL_MAT32_ARD) { const double s = 1.7320508075688772 * r; return sf2 * (1.0 + s) * exp_nonpos(-s); }
-  const double s = 2.23606797749979 * r;
-  return sf2 * (1.0 + s + 5.0 * r2 / 3.0) * exp_nonpos(-s);
-}
-
 __device__ __forceinline__ double block_sum(double v, double* red) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll

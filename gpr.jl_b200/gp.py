@@ -523,8 +523,8 @@ class GPBatch:
         return out
 
     # -- prediction ---------------------------------------------------------------------------
-    def predict_y(self, Xstar, var=True, per_gp=False):
-        """Xstar d x m shared by all GPs, or (per_gp=True) a sequence of B d x m blocks.  -> mu (B,m), var (B,m)|None."""
+    def _test_block(self, Xstar, per_gp):
+        """Staged test inputs for gprb_predict / gprb_predict_cov / gprb_sample_posterior -> (Xs, stride, m, mstar|None)."""
         if per_gp:
             blocks = [as_f64(np.asarray(x, dtype=np.float64).T) for x in Xstar]
             m = blocks[0].shape[0]
@@ -542,10 +542,56 @@ class GPBatch:
         mstar = None
         if not all(isinstance(g.mean, MeanZero) for g in self.gps):
             mstar = np.ascontiguousarray(np.stack(self._means(xs_cols if per_gp else [Xstar] * self.B)))
+        return Xs, stride, m, mstar
+
+    def predict_y(self, Xstar, var=True, per_gp=False, full_cov=False):
+        """Xstar d x m shared by all GPs, or (per_gp=True) a sequence of B d x m blocks.  -> mu (B,m), var (B,m)|None;
+        full_cov=True: mu (B,m), Sigma_y (B,m,m) (``predict_y(gp, X*; full_cov=true)``)."""
+        if full_cov:
+            return self._predict_cov(Xstar, per_gp, add_noise=True)
+        Xs, stride, m, mstar = self._test_block(Xstar, per_gp)
         mu = np.empty((self.B, m))
         v = np.empty((self.B, m)) if var else None
         self.lib.check(self.lib.dll.gprb_predict(self.handle, m, _d(Xs), stride, _d(mstar), _d(mu), _d(v)))
         return mu, v
+
+    def predict_f(self, Xstar, full_cov=False, per_gp=False):
+        """Latent posterior (``predict_f``): mu (B,m) and var_f (B,m) = max(predict_y's variance - exp(2 logNoise), 0),
+        or with full_cov=True Sigma_f (B,m,m) = K** - K*' K^-1 K* (symmetric, not clamped)."""
+        if full_cov:
+            return self._predict_cov(Xstar, per_gp, add_noise=False)
+        mu, v = self.predict_y(Xstar, var=True, per_gp=per_gp)
+        noise = np.exp(2.0 * np.array([g.logNoise for g in self.gps]))
+        return mu, np.maximum(v - noise[:, None], 0.0)
+
+    def _predict_cov(self, Xstar, per_gp, add_noise):
+        Xs, stride, m, mstar = self._test_block(Xstar, per_gp)
+        mu = np.empty((self.B, m))
+        cov = np.empty((self.B, m, m))
+        self.lib.check(self.lib.dll.gprb_predict_cov(self.handle, m, _d(Xs), stride, _d(mstar), 1 if add_noise else 0,
+                                                     _d(mu), _d(cov)))
+        return mu, cov.transpose(0, 2, 1)  # column-major m x m per GP; Sigma is symmetric, the transpose is a free view
+
+    def rand(self, Xstar, nsamples=1, Z=None, rng=None, per_gp=False):
+        """Posterior draws of the latent function at Xstar (``rand(gp, X*, n)``): draws[b] = mu_b 1' + L_b Z[b] with
+        L_b the lower factor of make_posdef!(Sigma_f).  Z (B, m, nsamples) standard normals; by default drawn from
+        ``rng`` (a numpy Generator) GP by GP in Julia's ``randn(m, n)`` order.  -> (draws (B, m, ns), info (B,)):
+        info 0..10 = jitter rung, -1 = indefinite after 10 jitters, -2 = non-finite Sigma_f or no state (NaN draws)."""
+        Xs, stride, m, mstar = self._test_block(Xstar, per_gp)
+        if Z is None:
+            rng = np.random.default_rng() if rng is None else rng
+            Zc = rng.standard_normal((self.B, nsamples, m))  # per GP: column-major m x ns, filled column by column
+        else:
+            Z = np.asarray(Z, dtype=np.float64)
+            if Z.shape != (self.B, m, nsamples):
+                raise ValueError(f"Z must have shape {(self.B, m, nsamples)}, got {Z.shape}")
+            Zc = Z.transpose(0, 2, 1)
+        Zc = np.ascontiguousarray(Zc, dtype=np.float64)
+        out = np.empty((self.B, nsamples, m))
+        info = np.zeros(self.B, dtype=np.int32)
+        self.lib.check(self.lib.dll.gprb_sample_posterior(self.handle, m, _d(Xs), stride, _d(mstar), nsamples, _d(Zc), _d(out),
+                                                          info.ctypes.data_as(C.POINTER(C.c_int32))))
+        return out.transpose(0, 2, 1), info
 
     def predict_async(self, slot, gp0, gp1, blocks, var=False, gps_per_block=1):
         """gprb_predict_async: enqueue the prediction of GPs gp0..gp1-1 on pipeline ``slot`` (0 or 1) and return at
@@ -664,3 +710,35 @@ def predict_y(gp, Xstar, var=True):
         return mu[0], (v[0] if var else None)
     mu, v = b.predict_y(Xstar, var=var)
     return mu[gp._slot], (v[gp._slot] if var else None)
+
+
+def _resident(gp):
+    if gp._batch is None:
+        GPBatch([gp]).update_mll()
+    return gp._batch
+
+
+def predict_f(gp, Xstar, full_cov=False):
+    """``predict_f(gp, Xstar; full_cov) -> (mu, sigma2 | Sigma_f)`` for one GPE, or batched for a GPBatch."""
+    if isinstance(gp, GPBatch):
+        return gp.predict_f(Xstar, full_cov=full_cov)
+    mu, v = _resident(gp).predict_f(Xstar, full_cov=full_cov)
+    return mu[gp._slot], v[gp._slot]
+
+
+def rand(gp, Xstar, nsamples=1, Z=None, rng=None):
+    """``rand(gp, Xstar, n)``: posterior draws (m, n) of one GPE (Z: (m, n) standard normals, or drawn from ``rng``);
+    raises LinAlgError where make_posdef! gives up.  For a GPBatch: ``GPBatch.rand`` -> (draws (B, m, n), info)."""
+    if isinstance(gp, GPBatch):
+        return gp.rand(Xstar, nsamples, Z=Z, rng=rng)
+    b = _resident(gp)
+    m = np.asarray(Xstar).reshape(np.asarray(Xstar).shape[0], -1).shape[1]
+    if Z is None:
+        rng = np.random.default_rng() if rng is None else rng
+        Z = rng.standard_normal((nsamples, m)).T
+    Zb = np.zeros((b.B, m, nsamples))
+    Zb[gp._slot] = Z
+    draws, info = b.rand(Xstar, nsamples, Z=Zb)
+    if info[gp._slot] < 0:
+        raise np.linalg.LinAlgError(f"posterior covariance is not positive definite (info {int(info[gp._slot])})")
+    return draws[gp._slot]

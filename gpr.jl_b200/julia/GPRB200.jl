@@ -26,13 +26,14 @@
 module GPRB200
 
 using Libdl
+import Random
 import GaussianProcesses
 import GaussianProcesses: GPE, Mean, MeanZero, Kernel, SEArd, Mat12Ard, Mat32Ard, Mat52Ard, CovarianceStrategy, KernelData, EmptyData,
                           get_params, set_params!, num_params
 import Optim
 import PDMats
 
-export B200Covariance, GPBatch, params_to_theta, theta_to_params, gather_results
+export B200Covariance, GPBatch, params_to_theta, theta_to_params, gather_results, predict_cov, sample_posterior!
 
 const LIB = get(ENV, "GPRB200_LIB", joinpath(@__DIR__, "..", "libgprb200.so"))
 
@@ -263,15 +264,101 @@ end
 
 # The reference's call `predict_y(gp, obs)[1][1]` (predictdynamics.jl:13), once per GP of the trial with the SAME obs:
 # the first call predicts every GP of the batch on the device, the other G-1 calls are served from the step cache
-# (the device-side twin of MDCache, src/mDynamics.jl:6-11).
-function GaussianProcesses.predict_y(gp::B200GPE, Xstar::AbstractMatrix)
+# (the device-side twin of MDCache, src/mDynamics.jl:6-11).  `full_cov=true` returns the joint m×m predictive covariance.
+function GaussianProcesses.predict_y(gp::B200GPE, Xstar::AbstractMatrix; full_cov::Bool = false)
     batch, slot = residence(gp)
+    if full_cov
+        μ, Σ = predict_cov(batch, Xstar; add_noise = true)
+        return μ[:, slot], Σ[:, :, slot]
+    end
     if size(batch.cache_key) != size(Xstar) || batch.cache_key != Xstar
         μ, σ2 = GaussianProcesses.predict_y(batch, Xstar; var = true)
         batch.cache_key, batch.cache_mu, batch.cache_var = Matrix{Float64}(Xstar), μ, σ2
     end
     batch.cache_mu[:, slot], batch.cache_var[:, slot]
 end
+
+# ---- predict_f / full_cov / rand (GaussianProcesses 0.12.4 GP.jl, GPE.jl) ------------------------------------------------
+# Without these methods the generic predictMVN / rand! of GaussianProcesses would read gp.cK (a placeholder here) and
+# gp.alpha (filled on demand): every call below goes to the device instead.
+prior_means(batch::GPBatch, Xs::Matrix{Float64}) = all(gp -> gp.mean isa MeanZero, batch.gps) ? nothing :
+    [GaussianProcesses.mean(batch.gps[b].mean, Xs[:, j]) for j in 1:size(Xs, 2), b in 1:batch.B]
+
+"predict_cov(batch, Xstar) -> (μ::m×B, Σ::m×m×B): Σ_f = K** - K*'K⁻¹K* (`add_noise=false`) or Σ_y = Σ_f + σ²_n I."
+function predict_cov(batch::GPBatch, Xstar::AbstractMatrix; add_noise::Bool)
+    Xs = Matrix{Float64}(Xstar)
+    m = size(Xs, 2)
+    mstar = prior_means(batch, Xs)
+    μ = Matrix{Float64}(undef, m, batch.B)
+    Σ = Array{Float64,3}(undef, m, m, batch.B)
+    GC.@preserve Xs mstar μ Σ begin
+        check(ccall((:gprb_predict_cov, LIB), Cint, (Ptr{Cvoid}, Int64, Ptr{Float64}, Int64, Ptr{Float64}, Int32, Ptr{Float64}, Ptr{Float64}),
+                    batch.handle, m, Xs, 0, mstar === nothing ? C_NULL : pointer(mstar), add_noise ? 1 : 0, μ, Σ))
+    end
+    μ, Σ
+end
+
+"predict_f(batch, Xstar; full_cov) -> (μ::m×B, σ²_f::m×B | Σ_f::m×m×B): the latent posterior (no observation noise)."
+function predict_f(batch::GPBatch, Xstar::AbstractMatrix; full_cov::Bool = false)
+    full_cov && return predict_cov(batch, Xstar; add_noise = false)
+    μ, σ2 = GaussianProcesses.predict_y(batch, Xstar; var = true)
+    for b in 1:batch.B
+        σ2[:, b] .= max.(σ2[:, b] .- exp(2 * batch.gps[b].logNoise), 0.0)
+    end
+    μ, σ2
+end
+
+function GaussianProcesses.predict_f(gp::B200GPE, Xstar::AbstractMatrix; full_cov::Bool = false)
+    batch, slot = residence(gp)
+    μ, v = predict_f(batch, Xstar; full_cov = full_cov)
+    full_cov ? (μ[:, slot], v[:, :, slot]) : (μ[:, slot], v[:, slot])
+end
+
+"""
+    sample_posterior!(batch, Xstar, A::Array{Float64,3}, Z::Array{Float64,3}) -> info::Vector{Int32}
+
+Draws of every GP's latent posterior at Xstar: A[:, :, b] = μ_b + L_b Z[:, :, b], L_b the lower factor of
+make_posdef!(Σ_f).  info[b]: jitter rung 0..10, -1 indefinite after 10 jitters, -2 non-finite Σ_f / no state (NaN draws).
+"""
+function sample_posterior!(batch::GPBatch, Xstar::AbstractMatrix, A::Array{Float64,3}, Z::Array{Float64,3})
+    Xs = Matrix{Float64}(Xstar)
+    m, ns = size(Xs, 2), size(A, 2)
+    size(A) == size(Z) == (m, ns, batch.B) || throw(DimensionMismatch("A and Z must be m × n × B"))
+    mstar = prior_means(batch, Xs)
+    info = zeros(Int32, batch.B)
+    GC.@preserve Xs mstar A Z info begin
+        check(ccall((:gprb_sample_posterior, LIB), Cint,
+                    (Ptr{Cvoid}, Int64, Ptr{Float64}, Int64, Ptr{Float64}, Int32, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}),
+                    batch.handle, m, Xs, 0, mstar === nothing ? C_NULL : pointer(mstar), ns, Z, A, info))
+    end
+    info
+end
+
+"Batched `rand`: draws m × n × B with Z = randn(m, n) per GP (the order GaussianProcesses' rand! draws them in)."
+function Random.rand(batch::GPBatch, Xstar::AbstractMatrix, n::Integer = 1)
+    m = size(Xstar, 2)
+    Z = Array{Float64,3}(undef, m, n, batch.B)
+    for b in 1:batch.B
+        Z[:, :, b] = randn(m, n)
+    end
+    A = similar(Z)
+    sample_posterior!(batch, Xstar, A, Z), A
+end
+
+# `rand!(gp, X, A)` (GPE.jl): Z = randn(nobs, n_sample) on the host exactly as GaussianProcesses draws it, then
+# A = μ + chol_lower(make_posdef!(Σ_f)) Z on the device.  A factorisation that fails raises PosDefException.
+function Random.rand!(gp::B200GPE, x::AbstractMatrix, A::DenseMatrix)
+    batch, slot = residence(gp)
+    m, ns = size(x, 2), size(A, 2)
+    Zb = zeros(m, ns, batch.B)
+    Zb[:, :, slot] = randn(m, ns)
+    Ab = similar(Zb)
+    info = sample_posterior!(batch, x, Ab, Zb)
+    info[slot] < 0 && throw(PDMats.PosDefException(Int(info[slot])))
+    A .= view(Ab, :, :, slot)
+end
+Random.rand(gp::B200GPE, x::AbstractMatrix, n::Int) = Random.rand!(gp, x, Matrix{Float64}(undef, size(x, 2), n))
+Random.rand(gp::B200GPE, x::AbstractMatrix) = vec(Random.rand(gp, x, 1))
 
 # ---- asynchronous rollout step (two trial groups alternate: device predict of one under the host projectv! of the other) -----
 "Enqueue the mean prediction of GPs gp0:gp1 (1-based, inclusive) at the per-trial state blocks `states` (d × m × trials) on pipeline `slot`."

@@ -13,6 +13,8 @@
  *       -> gprb_optimize       (batched lock-step restatement, per-GP masks)
  *   predict_y(gp, Xstar)                                   examples/utils/predictdynamics.jl:13
  *       -> gprb_predict
+ *   predict_f / predict_y(gp, Xstar; full_cov=true), rand(gp, Xstar, n)   (GaussianProcesses 0.12.4 GP.jl / GPE.jl)
+ *       -> gprb_predict_cov, gprb_sample_posterior
  *   gp.cK / gp.alpha inspection (parity taps)              -> gprb_get_K / _chol / _alpha / _Kinv
  *
  * Conventions
@@ -187,6 +189,27 @@ int gprb_predict_async(gprb_batch* batch, int32_t slot, int32_t gp0, int32_t gp1
 int gprb_predict_wait(gprb_batch* batch, int32_t slot, double* mu, double* var);
 /* Device time (ms, CUDA events on the slot's stream) of the most recent completed prediction on `slot`. */
 int gprb_last_predict_ms(gprb_batch* batch, int32_t slot, double* ms);
+
+/* ---- full covariance and posterior draws (predict_f / predict_y with full_cov = true, rand) -------------------- */
+/* Synchronous, on prediction slot 0 (refused while slot 0 has an asynchronous prediction in flight); 1 <= m <= 8192,
+ * larger m is GPRB_ERR_ARG, a workspace that cannot be allocated GPRB_ERR_NOMEM.  Xstar / xstar_stride / mstar as for
+ * gprb_predict.  gprb_last_predict_ms(batch, 0) reports the device time (without the copy of the m x m blocks).
+ * With T = L^-1 K*, K** = K_f(X*, X*) (no noise, no eps):
+ *   Sigma_f = K** - T'T (symmetric, not clamped),  Sigma_y = Sigma_f + exp(2 logNoise) I
+ *   mu   m x B      out, as gprb_predict
+ *   cov  m x m x B  out, both triangles; add_noise = 0: Sigma_f (predict_f), 1: Sigma_y (predict_y)
+ * A GP without an evaluated state gets NaN mu / cov and blocks nobody. */
+int gprb_predict_cov(gprb_batch* batch, int64_t m, const double* Xstar, int64_t xstar_stride, const double* mstar,
+                     int32_t add_noise, double* mu, double* cov);
+/* Posterior draws of the latent function (rand / rand!): out[:, s, b] = mu_b + L_b Z[:, s, b], L_b the lower Cholesky
+ * factor of make_posdef!(Sigma_f) (cumulative Sigma_ii += 1e-6 tr(Sigma)/m, up to 10 times).  The standard normals come
+ * from the caller's RNG.
+ *   Z    m x ns x B  in
+ *   out  m x ns x B  out
+ *   info B           out: 0..10 jitter rung, -1 still indefinite after 10 jitters, -2 non-finite Sigma_f or no evaluated
+ *                    state; a GP with info < 0 gets NaN draws and blocks nobody */
+int gprb_sample_posterior(gprb_batch* batch, int64_t m, const double* Xstar, int64_t xstar_stride, const double* mstar,
+                          int32_t ns, const double* Z, double* out, int32_t* info);
 
 /* ---- parity taps (state after the last gprb_eval of GP b) ------------------------------ */
 int gprb_get_K(gprb_batch* batch, int32_t b, double* out /* n x n, symmetric, noise + jitter included */);
