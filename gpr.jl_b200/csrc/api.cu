@@ -95,6 +95,11 @@ static void free_batch(gprb_batch* b) {
     if (w.list_host) cudaFreeHost(w.list_host);
     if (w.z_ready) cudaEventDestroy(w.z_ready);
   }
+  {
+    gprb_loo_ws& w = b->loo;
+    cudaFree(w.M); cudaFree(w.W); cudaFree(w.KD); cudaFree(w.vec); cudaFree(w.part); cudaFree(w.mll); cudaFree(w.out); cudaFree(w.skip);
+    if (w.skip_host) cudaFreeHost(w.skip_host);
+  }
   if (b->list_host) cudaFreeHost(b->list_host);
   if (b->fail_host) cudaFreeHost(b->fail_host);
   if (b->stage_host) cudaFreeHost(b->stage_host);
@@ -478,7 +483,7 @@ using namespace gprb;
 
 extern "C" {
 
-int gprb_version(void) { return 300; }
+int gprb_version(void) { return 301; }
 const char* gprb_last_error(void) { return g_err.c_str(); }
 
 int gprb_init(gprb_ctx** out, int device) {
@@ -1423,6 +1428,158 @@ int gprb_sample_posterior(gprb_batch* b, int64_t m, const double* Xstar, int64_t
   GPRB_CUDA(cudaMemcpyAsync(out, w.O, sizeof(double) * nz, cudaMemcpyDeviceToHost, st));
   GPRB_CUDA(cudaStreamSynchronize(st));
   return postcov_finish_time(b);
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------------
+// Leave-one-out cross-validation (gprb_eval_loo; kernels in loo.cu).  Value only: one pointwise launch over the batch.
+// With the gradient, per group of consecutive GPs: pointwise terms, u = K^-1 (alpha ./ d) by k_solve on the resident
+// factor, G = diag(sqrt(-c)) K^-1, W = -G'G (zero-initialised k_post_cov), A' = [K | -Q'], then the fused gradient
+// kernels unchanged on A' with a zero alpha.  launch_solve / launch_grad index every buffer by the GP index of their
+// launch: the batch buffers are passed offset to the group's first GP, the group buffers as they are.
+constexpr size_t LOO_WS_BYTES = (size_t)8 << 30;  // bound of the group buffers (about 2 npad^2 doubles per GP)
+
+static void loo_free_groups(gprb_loo_ws& w) {
+  cudaFree(w.M); cudaFree(w.W); cudaFree(w.KD); cudaFree(w.vec); cudaFree(w.part); cudaFree(w.mll);
+  w.M = w.W = w.KD = w.vec = w.part = w.mll = nullptr;
+  w.cap = 0;
+}
+
+// Group buffers for `want` GPs; when the device cannot hold them, for half as many, down to one GP.
+static int loo_alloc_groups(gprb_batch* b, int want) {
+  gprb_loo_ws& w = b->loo;
+  if (w.cap >= want) return 0;
+  loo_free_groups(w);
+  const size_t mat = (size_t)b->npad * b->npad, dn = (size_t)b->J * NB * NB;
+  const size_t part = (size_t)b->J * (b->J + 1) / 2 * GRAD_PARTS_PER_TILE * b->P;
+  for (int cap = want;; cap = std::max(1, cap / 2)) {
+    int rc;
+    if (!(rc = dev_alloc(&w.M, cap * mat)) && !(rc = dev_alloc(&w.W, cap * mat)) && !(rc = dev_alloc(&w.KD, cap * dn)) &&
+        !(rc = dev_alloc(&w.vec, 5 * (size_t)cap * b->npad)) && !(rc = dev_alloc(&w.part, cap * part)) &&
+        !(rc = dev_alloc(&w.mll, (size_t)cap))) {
+      GPRB_CUDA(cudaMemset(w.vec + 4 * (size_t)cap * b->npad, 0, sizeof(double) * cap * b->npad));  // the zero alpha
+      w.cap = cap;
+      return 0;
+    }
+    loo_free_groups(w);
+    if (rc != GPRB_ERR_NOMEM || cap == 1) return rc;
+    cudaGetLastError();  // an allocation failure is not sticky: clear it and try a smaller group
+  }
+}
+
+static int loo_stage(gprb_batch* b, const uint8_t* mode, const std::vector<int32_t>& info, double* logp, double* grad,
+                     double* mu, double* var) {
+  gprb_loo_ws& w = b->loo;
+  const int B = b->B, P = b->P, J = b->J;
+  const int64_t n = b->n, npad = b->npad, ms = npad * npad, ds = (int64_t)J * NB * NB;
+  const size_t nout = (size_t)B * (1 + P + 2 * n);
+  int rc;
+  if ((rc = ensure_dev(&w.out, &w.out_cap, nout))) return rc;
+  if (!w.skip) {
+    if ((rc = dev_alloc(&w.skip, (size_t)B))) return rc;
+    GPRB_CUDA(cudaMallocHost((void**)&w.skip_host, sizeof(int32_t) * B));
+  }
+  double* d_logp = w.out;
+  double* d_grad = d_logp + B;
+  double* d_mu = d_grad + (size_t)B * P;
+  double* d_var = d_mu + (size_t)B * n;
+  bool any = false;
+  for (int i = 0; i < B; ++i) {
+    w.skip_host[i] = (mode[i] && info[i] >= 0) ? 0 : 1;
+    any = any || !w.skip_host[i];
+  }
+  cudaStream_t st = b->stream[0];
+  int64_t& launches = b->ctx->launches;
+  if (any) {
+    GPRB_CUDA(cudaMemcpyAsync(w.skip, w.skip_host, sizeof(int32_t) * B, cudaMemcpyHostToDevice, st));
+    LooArgs la{b->A, b->KinvD, b->alpha, b->ymm, w.skip, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
+               d_mu, d_var, d_logp, ms, ds, (int)n, (int)npad, J, 0};
+    if (!grad) {
+      if ((rc = launch_loo_point(la, B, st))) return rc;
+      ++launches;
+    } else {
+      const size_t per_gp = sizeof(double) * (2 * (size_t)ms + ds + 5 * npad + (size_t)J * (J + 1) / 2 * GRAD_PARTS_PER_TILE * P + 1);
+      if ((rc = loo_alloc_groups(b, (int)std::max<size_t>(1, std::min<size_t>(B, LOO_WS_BYTES / per_gp))))) return rc;
+      const int cap = std::min(w.cap, B), nv = (int)((n + KT - 1) / KT * KT);
+      double* v = w.vec;
+      double* s = v + (size_t)cap * npad;
+      double* u = s + (size_t)cap * npad;
+      double* z = u + (size_t)cap * npad;
+      const double* zero = z + (size_t)cap * npad;
+      for (int g0 = 0; g0 < B; g0 += cap) {
+        const int cnt = std::min(cap, B - g0);
+        bool work = false;
+        for (int i = g0; i < g0 + cnt; ++i) work = work || !w.skip_host[i];
+        if (!work) continue;
+        la.gp0 = g0; la.v = v; la.s = s; la.u = u; la.G = w.M; la.W = w.W; la.Ap = w.M; la.KinvDp = w.KD;
+        if ((rc = launch_loo_point(la, cnt, st))) return rc;
+        SolveArgs sa{b->Lm + g0 * ms, b->Dinv + g0 * ds, v, b->logdet_part + (int64_t)g0 * J, w.skip + g0, z, u, w.mll, nullptr,
+                     ms, ds, (int)n, (int)npad, J, nv};
+        sa.cluster_below = b->solve_cluster_below;
+        if ((rc = launch_solve(sa, cnt, st))) return rc;
+        if ((rc = launch_loo_expand(la, cnt, st))) return rc;
+        PostCovArgs pa{nullptr, b->theta + (int64_t)g0 * P, w.skip + g0, w.W, nullptr, 0, nv, b->d, (int)n, (int)npad, b->kind,
+                       0, cnt, 0, 0, {}};
+        if ((rc = make_tensor_map(&pa.tm_T68, w.M, PT, (uint64_t)npad, (uint64_t)J * cnt, PT, (uint64_t)npad * PT, NB / 2 + 4, KT)))
+          return rc;
+        if ((rc = launch_loo_w(pa, cnt, st))) return rc;
+        if ((rc = launch_loo_assemble(la, cnt, st))) return rc;
+        GradArgs gr{b->Xtptr + g0, b->theta + (int64_t)g0 * P, w.M, w.KD, zero, w.part, d_grad + (int64_t)g0 * P, w.skip + g0,
+                    nullptr, ms, ds, (int)n, (int)npad, b->d, J, b->kind};
+        if ((rc = launch_grad(gr, cnt, st))) return rc;
+        launches += 7;  // point, solve, expand, W, assemble, gradient tiles + reduction
+      }
+    }
+  }
+  std::vector<double> h(nout);
+  if (any) {
+    GPRB_CUDA(cudaMemcpyAsync(h.data(), d_logp, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
+    if (grad) GPRB_CUDA(cudaMemcpyAsync(h.data() + B, d_grad, sizeof(double) * B * P, cudaMemcpyDeviceToHost, st));
+    if (mu || var) GPRB_CUDA(cudaMemcpyAsync(h.data() + B + (size_t)B * P, d_mu, sizeof(double) * 2 * B * n, cudaMemcpyDeviceToHost, st));
+    GPRB_CUDA(cudaStreamSynchronize(st));
+  }
+  const double ninf = -std::numeric_limits<double>::infinity(), qnan = std::numeric_limits<double>::quiet_NaN();
+  const double* hg = h.data() + B;
+  const double* hm = hg + (size_t)B * P;
+  const double* hv = hm + (size_t)B * n;
+  for (int gp = 0; gp < B; ++gp) {
+    if (!mode[gp]) continue;
+    const bool ok = info[gp] >= 0;
+    logp[gp] = ok ? h[gp] : ninf;
+    if (grad)
+      for (int p = 0; p < P; ++p) grad[(size_t)gp * P + p] = ok ? hg[(size_t)gp * P + p] : qnan;
+    for (int64_t i = 0; i < n; ++i) {
+      if (mu) mu[(size_t)gp * n + i] = ok ? hm[(size_t)gp * n + i] : qnan;
+      if (var) var[(size_t)gp * n + i] = ok ? hv[(size_t)gp * n + i] : qnan;
+    }
+  }
+  return 0;
+}
+
+extern "C" {
+
+int gprb_eval_loo(gprb_batch* b, const double* theta, const uint8_t* active, double* mll, double* grad, double* logp_loo,
+                  double* grad_loo, double* mu_loo, double* var_loo, int32_t* info) {
+  GPRB_REQUIRE(b && theta && logp_loo && info, "gprb_eval_loo: NULL argument");
+  GPRB_CUDA(cudaSetDevice(b->ctx->device));
+  const int B = b->B;
+  // the evaluation of gprb_eval with a gradient (the LOO terms need K^-1), with its state reuse
+  std::vector<uint8_t> mode(B);
+  std::vector<int32_t> act;
+  for (int i = 0; i < B; ++i) {
+    mode[i] = (!active || active[i]) ? 2 : 0;
+    if (mode[i]) act.push_back(i);
+  }
+  int rc = upload_theta_rows(b, theta, act);
+  if (rc) return rc;
+  std::vector<int32_t> inf;
+  if ((rc = evaluate_modes(b, theta, mode.data(), inf))) return rc;
+  std::vector<double> tmll, tgrad;
+  if (!mll) { tmll.resize(B); mll = tmll.data(); }
+  if (!grad) { tgrad.resize((size_t)B * b->P); grad = tgrad.data(); }
+  if ((rc = download_results(b, mode.data(), inf, nullptr, mll, grad, info))) return rc;
+  return loo_stage(b, mode.data(), inf, logp_loo, grad_loo, mu_loo, var_loo);
 }
 
 }  // extern "C"

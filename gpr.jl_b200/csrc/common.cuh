@@ -135,6 +135,22 @@ struct gprb_postcov_ws {
   cudaEvent_t z_ready = nullptr;  // Z has arrived (its copy runs on the upload stream, under the T solve)
 };
 
+// Workspace of gprb_eval_loo (allocated on first use, grow-only).  The GPs are processed in groups of at most `cap`
+// consecutive batch indices; the group buffers are indexed by the GP's position in its group.
+struct gprb_loo_ws {
+  double* M = nullptr;      // [cap][npad][npad] G = diag(sqrt(-c)) K^-1 (chunked right-hand-side layout), then A'
+  double* W = nullptr;      // [cap][npad][npad] K^-1 diag(c) K^-1
+  double* KD = nullptr;     // [cap][J][NB*NB] diagonal tiles of -Q'
+  double* vec = nullptr;    // [5][cap][npad] v = alpha ./ d, s = sqrt(-c), u = K^-1 v, the substitution's z, zero alpha
+  double* part = nullptr;   // [cap][ntiles * GRAD_PARTS_PER_TILE][P] gradient partial sums
+  double* mll = nullptr;    // [cap] the substitution's mll (not used)
+  int cap = 0;              // GPs per group the buffers above hold
+  double* out = nullptr;    // logp [B] | grad [B][P] | mu [B][n] | var [B][n], indexed by the batch GP index
+  int32_t* skip = nullptr;  // [B] 1 = not processed (inactive or failed evaluation)
+  int32_t* skip_host = nullptr;  // pinned [B]
+  size_t out_cap = 0;
+};
+
 // Per-GP device state (structure-of-arrays over the batch), all resident in HBM:
 //   A   [B][npad*npad]  K in the lower tiles (kept); after the inverse stage the strictly-upper tile (j,i) holds the
 //                       K^-1 tile (i,j) un-transposed, and KinvD the diagonal tiles of K^-1
@@ -192,6 +208,7 @@ struct gprb_batch {
   // prediction pipelines (scratch allocated on first use and kept, grow-only): slot s runs on stream[4s .. 4s+3]
   gprb_predict_slot ps[2];
   gprb_postcov_ws pc;             // full covariance / posterior draws (gprb_predict_cov, gprb_sample_posterior)
+  gprb_loo_ws loo;                // leave-one-out cross-validation (gprb_eval_loo)
   // TMA tensor maps of the tile GEMM's operands (encoded once per batch; box = padded rows x KT columns x 1 GP)
   CUtensorMap tm_L132, tm_L68;     // Lm  [B][npad][npad]
   CUtensorMap tm_A68;              // A   [B][npad][npad] (L2 prefetch of the K tiles the Cholesky modes start from)

@@ -195,4 +195,32 @@ struct PostDrawArgs {
 };
 int launch_post_draws(const PostDrawArgs& a, int count, cudaStream_t stream);
 
+// Leave-one-out cross-validation (loo.cu), Rasmussen & Williams eqs. 5.10-5.13 on the resident K^-1 and alpha, for the
+// GPs gp0 .. gp0 + cnt - 1.  Batch buffers (A, KinvD, alpha, ymm, skip, mu, var, logp) are indexed by the global GP
+// index, the per-call workspace (v, s, u, G, W, Ap, KinvDp) by the local one (gp - gp0).  skip[gp] != 0: not processed.
+struct LooArgs {
+  const double* A;       // batch [B][npad*npad]: K in the lower tiles, K^-1 tile (i,j), i > j, at tile position (j,i)
+  const double* KinvD;   // batch [B][J][NB*NB] diagonal tiles of K^-1
+  const double* alpha;   // batch [B][npad]
+  const double* ymm;     // batch [B][npad]
+  const int32_t* skip;   // [B]
+  double* v;             // [cnt][npad] alpha ./ diag(K^-1), zero padded (nullptr: value only)
+  double* s;             // [cnt][npad] sqrt(-c), c_i = -1/2 (1 + alpha_i^2 / d_i) / d_i, zero padded
+  const double* u;       // [cnt][npad] K^-1 v
+  double* G;             // [J][cnt][npad][PT] diag(s) K^-1 in the right-hand-side layout of GEMM_FWD_ROW / k_post_cov
+  const double* W;       // [cnt][npad][npad] K^-1 diag(c) K^-1, exactly symmetric
+  double* Ap;            // [cnt][npad][npad] K in the lower tiles, -Q' in the strictly-upper ones (K^-1 convention)
+  double* KinvDp;        // [cnt][J][NB*NB] diagonal tiles of -Q'
+  double* mu;            // [B][n] y - m(X) - alpha_i / d_i
+  double* var;           // [B][n] 1 / d_i
+  double* logp;          // [B]
+  int64_t mat_stride, dinv_stride;
+  int n, npad, J, gp0;
+};
+int launch_loo_point(const LooArgs& a, int count, cudaStream_t stream);     // pointwise terms, logp, v and s
+int launch_loo_expand(const LooArgs& a, int count, cudaStream_t stream);    // G = diag(s) K^-1
+int launch_loo_assemble(const LooArgs& a, int count, cudaStream_t stream);  // Ap, KinvDp
+// W = -G'G on the DMMA pipe: k_post_cov with zero-initialised accumulators (no K** prologue, no noise), m = n, mpad = npad
+int launch_loo_w(const PostCovArgs& a, int count, cudaStream_t stream);
+
 }  // namespace gprb

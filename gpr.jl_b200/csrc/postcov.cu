@@ -36,8 +36,13 @@ __device__ __forceinline__ void post_tile_index(int bx, int& i, int& j) {  // bx
   j = bx - i * (i + 1) / 2;
 }
 
+// KIND = PCV_ZERO: the leave-one-out product W = -G'G (loo.cu) - the accumulators start at zero instead of K**, no test
+// inputs, theta or noise are read; T is G.
+constexpr int PCV_ZERO = 4;
+
 template <int KIND>
 __global__ void __launch_bounds__(PCV_THREADS, 1) k_post_cov(const __grid_constant__ PostCovArgs g) {
+  constexpr bool ZERO = KIND == PCV_ZERO;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   double* ring = reinterpret_cast<double*>(smem_raw);
   uint64_t* full = reinterpret_cast<uint64_t*>(ring + PCV_NSTAGE * PCV_STAGE);
@@ -68,12 +73,13 @@ __global__ void __launch_bounds__(PCV_THREADS, 1) k_post_cov(const __grid_consta
 #pragma unroll
     for (int ni = 0; ni < 4; ++ni) acc[mi][ni][0] = acc[mi][ni][1] = 0.0;
   const double* th = g.theta + (int64_t)gp * (d + 2);
-  const double sf2 = exp(2.0 * th[d + 1]);
+  const double sf2 = ZERO ? 0.0 : exp(2.0 * th[d + 1]);
   if (!masked) {
     if (threadIdx.x == 0) {
       for (int s = 0; s < PCV_NSTAGE; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], PCV_WARPS); }
       mbar_fence_init();
     }
+    if constexpr (!ZERO) {
     // prologue: the ring holds the tile's test inputs xi [d][NB] (rows) and xj [d][NB] (columns) while the accumulators
     // are set to K** by direct differences; then it becomes the operand ring of the k-loop
     const double* xi = ring;
@@ -110,6 +116,7 @@ __global__ void __launch_bounds__(PCV_THREADS, 1) k_post_cov(const __grid_consta
           for (int e = 0; e < 2; ++e)
             if (c0t + ni * 8 + 2 * t + e < mvj) acc[mi][ni][e] = kcross<KIND>(r2[ni][e], sf2);
       }
+    }
     }
     fence_proxy_async();  // the generic-proxy reads of the inputs are ordered before the TMA writes into the same ring
     __syncthreads();
@@ -164,7 +171,7 @@ __global__ void __launch_bounds__(PCV_THREADS, 1) k_post_cov(const __grid_consta
       if (++stage == PCV_NSTAGE) { stage = 0; phase ^= 1; }
     }
   }
-  const double noise = g.add_noise ? exp(2.0 * th[0]) : 0.0;
+  const double noise = (!ZERO && g.add_noise) ? exp(2.0 * th[0]) : 0.0;
   const double qnan = __longlong_as_double(0x7ff8000000000000LL);
   const int64_t mpad = g.mpad;
   double* S = g.S + (int64_t)gl * mpad * mpad;
@@ -200,7 +207,17 @@ int configure_post_cov() {
   if (e == cudaSuccess) e = cudaFuncSetAttribute(k_post_cov<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PCV_SMEM);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(k_post_cov<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PCV_SMEM);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(k_post_cov<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PCV_SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_post_cov<PCV_ZERO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PCV_SMEM);
   if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(k_post_cov)", __FILE__, __LINE__);
+  return 0;
+}
+
+int launch_loo_w(const PostCovArgs& a, int count, cudaStream_t stream) {
+  if (count <= 0) return 0;
+  const int Jm = a.mpad / NB;
+  k_post_cov<PCV_ZERO><<<dim3(Jm * (Jm + 1) / 2, count), PCV_THREADS, PCV_SMEM, stream>>>(a);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return cuda_fail(e, "k_post_cov (leave-one-out W) launch", __FILE__, __LINE__);
   return 0;
 }
 

@@ -459,6 +459,36 @@ class GPBatch:
         self._grad[wg] = g[wg]
         return mll, g, info
 
+    def eval_loo(self, theta=None, grad=True, active=None, mu_var=False):
+        """Leave-one-out cross-validation (gprb_eval_loo): evaluates like ``eval(theta, grad=True)`` - the batch's mll,
+        dmll and info are updated - then logp_CVLOO and, with ``grad``, its gradient for every active GP.
+        -> (logp (B,), grad (B,P) | None, info (B,)); with ``mu_var`` also (mu (B,n), var (B,n)) of y - m(X).
+        A GP with info < 0 gets logp = -Inf and NaN rows; rows of inactive GPs are NaN."""
+        theta = as_f64(self.get_params() if theta is None else theta).reshape(self.B, self.P)
+        mll = np.full(self.B, np.nan)
+        g = np.full((self.B, self.P), np.nan)
+        logp = np.full(self.B, np.nan)
+        gl = np.full((self.B, self.P), np.nan) if grad else None
+        mu = np.full((self.B, self.n), np.nan) if mu_var else None
+        var = np.full((self.B, self.n), np.nan) if mu_var else None
+        info = np.zeros(self.B, dtype=np.int32)
+        act = None if active is None else np.ascontiguousarray(active, dtype=np.uint8)
+        self.lib.check(self.lib.dll.gprb_eval_loo(
+            self.handle, _d(theta), act.ctypes.data_as(C.POINTER(C.c_uint8)) if act is not None else None,
+            _d(mll), _d(g), _d(logp), _d(gl), _d(mu), _d(var), info.ctypes.data_as(C.POINTER(C.c_int32))))
+        sel = slice(None) if act is None else act.astype(bool)
+        self._mll[sel], self._info[sel], self._has_grad[sel] = mll[sel], info[sel], True
+        self._grad[sel] = g[sel]
+        if mu_var:
+            return logp, gl, info, (mu, var)
+        return logp, gl, info
+
+    def predict_LOO(self, active=None):
+        """``predict_LOO``: leave-one-out predictive mean (m(X) included) and variance of every training point
+        -> (mu (B,n), var (B,n)), NaN rows for a GP whose evaluation failed."""
+        _, _, _, (mu, var) = self.eval_loo(grad=False, active=active, mu_var=True)
+        return mu + np.stack(self._means([g.x for g in self.gps])), var
+
     def eval_device(self, theta_ptr, mll_ptr, grad_ptr=None, info_ptr=None, stream=0):
         """gprb_eval_device: theta (B,P) / mll (B,) / grad (B,P) / info (B,) are raw device pointers (ints, e.g.
         ``torch.Tensor.data_ptr()``); no payload crosses PCIe.  Ordered after ``stream`` (a cudaStream_t handle)."""
@@ -724,6 +754,42 @@ def predict_f(gp, Xstar, full_cov=False):
         return gp.predict_f(Xstar, full_cov=full_cov)
     mu, v = _resident(gp).predict_f(Xstar, full_cov=full_cov)
     return mu[gp._slot], v[gp._slot]
+
+
+def _only(gp):
+    """(batch, active mask) for a call that evaluates one GPE alone in its batch's pass."""
+    b = _resident(gp)
+    act = np.zeros(b.B, dtype=np.uint8)
+    act[gp._slot] = 1
+    return b, act
+
+
+def predict_LOO(gp):
+    """``predict_LOO(gp) -> (mu, sigma2)``: leave-one-out predictive mean and variance at the n training inputs of one
+    GPE ((n,), (n,)), or batched ((B,n), (B,n)) for a GPBatch."""
+    if isinstance(gp, GPBatch):
+        return gp.predict_LOO()
+    b, act = _only(gp)
+    mu, var = b.predict_LOO(active=act)
+    return mu[gp._slot], var[gp._slot]
+
+
+def logp_CVLOO(gp):
+    """``logp_CVLOO(gp)``: leave-one-out log predictive probability of one GPE (float), or (B,) for a GPBatch
+    (-Inf where the factorisation failed)."""
+    if isinstance(gp, GPBatch):
+        return gp.eval_loo(grad=False)[0]
+    b, act = _only(gp)
+    return float(b.eval_loo(grad=False, active=act)[0][gp._slot])
+
+
+def dlogpdtheta_CVLOO(gp):
+    """``dlogpdθ_CVLOO(gp)``: gradient of logp_CVLOO with respect to [logNoise; kernel params] (P,), or (B,P) for a
+    GPBatch (NaN rows where the factorisation failed)."""
+    if isinstance(gp, GPBatch):
+        return gp.eval_loo(grad=True)[1]
+    b, act = _only(gp)
+    return b.eval_loo(grad=True, active=act)[1][gp._slot]
 
 
 def rand(gp, Xstar, nsamples=1, Z=None, rng=None):

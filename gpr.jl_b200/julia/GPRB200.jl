@@ -360,6 +360,87 @@ end
 Random.rand(gp::B200GPE, x::AbstractMatrix, n::Int) = Random.rand!(gp, x, Matrix{Float64}(undef, size(x, 2), n))
 Random.rand(gp::B200GPE, x::AbstractMatrix) = vec(Random.rand(gp, x, 1))
 
+# ---- leave-one-out cross-validation (GaussianProcesses crossvalidation.jl: predict_LOO, logp_CVLOO, dlogpdθ_CVLOO) --------
+# The generic methods work from gp.cK (a placeholder here) and gp.alpha (filled on demand): these go to the device.  The
+# GaussianProcesses function is extended where the installed version defines it; otherwise GPRB200 defines and exports
+# its own, so the module loads either way.
+for name in (:predict_LOO, :logp_CVLOO, :dlogpdθ_CVLOO)
+    if isdefined(GaussianProcesses, name)
+        @eval import GaussianProcesses: $name
+    else
+        @eval function $name end
+        @eval export $name
+    end
+end
+
+"""
+    eval_loo!(batch; grad=true, mu_var=false, active=nothing) -> (logp::B, ∇::P×B | nothing, info::B, μ::n×B | nothing, σ²::n×B | nothing)
+
+One evaluation with gradient per active GP (gp.mll / gp.dmll are written back as by update_mll_and_dmll!), then the
+leave-one-out terms on the factorised K.  μ is the LOO mean of y - m(X).  A GP with info < 0 gets logp = -Inf and NaN rows.
+"""
+function eval_loo!(batch::GPBatch; grad::Bool = true, mu_var::Bool = false, active::Union{Nothing,Vector{UInt8}} = nothing)
+    θ = thetas(batch)
+    mll = fill(NaN, batch.B)
+    g = fill(NaN, batch.P, batch.B)
+    logp = fill(NaN, batch.B)
+    gl = grad ? fill(NaN, batch.P, batch.B) : nothing
+    μ = mu_var ? fill(NaN, batch.n, batch.B) : nothing
+    σ2 = mu_var ? fill(NaN, batch.n, batch.B) : nothing
+    info = zeros(Int32, batch.B)
+    GC.@preserve θ mll g logp gl μ σ2 info active begin
+        check(ccall((:gprb_eval_loo, LIB), Cint,
+                    (Ptr{Cvoid}, Ptr{Float64}, Ptr{UInt8}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}),
+                    batch.handle, θ, active === nothing ? C_NULL : pointer(active), mll, g, logp, grad ? pointer(gl) : C_NULL,
+                    mu_var ? pointer(μ) : C_NULL, mu_var ? pointer(σ2) : C_NULL, info))
+    end
+    for (b, gp) in enumerate(batch.gps)
+        (active === nothing || active[b] != 0) || continue
+        gp.mll = mll[b]; gp.target = mll[b]
+        gp.dmll = g[:, b]; gp.dtarget = g[:, b]
+    end
+    batch.cache_key = zeros(0, 0)
+    logp, gl, info, μ, σ2
+end
+
+loo_active(batch::GPBatch, slot::Int) = batch.B == 1 ? nothing : only_active(batch, slot)
+loo_rows(P::Int, noise::Bool, kern::Bool) = vcat(noise ? [1] : Int[], kern ? collect(2:P) : Int[])   # [logNoise; kernel]: means have no parameters
+
+"predict_LOO(batch) -> (μ::n×B, σ²::n×B): leave-one-out predictive mean (m(X) included) and variance at the training inputs."
+function predict_LOO(batch::GPBatch)
+    _, _, _, μ, σ2 = eval_loo!(batch; grad = false, mu_var = true)
+    for (b, gp) in enumerate(batch.gps)
+        gp.mean isa MeanZero && continue
+        μ[:, b] .+= [GaussianProcesses.mean(gp.mean, gp.x[:, i]) for i in 1:batch.n]
+    end
+    μ, σ2
+end
+"logp_CVLOO(batch) -> logp::B (-Inf for a GP whose factorisation failed)."
+logp_CVLOO(batch::GPBatch) = eval_loo!(batch; grad = false)[1]
+"dlogpdθ_CVLOO(batch; noise, domean, kern) -> ∇::rows×B, rows of [logNoise; kernel params] selected by the flags."
+dlogpdθ_CVLOO(batch::GPBatch; noise::Bool = true, domean::Bool = true, kern::Bool = true) =
+    eval_loo!(batch; grad = true)[2][loo_rows(batch.P, noise, kern), :]
+
+function predict_LOO(gp::B200GPE)
+    batch, slot = residence(gp)
+    _, _, info, μ, σ2 = eval_loo!(batch; grad = false, mu_var = true, active = loo_active(batch, slot))
+    info[slot] < 0 && throw(PDMats.PosDefException(Int(info[slot])))
+    mX = gp.mean isa MeanZero ? 0.0 : [GaussianProcesses.mean(gp.mean, gp.x[:, i]) for i in 1:batch.n]
+    μ[:, slot] .+ mX, σ2[:, slot]
+end
+function logp_CVLOO(gp::B200GPE)
+    batch, slot = residence(gp)
+    logp, _, info = eval_loo!(batch; grad = false, active = loo_active(batch, slot))
+    info[slot] < 0 && throw(PDMats.PosDefException(Int(info[slot])))
+    logp[slot]
+end
+function dlogpdθ_CVLOO(gp::B200GPE; noise::Bool = true, domean::Bool = true, kern::Bool = true)
+    batch, slot = residence(gp)
+    _, ∇, info = eval_loo!(batch; grad = true, active = loo_active(batch, slot))
+    info[slot] < 0 && throw(PDMats.PosDefException(Int(info[slot])))
+    ∇[loo_rows(batch.P, noise, kern), slot]
+end
+
 # ---- asynchronous rollout step (two trial groups alternate: device predict of one under the host projectv! of the other) -----
 "Enqueue the mean prediction of GPs gp0:gp1 (1-based, inclusive) at the per-trial state blocks `states` (d × m × trials) on pipeline `slot`."
 function predict_async!(batch::GPBatch, slot::Integer, gp0::Integer, gp1::Integer, states::Array{Float64,3}, G::Integer; var::Bool = false)

@@ -15,6 +15,8 @@
  *       -> gprb_predict
  *   predict_f / predict_y(gp, Xstar; full_cov=true), rand(gp, Xstar, n)   (GaussianProcesses 0.12.4 GP.jl / GPE.jl)
  *       -> gprb_predict_cov, gprb_sample_posterior
+ *   predict_LOO(gp), logp_CVLOO(gp), dlogpdtheta_CVLOO(gp)   (GaussianProcesses 0.12 crossvalidation.jl)
+ *       -> gprb_eval_loo
  *   gp.cK / gp.alpha inspection (parity taps)              -> gprb_get_K / _chol / _alpha / _Kinv
  *
  * Conventions
@@ -210,6 +212,23 @@ int gprb_predict_cov(gprb_batch* batch, int64_t m, const double* Xstar, int64_t 
  *                    state; a GP with info < 0 gets NaN draws and blocks nobody */
 int gprb_sample_posterior(gprb_batch* batch, int64_t m, const double* Xstar, int64_t xstar_stride, const double* mstar,
                           int32_t ns, const double* Z, double* out, int32_t* info);
+
+/* ---- leave-one-out cross-validation (predict_LOO, logp_CVLOO, dlogpdtheta_CVLOO) ---------------------------------- */
+/* Evaluates like gprb_eval with a gradient (same make_posdef! ladder, info codes, active semantics and state reuse; the
+ * resident state afterwards is what gprb_eval(theta, grad) leaves), then the leave-one-out terms of every GP with
+ * info >= 0 (Rasmussen & Williams eqs. 5.10-5.13) on the K that was factorised - noise, eps, jitter and diagonal offset
+ * included.  With d = diag(K^-1), alpha = K^-1 (y - m(X)):
+ *   mll, grad  B, P x B  out, as gprb_eval with a gradient; either may be NULL
+ *   logp_loo   B         out  sum_i 1/2 log d_i - 1/2 alpha_i^2 / d_i - 1/2 log 2pi
+ *   grad_loo   P x B     out  d logp_loo / d theta; NULL = value only (no n^3 stage)
+ *   mu_loo     n x B     out  y_i - m(x_i) - alpha_i / d_i (the caller adds m(X) back), or NULL
+ *   var_loo    n x B     out  1 / d_i, or NULL
+ *   info       B         out
+ * A GP with info < 0 gets logp_loo = -Inf and NaN grad_loo / mu_loo / var_loo and blocks nobody; inactive GPs' outputs
+ * are untouched.  The gradient stage works on groups of GPs with a bounded per-call workspace (about 2 n^2 doubles per
+ * GP of a group, groups of at most 8 GiB, halved while the device cannot hold them). */
+int gprb_eval_loo(gprb_batch* batch, const double* theta, const uint8_t* active, double* mll, double* grad,
+                  double* logp_loo, double* grad_loo, double* mu_loo, double* var_loo, int32_t* info);
 
 /* ---- parity taps (state after the last gprb_eval of GP b) ------------------------------ */
 int gprb_get_K(gprb_batch* batch, int32_t b, double* out /* n x n, symmetric, noise + jitter included */);
