@@ -100,6 +100,7 @@ static void free_batch(gprb_batch* b) {
     cudaFree(w.M); cudaFree(w.W); cudaFree(w.KD); cudaFree(w.vec); cudaFree(w.part); cudaFree(w.mll); cudaFree(w.out); cudaFree(w.skip);
     if (w.skip_host) cudaFreeHost(w.skip_host);
   }
+  cudaFree(b->pg.jac); cudaFree(b->pg.dms);
   if (b->list_host) cudaFreeHost(b->list_host);
   if (b->fail_host) cudaFreeHost(b->fail_host);
   if (b->stage_host) cudaFreeHost(b->stage_host);
@@ -483,7 +484,7 @@ using namespace gprb;
 
 extern "C" {
 
-int gprb_version(void) { return 301; }
+int gprb_version(void) { return 302; }
 const char* gprb_last_error(void) { return g_err.c_str(); }
 
 int gprb_init(gprb_ctx** out, int device) {
@@ -769,7 +770,8 @@ int gprb_batch_create(gprb_ctx* ctx, int32_t B, gprb_dataset* const* ds, const d
         (rc = make_tensor_map(&b->tm_A68, b->A, (uint64_t)b->npad, (uint64_t)b->npad, B, (uint64_t)b->npad, mat, NB / 2 + 4, KT)) ||
         (rc = make_tensor_map(&b->tm_DT132, b->DinvT, NB, (uint64_t)b->J * NB, B, NB, dinv, NB + 4, KT)) ||
         (rc = make_tensor_map(&b->tm_DT68, b->DinvT, NB, (uint64_t)b->J * NB, B, NB, dinv, NB / 2 + 4, KT)) ||
-        (rc = make_tensor_map(&b->tm_D132, b->Dinv, NB, (uint64_t)b->J * NB, B, NB, dinv, NB + 4, KT)))
+        (rc = make_tensor_map(&b->tm_D132, b->Dinv, NB, (uint64_t)b->J * NB, B, NB, dinv, NB + 4, KT)) ||
+        (rc = make_tensor_map(&b->tm_LT, b->Lm, (uint64_t)b->npad, (uint64_t)b->npad, B, (uint64_t)b->npad, mat, KT, NB)))
       break;
     b->nstreams = 4;
     b->rl_max = 24;
@@ -1580,6 +1582,150 @@ int gprb_eval_loo(gprb_batch* b, const double* theta, const uint8_t* active, dou
   if (!grad) { tgrad.resize((size_t)B * b->P); grad = tgrad.data(); }
   if ((rc = download_results(b, mode.data(), inf, nullptr, mll, grad, info))) return rc;
   return loo_stage(b, mode.data(), inf, logp_loo, grad_loo, mu_loo, var_loo);
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------------
+// Predictive gradients (gprb_predict_grad) on prediction slot 0, chunk by chunk (128 test columns).  Per chunk:
+// k_predict_cross on the slot's stream, then per stream group of GPs: the FWD_ROW chain (T = L^-1 K*, when a variance is
+// asked for), k_predict_finish for the group's mu / var (the launches gprb_predict's tiled path issues, so mu and var are
+// bit-identical to it), the BWD_ROW chain (beta = L^-T T in place, only with dvar) and k_predict_jac.
+static int predgrad_enqueue(gprb_batch* b, int64_t m, const double* Xstar, int64_t xstar_stride, const double* mstar,
+                            const double* dmstar, bool want_var, bool want_dvar) {
+  gprb_predict_slot& sl = b->ps[0];
+  gprb_predgrad_ws& w = b->pg;
+  const int B = b->B, J = b->J, count = B, d = b->d;
+  const int64_t npad = b->npad;
+  cudaStream_t* str = b->stream;
+  cudaStream_t st = str[0];
+  const bool want_T = want_var || want_dvar;
+  const size_t nx = (size_t)(xstar_stride ? xstar_stride * (B - 1) + m * d : m * d);
+  const size_t nout = (size_t)count * m, njac = nout * d;
+  int rc;
+  if (!sl.t0) {
+    GPRB_CUDA(cudaEventCreate(&sl.t0));
+    GPRB_CUDA(cudaEventCreate(&sl.t1));
+    GPRB_CUDA(cudaMallocHost((void**)&sl.h_mask, sizeof(int32_t) * B));
+    if ((rc = dev_alloc(&sl.mask, (size_t)B))) return rc;
+  }
+  if ((rc = ensure_dev(&sl.pX, &sl.pX_cap, nx)) || (rc = ensure_dev(&sl.pmu, &sl.pmu_cap, nout)) ||
+      (rc = ensure_dev(&sl.pmupart, &sl.pmupart_cap, (size_t)count * J * PT)) ||
+      (rc = ensure_pinned(&sl.h_in, &sl.h_in_cap, nx + (mstar ? nout : 0))) || (rc = ensure_pinned(&sl.h_out, &sl.h_out_cap, 2 * nout)) ||
+      (rc = ensure_dev(&w.jac, &w.jac_cap, (want_dvar ? 2 : 1) * njac)))
+    return rc;
+  if (mstar && (rc = ensure_dev(&sl.pms, &sl.pms_cap, nout))) return rc;
+  if (dmstar && (rc = ensure_dev(&w.dms, &w.dms_cap, njac))) return rc;
+  if (want_var && (rc = ensure_dev(&sl.pvar, &sl.pvar_cap, nout))) return rc;
+  if (want_T) {
+    if ((rc = ensure_dev(&sl.pT, &sl.pT_cap, (size_t)count * npad * PT))) return rc;
+    if (sl.tm_T_cap != sl.pT_cap) {
+      if ((rc = make_tensor_map(&sl.tm_T68, sl.pT, PT, (uint64_t)npad, sl.pT_cap / ((size_t)npad * PT), PT, (uint64_t)npad * PT,
+                                NB / 2 + 4, KT)))
+        return rc;
+      sl.tm_T_cap = sl.pT_cap;
+    }
+  }
+  for (int i = 0; i < B; ++i) sl.h_mask[i] = b->state_ok[i] ? 0 : 1;
+  memcpy(sl.h_in, Xstar, sizeof(double) * nx);
+  if (mstar) memcpy(sl.h_in + nx, mstar, sizeof(double) * nout);
+  GPRB_CUDA(cudaEventRecord(sl.t0, st));
+  GPRB_CUDA(cudaMemcpyAsync(sl.mask, sl.h_mask, sizeof(int32_t) * B, cudaMemcpyHostToDevice, st));
+  GPRB_CUDA(cudaMemcpyAsync(sl.pX, sl.h_in, sizeof(double) * nx, cudaMemcpyHostToDevice, st));
+  if (mstar) GPRB_CUDA(cudaMemcpyAsync(sl.pms, sl.h_in + nx, sizeof(double) * nout, cudaMemcpyHostToDevice, st));
+  if (dmstar) GPRB_CUDA(cudaMemcpyAsync(w.dms, dmstar, sizeof(double) * njac, cudaMemcpyHostToDevice, st));
+
+  const int nv = (int)((b->n + KT - 1) / KT * KT);
+  const int ns = std::min(4, b->nstreams);
+  const int S = (count >= 8 * ns) ? ns : 1;
+  for (int64_t s0 = 0; s0 < m; s0 += PT) {
+    PredictTileArgs ta{b->Xtptr, b->theta, b->alpha, sl.pX, mstar ? sl.pms : nullptr, want_T ? sl.pT : nullptr, sl.pmupart,
+                       sl.pmu, want_var ? sl.pvar : nullptr, xstar_stride, (int)b->n, (int)npad, d, J, (int)m, b->kind,
+                       (int)s0, (int)std::min<int64_t>(PT, m - s0)};
+    ta.gp_off = 0;
+    ta.mask = sl.mask;
+    if ((rc = launch_predict_cross(ta, count, st))) return rc;
+    b->ctx->launches++;
+    GemmArgs ga{b->Lm, b->DinvT, b->Dinv, nullptr, b->Lm, b->KinvD, nullptr, npad * npad, (int64_t)J * NB * NB,
+                (int)npad, J, 0, GEMM_FWD_ROW, nv};
+    ga.Tm = sl.pT; ga.t_stride = npad * PT; ga.ldt = PT; ga.t_gp_off = 0;
+    set_gemm_maps(ga, b);
+    ga.tm_T68 = sl.tm_T68;
+    ga.tm_LT = b->tm_LT;
+    ga.ncols = ta.mc;
+    ga.fail = sl.mask;
+    ga.colw = (int64_t)count * ((ta.mc + 63) / 64) >= b->ctx->sm_count ? 64 : 32;
+    const int ntl = (ta.mc + ga.colw - 1) / ga.colw;
+    if (S > 1) GPRB_CUDA(cudaEventRecord(b->join[0], st));
+    for (int s = 0; s < S; ++s) {
+      const int g0 = (int)((int64_t)count * s / S), g1 = (int)((int64_t)count * (s + 1) / S);
+      cudaStream_t ss = str[s];
+      if (s > 0) GPRB_CUDA(cudaStreamWaitEvent(ss, b->join[0], 0));
+      ga.gp_off = g0;
+      if (want_T) {
+        ga.mode = GEMM_FWD_ROW;
+        for (int i = 0; i < J; ++i) {
+          ga.step = i;
+          if ((rc = launch_tile_gemm(ga, ntl, g1 - g0, ss))) return rc;
+          b->ctx->launches++;
+        }
+      }
+      // the group's mu / var: k_predict_finish indexes its outputs and T by blockIdx, so the group's GPs start at g0
+      PredictTileArgs tg = ta;
+      tg.gp_off = g0;
+      if (tg.T) tg.T += (size_t)g0 * npad * PT;
+      tg.mupart += (size_t)g0 * J * PT;
+      tg.mu += (size_t)g0 * m;
+      if (tg.var) tg.var += (size_t)g0 * m;
+      if (tg.mstar) tg.mstar += (size_t)g0 * m;
+      if ((rc = launch_predict_finish(tg, g1 - g0, ss))) return rc;
+      b->ctx->launches++;
+      if (want_dvar) {
+        ga.mode = GEMM_BWD_ROW;
+        for (int i = J - 1; i >= 0; --i) {
+          ga.step = i;
+          if ((rc = launch_tile_gemm(ga, ntl, g1 - g0, ss))) return rc;
+          b->ctx->launches++;
+        }
+      }
+      PredictJacArgs ja{b->Xtptr, b->theta, b->alpha, want_dvar ? sl.pT + (size_t)g0 * npad * PT : nullptr,
+                        sl.pX + (size_t)g0 * xstar_stride, dmstar ? w.dms + (size_t)g0 * m * d : nullptr,
+                        w.jac + (size_t)g0 * m * d, want_dvar ? w.jac + njac + (size_t)g0 * m * d : nullptr, sl.mask,
+                        xstar_stride, (int)b->n, (int)npad, d, (int)m, b->kind, (int)s0, ta.mc, g0};
+      if ((rc = launch_predict_jac(ja, g1 - g0, ss))) return rc;
+      b->ctx->launches++;
+      if (s > 0) {
+        GPRB_CUDA(cudaEventRecord(b->join[s], ss));
+        GPRB_CUDA(cudaStreamWaitEvent(st, b->join[s], 0));
+      }
+    }
+  }
+  GPRB_CUDA(cudaMemcpyAsync(sl.h_out, sl.pmu, sizeof(double) * nout, cudaMemcpyDeviceToHost, st));
+  if (want_var) GPRB_CUDA(cudaMemcpyAsync(sl.h_out + nout, sl.pvar, sizeof(double) * nout, cudaMemcpyDeviceToHost, st));
+  GPRB_CUDA(cudaEventRecord(sl.t1, st));
+  return 0;
+}
+
+extern "C" {
+
+int gprb_predict_grad(gprb_batch* b, int64_t m, const double* Xstar, int64_t xstar_stride, const double* mstar,
+                      const double* dmstar, double* mu, double* var, double* dmu, double* dvar) {
+  GPRB_REQUIRE(b && mu && dmu, "gprb_predict_grad: NULL argument");
+  int rc = predict_check(b, 0, 0, b->B, m, Xstar, xstar_stride);
+  if (rc) return rc;
+  GPRB_CUDA(cudaSetDevice(b->ctx->device));
+  if ((rc = predgrad_enqueue(b, m, Xstar, xstar_stride, mstar, dmstar, var != nullptr, dvar != nullptr))) return rc;
+  gprb_predict_slot& sl = b->ps[0];
+  cudaStream_t st = b->stream[0];
+  const size_t nout = (size_t)b->B * m, njac = nout * b->d;
+  // the Jacobians go straight to the caller's memory, after t1: the device time does not include their copy
+  GPRB_CUDA(cudaMemcpyAsync(dmu, b->pg.jac, sizeof(double) * njac, cudaMemcpyDeviceToHost, st));
+  if (dvar) GPRB_CUDA(cudaMemcpyAsync(dvar, b->pg.jac + njac, sizeof(double) * njac, cudaMemcpyDeviceToHost, st));
+  GPRB_CUDA(cudaStreamSynchronize(st));
+  if ((rc = postcov_finish_time(b))) return rc;
+  memcpy(mu, sl.h_out, sizeof(double) * nout);
+  if (var) memcpy(var, sl.h_out + nout, sizeof(double) * nout);
+  return GPRB_OK;
 }
 
 }  // extern "C"

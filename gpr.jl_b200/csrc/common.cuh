@@ -151,6 +151,14 @@ struct gprb_loo_ws {
   size_t out_cap = 0;
 };
 
+// Workspace of gprb_predict_grad (allocated on first use, grow-only; slot 0's streams, staging, T block and events run the
+// call).  Only the outputs grow with m: the right-hand sides are one 128-column chunk per GP (the slot's pT).
+struct gprb_predgrad_ws {
+  double* jac = nullptr;    // [2][B][m][d] dmu | dvar
+  double* dms = nullptr;    // [B][m][d] prior-mean Jacobian
+  size_t jac_cap = 0, dms_cap = 0;
+};
+
 // Per-GP device state (structure-of-arrays over the batch), all resident in HBM:
 //   A   [B][npad*npad]  K in the lower tiles (kept); after the inverse stage the strictly-upper tile (j,i) holds the
 //                       K^-1 tile (i,j) un-transposed, and KinvD the diagonal tiles of K^-1
@@ -209,11 +217,13 @@ struct gprb_batch {
   gprb_predict_slot ps[2];
   gprb_postcov_ws pc;             // full covariance / posterior draws (gprb_predict_cov, gprb_sample_posterior)
   gprb_loo_ws loo;                // leave-one-out cross-validation (gprb_eval_loo)
+  gprb_predgrad_ws pg;            // predictive gradients (gprb_predict_grad)
   // TMA tensor maps of the tile GEMM's operands (encoded once per batch; box = padded rows x KT columns x 1 GP)
   CUtensorMap tm_L132, tm_L68;     // Lm  [B][npad][npad]
   CUtensorMap tm_A68;              // A   [B][npad][npad] (L2 prefetch of the K tiles the Cholesky modes start from)
   CUtensorMap tm_DT132, tm_DT68;   // DinvT [B][J*128][128]
   CUtensorMap tm_D132;             // Dinv  [B][J*128][128]
+  CUtensorMap tm_LT;               // Lm with box = KT rows x 128 columns (GEMM_BWD_ROW reads L's lower tiles transposed)
   std::vector<cudaEvent_t> gemm_ev;  // profiling: start/stop pairs around every tile-GEMM launch
   int gemm_ev_used = 0;
   std::vector<double> gemm_ms;  // per tile-GEMM launch time of the last profiled evaluation, launch order

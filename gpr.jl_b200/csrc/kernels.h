@@ -7,7 +7,8 @@
 namespace gprb {
 
 enum { GEMM_CHOL_DIAG = 0, GEMM_CHOL_COL = 1, GEMM_TRTRI_ROW = 2, GEMM_LAUUM = 3, GEMM_FWD_ROW = 4,
-       GEMM_CHOL_PANEL = 5, GEMM_CHOL_TRAIL = 6 };  // right-looking Cholesky for small batches (latency-bound chains)
+       GEMM_CHOL_PANEL = 5, GEMM_CHOL_TRAIL = 6,   // right-looking Cholesky for small batches (latency-bound chains)
+       GEMM_BWD_ROW = 7 };                         // backward substitution L^-T T of the predictive gradient (k_tile_bwd)
 
 struct GemmArgs {
   const double* Lm;     // operand matrices [B][npad*npad]
@@ -34,6 +35,7 @@ struct GemmArgs {
   // TMA tensor maps of the operands (gprb_batch / gprb_predict_slot own them): box = 132 or 68 padded rows x KT columns
   CUtensorMap tm_L132, tm_L68, tm_DT132, tm_DT68, tm_D132, tm_T68, tm_A68;
   int pf_cin = 0;       // 1: Cin is the matrix tm_A68 describes - the CTA prefetches its K half tile into L2 with TMA requests at entry
+  CUtensorMap tm_LT;    // GEMM_BWD_ROW only: Lm with box = KT rows x NB columns (L(k, i)^T lands row-major)
 };
 
 int launch_tile_gemm(const GemmArgs& g, int ntiles, int count, cudaStream_t stream);
@@ -159,6 +161,26 @@ struct PredictTileArgs {
 };
 int launch_predict_cross(const PredictTileArgs& a, int count, cudaStream_t stream);
 int launch_predict_finish(const PredictTileArgs& a, int count, cudaStream_t stream);
+
+// Predictive gradients (predgrad.cu): dmu / dx* = dm(x*) + sum_i alpha_i dk(x*, x_i) / dx* and
+// dvar / dx* = -2 sum_i beta_i dk(x*, x_i) / dx*, beta = L^-T L^-1 K* (the T block after the FWD_ROW and BWD_ROW chains),
+// for one chunk of <= PT test columns.  One CTA per GP; blockIdx.x = gp - gp_off like k_predict_finish.
+struct PredictJacArgs {
+  const double* const* Xt;  // [B] transposed training inputs Xt[d][npad]
+  const double* theta;
+  const double* alpha;
+  const double* beta;       // [count][npad][PT] or nullptr (mean only)
+  const double* Xstar;      // d x m (+ local gp * xstar_stride)
+  const double* dmstar;     // [count][m][d] or nullptr
+  double* dmu;              // [count][m][d]
+  double* dvar;             // [count][m][d] or nullptr
+  const int32_t* mask;      // [B]
+  int64_t xstar_stride;
+  int n, npad, d, m, kind;
+  int s0, mc;               // chunk: test columns s0 .. s0 + mc
+  int gp_off;
+};
+int launch_predict_jac(const PredictJacArgs& a, int count, cudaStream_t stream);
 
 // Full posterior covariance (postcov.cu): Sigma = K** - T'T (+ exp(2 logNoise) I) from the solved right-hand sides
 // T = L^-1 K* of every 128-column chunk, one CTA per lower 128 x 128 tile of Sigma and GP, both triangles written.

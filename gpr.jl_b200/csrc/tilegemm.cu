@@ -37,6 +37,9 @@
 //               index)
 //   FWD_ROW    T(i,:)   = inv(L_ii) * [T(i,:) - sum_{k<i} L(i,k) T(k,:)]   in place in the right-hand-side block
 //              (blocked forward substitution L^-1 K* of the predictive variance, PDMats whiten!), i = step
+//   BWD_ROW    B(i,:)   = inv(L_ii)^T [T(i,:) - sum_{k>i} L(k,i)^T B(k,:)]   in place, i = step = J-1 .. 0
+//              (blocked backward substitution L^-T (L^-1 K*) of the predictive gradient; its own kernel, k_tile_bwd: the
+//               A operand is L's lower tiles read transposed through tm_LT, the post-multiplier inv(L_ii)^T comes from DinvT)
 // where V = L^-T lives in the strictly-upper tiles of Lm and its diagonal blocks in DinvT.
 // The per-element summation order is that of the full-tile kernel of round 1 (k-blocks ascending, 4 k per DMMA), so
 // results are unchanged bit for bit and both Cholesky schedules stay bit-identical to each other.
@@ -118,16 +121,17 @@ enum { SEL_FULL = 0, SEL_SKIP, SEL_MI2, SEL_NI1, SEL_NI2, SEL_NI3, SEL_TRI0, SEL
 
 // One k-chunk (KT = 16) of a warp's 64x32 register tile restricted, at compile time, to the 8x8 blocks
 // (mi, ni) with MI_LO <= mi < MI_LIM, NI_LO <= ni < NI_LIM and mi >= ni + OFF: straight-line unpredicated DMMAs.
-// LDA / LDB: smem row strides of the two k-major operand chunks.
-template <int LDA, int LDB, int MI_LIM, int NI_LIM, int OFF, int MI_LO = 0, int NI_LO = 0>
+// LDA / LDB: smem row strides of the two k-major operand chunks.  AK / AM: k and row strides of the A operand (k-major:
+// LDA and 1; the row-major A chunk of BWD_ROW: 1 and KT).
+template <int LDA, int LDB, int MI_LIM, int NI_LIM, int OFF, int MI_LO = 0, int NI_LO = 0, int AK = LDA, int AM = 1>
 __device__ __forceinline__ void chunk_mma(double (&acc)[MI_N][4][2], const double* ap, const double* bp) {
   // ap / bp: this lane's fragment pointers at k4 = 0, i.e. base + t * LD + row0 (resp. col0)
 #pragma unroll
-  for (int k4 = 0; k4 < KT / 4; ++k4, ap += 4 * LDA, bp += 4 * LDB) {
+  for (int k4 = 0; k4 < KT / 4; ++k4, ap += 4 * AK, bp += 4 * LDB) {
     double a[MI_N], b[4];
 #pragma unroll
     for (int mi = MI_LO; mi < MI_LIM; ++mi)
-      if (mi >= OFF) a[mi] = ap[mi * 8];
+      if (mi >= OFF) a[mi] = ap[mi * 8 * AM];
 #pragma unroll
     for (int ni = NI_LO; ni < NI_LIM; ++ni)
       if (ni + OFF <= MI_N - 1) b[ni] = bp[ni * 8];
@@ -140,19 +144,19 @@ __device__ __forceinline__ void chunk_mma(double (&acc)[MI_N][4][2], const doubl
 }
 
 // Dispatch one chunk to the specialised body `sel` (warp-uniform).
-template <int LDA, int LDB>
+template <int LDA, int LDB, int AK = LDA, int AM = 1>
 __device__ __forceinline__ void chunk_dispatch(int sel, double (&acc)[MI_N][4][2], const double* ap, const double* bp) {
   switch (sel) {
     case SEL_SKIP: break;
-    case SEL_MI2: chunk_mma<LDA, LDB, 2, 4, -64>(acc, ap, bp); break;
-    case SEL_NI1: chunk_mma<LDA, LDB, MI_N, 1, -64>(acc, ap, bp); break;
-    case SEL_NI2: chunk_mma<LDA, LDB, MI_N, 2, -64>(acc, ap, bp); break;
-    case SEL_NI3: chunk_mma<LDA, LDB, MI_N, 3, -64>(acc, ap, bp); break;
-    case SEL_TRI0: chunk_mma<LDA, LDB, MI_N, 4, 0>(acc, ap, bp); break;
-    case SEL_MLO2: chunk_mma<LDA, LDB, MI_N, 4, -64, 2>(acc, ap, bp); break;
-    case SEL_MLO2_NI3: chunk_mma<LDA, LDB, MI_N, 3, -64, 2>(acc, ap, bp); break;
-    case SEL_NLO2: chunk_mma<LDA, LDB, MI_N, 4, -64, 0, 2>(acc, ap, bp); break;
-    default: chunk_mma<LDA, LDB, MI_N, 4, -64>(acc, ap, bp); break;
+    case SEL_MI2: chunk_mma<LDA, LDB, 2, 4, -64, 0, 0, AK, AM>(acc, ap, bp); break;
+    case SEL_NI1: chunk_mma<LDA, LDB, MI_N, 1, -64, 0, 0, AK, AM>(acc, ap, bp); break;
+    case SEL_NI2: chunk_mma<LDA, LDB, MI_N, 2, -64, 0, 0, AK, AM>(acc, ap, bp); break;
+    case SEL_NI3: chunk_mma<LDA, LDB, MI_N, 3, -64, 0, 0, AK, AM>(acc, ap, bp); break;
+    case SEL_TRI0: chunk_mma<LDA, LDB, MI_N, 4, 0, 0, 0, AK, AM>(acc, ap, bp); break;
+    case SEL_MLO2: chunk_mma<LDA, LDB, MI_N, 4, -64, 2, 0, AK, AM>(acc, ap, bp); break;
+    case SEL_MLO2_NI3: chunk_mma<LDA, LDB, MI_N, 3, -64, 2, 0, AK, AM>(acc, ap, bp); break;
+    case SEL_NLO2: chunk_mma<LDA, LDB, MI_N, 4, -64, 0, 2, AK, AM>(acc, ap, bp); break;
+    default: chunk_mma<LDA, LDB, MI_N, 4, -64, 0, 0, AK, AM>(acc, ap, bp); break;
   }
 }
 
@@ -172,7 +176,8 @@ struct HalfGeom {
 
 // Consumer side of one half tile (warps 0-3).  RAGGED = the tile touches the padded tail of the last block row:
 // only then are the DMMAs / loads / stores predicated per 8-row slab (mi < mi_valid); full tiles run the clean loop.
-template <bool COLSPLIT, bool RAGGED>
+// BWD = the BWD_ROW tiles of k_tile_bwd (COLSPLIT, laid out like FWD_ROW); false compiles exactly the code of k_tile_gemm.
+template <bool COLSPLIT, bool RAGGED, bool BWD = false>
 __device__ __forceinline__ void consume_tile(const GemmArgs& g, const TileCoord& tc, const HalfGeom& hg, double* stages,
                                              double* rbuf, uint64_t* full, uint64_t* empty, uint64_t* rfull, uint64_t* rempty,
                                              int gp, int nchunks, int rows_valid) {
@@ -189,7 +194,7 @@ __device__ __forceinline__ void consume_tile(const GemmArgs& g, const TileCoord&
   const int wn = COLSPLIT ? (warp & 1) : (warp & 3);
   const int r0t = hg.r0h + wm * WROWS;       // tile-relative row of the warp tile's first row
   const int gq = lane >> 2, t = lane & 3;
-  const bool fwd = g.mode == GEMM_FWD_ROW;
+  const bool fwd = BWD || g.mode == GEMM_FWD_ROW;
   // Column layout.  Default: column group wn owns the four 8-column blocks at 32 wn.  FWD_ROW tiles with fewer than 64
   // valid test columns (the reference predicts m = 100 test states per step: 64 + 36; narrow 32-column tiles when a
   // launch would otherwise have too few CTAs) use a compact layout: the nblk = ceil(ncols / 8) valid 8-column blocks are
@@ -225,15 +230,20 @@ __device__ __forceinline__ void consume_tile(const GemmArgs& g, const TileCoord&
     if (kb == tc.b_diag_kb) { mb = mapB_D; rb = hg.c0h; }
     else if (fwd) { mb = &g.tm_T68; rb = hg.gcol_off; gb = gp - g.t_gp_off; }
     else { mb = mapB_L; rb = tc.j * NB + hg.c0h; }
-    mbar_expect_tx(&full[stage], STAGE_DOUBLES * sizeof(double));
     double* dst = stages + stage * STAGE_DOUBLES;
-    tma_load_3d(dst, ma, ra, kc, gp, &full[stage]);
+    if (BWD) {  // A = L(k rows, i columns)^T: the box of KT rows x NB columns lands row-major, [column][KT]
+      mbar_expect_tx(&full[stage], (KT * NB + KT * LDB) * sizeof(double));
+      tma_load_3d(dst, &g.tm_LT, kc, tc.i * NB, gp, &full[stage]);
+    } else {
+      mbar_expect_tx(&full[stage], STAGE_DOUBLES * sizeof(double));
+      tma_load_3d(dst, ma, ra, kc, gp, &full[stage]);
+    }
     tma_load_3d(dst + KT * LDA, mb, rb, kc, gb, &full[stage]);
   };
   auto issue_r = [&](int c) {  // chunk c of the post-multiplier inv(L_rblk) -> rbuf[c % NRBUF]
     const int buf = c % NRBUF;
     mbar_expect_tx(&rfull[buf], RBUF_DOUBLES * sizeof(double));
-    tma_load_3d(rbuf + buf * RBUF_DOUBLES, &g.tm_D132, 0, tc.rblk * NB + c * KT, gp, &rfull[buf]);
+    tma_load_3d(rbuf + buf * RBUF_DOUBLES, BWD ? &g.tm_DT132 : &g.tm_D132, 0, tc.rblk * NB + c * KT, gp, &rfull[buf]);
   };
   if (warp == 0 && lane == 0) {  // prologue: fill the ring, start the post-multiplier
     for (int c = 0; c < min(NSTAGE, nchunks); ++c) issue_main(c);
@@ -314,7 +324,8 @@ __device__ __forceinline__ void consume_tile(const GemmArgs& g, const TileCoord&
           sel = nl <= 0 ? SEL_SKIP : nl == 2 ? SEL_NI2 : SEL_FULL;
         } else sel = sel_tri;
       } else if (lsym) sel = sel_tri;
-      chunk_dispatch<LDA, LDB>(sel, acc, As + t * LDA + row0, As + KT * LDA + t * LDB + col0);
+      if (BWD) chunk_dispatch<LDA, LDB, 1, KT>(sel, acc, As + row0 * KT + t, As + KT * LDA + t * LDB + col0);
+      else chunk_dispatch<LDA, LDB>(sel, acc, As + t * LDA + row0, As + KT * LDA + t * LDB + col0);
       __syncwarp();
       if (lane == 0) mbar_arrive(&empty[stage]);
       if (warp == 0 && c + NSTAGE < nchunks) {  // refill: every consumer warp has released this stage
@@ -389,11 +400,19 @@ __device__ __forceinline__ void consume_tile(const GemmArgs& g, const TileCoord&
 
   // Dinv is lower triangular: R[x][k] == 0 for k > x.  post 1: x = output column, post 2: x = output row
   // (tile-relative; the post-multiplier chunk c covers k = 16c .. 16c + 15 of the whole tile).
-  const int kmax = (tc.post == 1) ? (c0t + 31) : min(r0t + WROWS - 1, rows_valid - 1);
+  // BWD: R = DinvT is upper triangular, R[x][k] == 0 for k < x: chunk c only meets the rows x <= 16c + 15.
+  const int kmax = (tc.post == 1) ? (c0t + 31) : BWD ? rows_valid - 1 : min(r0t + WROWS - 1, rows_valid - 1);
   for (int c = 0; c < NB / KT; ++c) {
     const int buf = c % NRBUF;
     mbar_wait(&rfull[buf], (c / NRBUF) & 1);
-    if (c * KT <= kmax) {
+    if (BWD) {
+      if (c * KT <= kmax && c * KT + KT - 1 >= r0t) {
+        const double* Rs = rbuf + buf * RBUF_DOUBLES + t * LDS_T;
+        const double* Tc = Ts + (c * KT + t) * LDT;
+        const int sel = (sel_plain == SEL_FULL && 2 * c == r0t / 8) ? SEL_MI2 : sel_plain;  // rows r0t + 16 .. lie below chunk c
+        chunk_dispatch<LDA, LDB>(sel, acc, Rs + r0t + gq, Tc + col0);
+      }
+    } else if (c * KT <= kmax) {
       const double* Rs = rbuf + buf * RBUF_DOUBLES + t * LDS_T;
       const double* Tc = Ts + (c * KT + t) * LDT;
       // triangular skip inside the warp tile: chunk c only meets output columns (post 1) / rows (post 2) x >= 16 c
@@ -444,9 +463,10 @@ __device__ __forceinline__ void consume_tile(const GemmArgs& g, const TileCoord&
   GPRB_TL(6);
 }
 
-// COLSPLIT = false: 64 x 128 halves (CHOL_*, LAUUM); true: 128 x 64 halves (TRTRI_ROW) / <= 64-column tiles (FWD_ROW).
-template <bool COLSPLIT>
-__global__ void __launch_bounds__(GEMM_THREADS, 2) k_tile_gemm(const __grid_constant__ GemmArgs g) {
+// COLSPLIT = false: 64 x 128 halves (CHOL_*, LAUUM); true: 128 x 64 halves (TRTRI_ROW) / <= 64-column tiles (FWD_ROW,
+// BWD_ROW).
+template <bool COLSPLIT, bool BWD>
+__device__ __forceinline__ void tile_gemm_body(const GemmArgs& g) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   double* stages = reinterpret_cast<double*>(smem_raw);
   double* rbuf = stages + NSTAGE * STAGE_DOUBLES;
@@ -463,10 +483,16 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) k_tile_gemm(const __grid_cons
   // A GP whose factorisation already hit a non-positive pivot (make_posdef! will retry it with more jitter) skips the
   // rest of the failed attempt, like dpotrf stopping at the failing column.  The load overlaps the setup below.
   const int failed = g.fail ? g.fail[gp] : 0;
-  const bool fwd = g.mode == GEMM_FWD_ROW;
-  // blockIdx.x: (tile, half) for every mode but FWD_ROW, whose tiles are already <= 64 columns wide
+  const bool fwd = BWD || g.mode == GEMM_FWD_ROW;
+  // blockIdx.x: (tile, half) for every mode but FWD_ROW / BWD_ROW, whose tiles are already <= 64 columns wide
   const int half = fwd ? 0 : (int)(blockIdx.x & 1);
-  const TileCoord tc = tile_coord(g.mode, g.step, g.J, fwd ? (int)blockIdx.x : (int)(blockIdx.x >> 1));
+  TileCoord tc;
+  if (BWD) {
+    tc.i = g.step; tc.j = blockIdx.x; tc.kb0 = g.step + 1; tc.kb1 = g.J; tc.a_diag_kb = tc.b_diag_kb = -1;
+    tc.use_cin = true; tc.post = 2; tc.rblk = g.step;
+  } else {
+    tc = tile_coord(g.mode, g.step, g.J, fwd ? (int)blockIdx.x : (int)(blockIdx.x >> 1));
+  }
   HalfGeom hg;
   hg.r0h = COLSPLIT ? 0 : half * HB;
   hg.c0h = COLSPLIT ? (fwd ? 0 : half * HB) : 0;
@@ -499,8 +525,19 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) k_tile_gemm(const __grid_cons
   // RAGGED whenever the warp tiles of this half do not all have 64 valid rows
   const int rows_here = rows_valid - hg.r0h;  // valid rows from the half's first row on (ROWSPLIT: up to 64 matter)
   const bool ragged = COLSPLIT ? (rows_valid < NB) : (rows_here < HB);
-  if (!ragged) consume_tile<COLSPLIT, false>(g, tc, hg, stages, rbuf, full, empty, rfull, rempty, gp, nchunks, rows_valid);
-  else consume_tile<COLSPLIT, true>(g, tc, hg, stages, rbuf, full, empty, rfull, rempty, gp, nchunks, rows_valid);
+  if (!ragged) consume_tile<COLSPLIT, false, BWD>(g, tc, hg, stages, rbuf, full, empty, rfull, rempty, gp, nchunks, rows_valid);
+  else consume_tile<COLSPLIT, true, BWD>(g, tc, hg, stages, rbuf, full, empty, rfull, rempty, gp, nchunks, rows_valid);
+}
+
+template <bool COLSPLIT>
+__global__ void __launch_bounds__(GEMM_THREADS, 2) k_tile_gemm(const __grid_constant__ GemmArgs g) {
+  tile_gemm_body<COLSPLIT, false>(g);
+}
+
+// GEMM_BWD_ROW tiles (the backward block substitution of the predictive gradient), a kernel of their own so that the
+// modes of k_tile_gemm keep their code.
+__global__ void __launch_bounds__(GEMM_THREADS, 2) k_tile_bwd(const __grid_constant__ GemmArgs g) {
+  tile_gemm_body<true, true>(g);
 }
 
 // The dynamic shared-memory opt-in is a per-device function attribute: gprb_init calls this for the device of every
@@ -510,21 +547,25 @@ int configure_tile_gemm() {
   if (e == cudaSuccess) e = cudaFuncSetAttribute(k_tile_gemm<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GEMM_SMEM);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(k_tile_gemm<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(k_tile_gemm<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_tile_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GEMM_SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_tile_bwd, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(k_tile_gemm)", __FILE__, __LINE__);
   return 0;
 }
 
-// ntiles = logical tiles of the launch: 128x128 tiles for every mode but FWD_ROW (each becomes two CTAs), column tiles of
-// g.colw <= 64 test columns for FWD_ROW (one CTA each).
+// ntiles = logical tiles of the launch: 128x128 tiles for every mode but FWD_ROW / BWD_ROW (each becomes two CTAs), column
+// tiles of g.colw <= 64 test columns for FWD_ROW / BWD_ROW (one CTA each).
 int launch_tile_gemm(const GemmArgs& g, int ntiles, int count, cudaStream_t stream) {
   if (ntiles <= 0 || count <= 0) return 0;
   const bool colsplit = g.mode == GEMM_TRTRI_ROW || g.mode == GEMM_FWD_ROW;
-  if (g.mode == GEMM_FWD_ROW && (g.colw > HB || g.colw < 8 || (g.colw & 7))) {
-    set_error("k_tile_gemm: FWD_ROW tiles are at most 64 columns wide");
+  const bool rhs = g.mode == GEMM_FWD_ROW || g.mode == GEMM_BWD_ROW;
+  if (rhs && (g.colw > HB || g.colw < 8 || (g.colw & 7))) {
+    set_error("k_tile_gemm: FWD_ROW / BWD_ROW tiles are at most 64 columns wide");
     return GPRB_ERR_ARG;
   }
-  dim3 grid(g.mode == GEMM_FWD_ROW ? ntiles : 2 * ntiles, count);
-  if (colsplit) k_tile_gemm<true><<<grid, GEMM_THREADS, GEMM_SMEM, stream>>>(g);
+  dim3 grid(rhs ? ntiles : 2 * ntiles, count);
+  if (g.mode == GEMM_BWD_ROW) k_tile_bwd<<<grid, GEMM_THREADS, GEMM_SMEM, stream>>>(g);
+  else if (colsplit) k_tile_gemm<true><<<grid, GEMM_THREADS, GEMM_SMEM, stream>>>(g);
   else k_tile_gemm<false><<<grid, GEMM_THREADS, GEMM_SMEM, stream>>>(g);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return cuda_fail(e, "k_tile_gemm launch", __FILE__, __LINE__);

@@ -101,6 +101,9 @@ class MeanFunction:
     def mean_matrix(self, X):  # X: d x n  ->  [mean(m, X[:, i]) for i]
         return np.array([self.mean(X[:, i]) for i in range(X.shape[1])], dtype=np.float64)
 
+    def jacobian(self, x):  # x: one sample (d,)  ->  d m(x) / dx, (d,); needed by predict_grad
+        raise NotImplementedError(f"{type(self).__name__} has no jacobian(x)")
+
 
 class MeanZero(MeanFunction):
     def mean(self, x):
@@ -623,6 +626,32 @@ class GPBatch:
                                                           info.ctypes.data_as(C.POINTER(C.c_int32))))
         return out.transpose(0, 2, 1), info
 
+    def predict_grad(self, Xstar, var=True, per_gp=False):
+        """Posterior mean and variance with their Jacobians with respect to the test inputs (gprb_predict_grad)
+        -> (mu (B,m), var (B,m) | None, dmu (B,m,d), dvar (B,m,d) | None); dmu[b, j, p] = d mu_bj / d x*_jp.
+        ``var=False`` computes the mean and its Jacobian only (no triangular substitution).  dvar is the gradient of the
+        unclamped variance K** - k*' K^-1 k* (the same for predict_f and predict_y; the floor at 0 is not differentiated).
+        A prior mean other than MeanZero must implement ``jacobian(x)``."""
+        for g in self.gps:
+            if not isinstance(g.mean, MeanZero) and type(g.mean).jacobian is MeanFunction.jacobian:
+                raise NotImplementedError(f"predict_grad: the prior mean {type(g.mean).__name__} has no jacobian(x)")
+        Xs, stride, m, mstar = self._test_block(Xstar, per_gp)
+        dmstar = None
+        if mstar is not None:
+            blocks = [np.asarray(x, dtype=np.float64) for x in Xstar] if per_gp else [Xs.T] * self.B
+            dmstar = np.zeros((self.B, m, self.d))
+            for b, g in enumerate(self.gps):
+                if not isinstance(g.mean, MeanZero):
+                    for s in range(m):
+                        dmstar[b, s] = g.mean.jacobian(np.ascontiguousarray(blocks[b][:, s]))
+        mu = np.empty((self.B, m))
+        v = np.empty((self.B, m)) if var else None
+        dmu = np.empty((self.B, m, self.d))
+        dv = np.empty((self.B, m, self.d)) if var else None
+        self.lib.check(self.lib.dll.gprb_predict_grad(self.handle, m, _d(Xs), stride, _d(mstar), _d(dmstar), _d(mu), _d(v),
+                                                      _d(dmu), _d(dv)))
+        return mu, v, dmu, dv
+
     def predict_async(self, slot, gp0, gp1, blocks, var=False, gps_per_block=1):
         """gprb_predict_async: enqueue the prediction of GPs gp0..gp1-1 on pipeline ``slot`` (0 or 1) and return at
         once.  ``blocks``: one d x m array shared by the range, or a sequence of d x m blocks, one per ``gps_per_block``
@@ -762,6 +791,17 @@ def _only(gp):
     act = np.zeros(b.B, dtype=np.uint8)
     act[gp._slot] = 1
     return b, act
+
+
+def predict_grad(gp, Xstar, var=True):
+    """``predict_grad(gp, Xstar) -> (mu (m,), var (m,) | None, dmu (m,d), dvar (m,d) | None)`` for one GPE (d x m test
+    block): the posterior mean and variance with their Jacobians with respect to the test inputs; batched
+    ((B,m), (B,m), (B,m,d), (B,m,d)) for a GPBatch.  See ``GPBatch.predict_grad``."""
+    if isinstance(gp, GPBatch):
+        return gp.predict_grad(Xstar, var=var)
+    mu, v, dmu, dv = _resident(gp).predict_grad(Xstar, var=var)
+    k = gp._slot
+    return mu[k], (v[k] if var else None), dmu[k], (dv[k] if var else None)
 
 
 def predict_LOO(gp):

@@ -441,6 +441,67 @@ function dlogpdθ_CVLOO(gp::B200GPE; noise::Bool = true, domean::Bool = true, ke
     ∇[loo_rows(batch.P, noise, kern), slot]
 end
 
+# ---- predictive gradients: Jacobians of the posterior mean and variance with respect to the test inputs ---------------
+# For the linearisation of a learned one-step map (stability analysis, Σₜ₊₁ = Jₜ Σₜ Jₜᵀ + diag σ²(xₜ), LQR / MPC).  ∂σ² is
+# the gradient of the unclamped K** - K*ᵀK⁻¹K* (the same for σ²_f and σ²_y; predict_f's floor at 0 is not differentiated).
+# A prior mean other than MeanZero needs its Jacobian from the caller (`mean_jacobian`): ForwardDiff cannot pass a ccall.
+for name in (:predict_grad,)
+    if isdefined(GaussianProcesses, name)
+        @eval import GaussianProcesses: $name
+    else
+        @eval function $name end
+        @eval export $name
+    end
+end
+
+"""
+    predict_grad(batch, Xstar::d×m; var=true, mean_jacobian=nothing) -> (μ::m×B, σ²::m×B | nothing, ∂μ::d×m×B, ∂σ²::d×m×B | nothing)
+
+∂μ[p, j, b] = ∂μ_bj/∂x*_pj.  `var=false`: the mean and its Jacobian only (no triangular substitution on the device).
+`mean_jacobian(b, x) -> d-vector` is the Jacobian of GP b's prior mean; required when a GP's mean is not MeanZero.
+GPs without state give NaN columns.
+"""
+function predict_grad(batch::GPBatch, Xstar::AbstractMatrix; var::Bool = true, mean_jacobian = nothing)
+    for gp in batch.gps
+        gp.mean isa MeanZero || mean_jacobian !== nothing ||
+            throw(ArgumentError("predict_grad: the prior mean $(typeof(gp.mean)) needs `mean_jacobian`"))
+    end
+    Xs = Matrix{Float64}(Xstar)
+    d, m = size(Xs)
+    mstar = prior_means(batch, Xs)
+    dmstar = nothing
+    if mstar !== nothing
+        dmstar = zeros(d, m, batch.B)
+        for b in 1:batch.B, j in 1:m
+            batch.gps[b].mean isa MeanZero || (dmstar[:, j, b] .= mean_jacobian(b, Xs[:, j]))
+        end
+    end
+    μ = Matrix{Float64}(undef, m, batch.B)
+    σ2 = var ? Matrix{Float64}(undef, m, batch.B) : nothing
+    ∂μ = Array{Float64,3}(undef, d, m, batch.B)
+    ∂σ2 = var ? Array{Float64,3}(undef, d, m, batch.B) : nothing
+    GC.@preserve Xs mstar dmstar μ σ2 ∂μ ∂σ2 begin
+        check(ccall((:gprb_predict_grad, LIB), Cint,
+                    (Ptr{Cvoid}, Int64, Ptr{Float64}, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+                    batch.handle, m, Xs, 0, mstar === nothing ? C_NULL : pointer(mstar), dmstar === nothing ? C_NULL : pointer(dmstar),
+                    μ, var ? pointer(σ2) : C_NULL, ∂μ, var ? pointer(∂σ2) : C_NULL))
+    end
+    μ, σ2, ∂μ, ∂σ2
+end
+
+"predict_grad(gp, x::d×m; var=true, mean_jacobian=nothing) -> (μ::m, σ²::m, ∂μ::d×m, ∂σ²::d×m); `mean_jacobian(x) -> d-vector`."
+function predict_grad(gp::B200GPE, x::AbstractMatrix; var::Bool = true, mean_jacobian = nothing)
+    gp.mean isa MeanZero || mean_jacobian !== nothing ||
+        throw(ArgumentError("predict_grad: the prior mean $(typeof(gp.mean)) needs `mean_jacobian`"))
+    batch, slot = residence(gp)
+    mj = mean_jacobian === nothing ? nothing : (b, xj) -> b == slot ? mean_jacobian(xj) : zeros(length(xj))
+    if mj === nothing && !all(g -> g.mean isa MeanZero, batch.gps)
+        mj = (b, xj) -> zeros(length(xj))  # the other GPs of the batch: their rows are not returned
+    end
+    μ, σ2, ∂μ, ∂σ2 = predict_grad(batch, x; var = var, mean_jacobian = mj)
+    μ[:, slot], var ? σ2[:, slot] : nothing, ∂μ[:, :, slot], var ? ∂σ2[:, :, slot] : nothing
+end
+
 # ---- asynchronous rollout step (two trial groups alternate: device predict of one under the host projectv! of the other) -----
 "Enqueue the mean prediction of GPs gp0:gp1 (1-based, inclusive) at the per-trial state blocks `states` (d × m × trials) on pipeline `slot`."
 function predict_async!(batch::GPBatch, slot::Integer, gp0::Integer, gp1::Integer, states::Array{Float64,3}, G::Integer; var::Bool = false)

@@ -15,7 +15,7 @@ EXPORTS = [
     "gprb_batch_create", "gprb_batch_set_targets", "gprb_batch_set_diag_offset", "gprb_batch_destroy",
     "gprb_eval", "gprb_eval_mixed", "gprb_eval_device", "gprb_lbfgs_default_opts", "gprb_optimize", "gprb_lbfgs_selftest",
     "gprb_predict", "gprb_predict_async", "gprb_predict_wait", "gprb_last_predict_ms",
-    "gprb_predict_cov", "gprb_sample_posterior", "gprb_eval_loo",
+    "gprb_predict_cov", "gprb_sample_posterior", "gprb_eval_loo", "gprb_predict_grad",
     "gprb_get_K", "gprb_get_chol", "gprb_get_alpha", "gprb_get_Kinv",
     "gprb_comm_unique_id", "gprb_comm_init_rank", "gprb_gather", "gprb_gather_multi",
     "gprb_set_profiling", "gprb_last_stage_ms", "gprb_last_gemm_launch_ms", "gprb_launch_count",
@@ -91,6 +91,7 @@ class Library:
         L.gprb_last_predict_ms.argtypes = [_vp, C.c_int32, _dp]
         L.gprb_predict_cov.argtypes = [_vp, C.c_int64, _dp, C.c_int64, _dp, C.c_int32, _dp, _dp]
         L.gprb_sample_posterior.argtypes = [_vp, C.c_int64, _dp, C.c_int64, _dp, C.c_int32, _dp, _dp, C.POINTER(C.c_int32)]
+        L.gprb_predict_grad.argtypes = [_vp, C.c_int64, _dp, C.c_int64, _dp, _dp, _dp, _dp, _dp, _dp]
         L.gprb_eval_loo.argtypes = [_vp, _dp, C.POINTER(C.c_uint8), _dp, _dp, _dp, _dp, _dp, _dp, C.POINTER(C.c_int32)]
         L.gprb_comm_unique_id.argtypes = [C.c_void_p]
         L.gprb_comm_init_rank.argtypes = [_vp, C.c_int32, C.c_int32, C.c_void_p]

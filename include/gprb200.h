@@ -230,6 +230,25 @@ int gprb_sample_posterior(gprb_batch* batch, int64_t m, const double* Xstar, int
 int gprb_eval_loo(gprb_batch* batch, const double* theta, const uint8_t* active, double* mll, double* grad,
                   double* logp_loo, double* grad_loo, double* mu_loo, double* var_loo, int32_t* info);
 
+/* ---- predictive gradients: Jacobians of the posterior mean and variance with respect to the test inputs -------- */
+/* Synchronous, on prediction slot 0 (refused while slot 0 has an asynchronous prediction in flight), any m >= 1.
+ * Works on any state gprb_predict works on, value-only states included (it needs L, the inverted diagonal blocks and
+ * alpha).  For stationary ARD kernels k = g(r2), dk(x*, x_i) / dx*_p = 2 g'(r2) w_p (x*_p - x_ip), and with
+ * beta = K^-1 K* (K the resident matrix: noise, eps, jitter and diagonal offset included):
+ *   dmu_j  / dx*_jp = dm(x*_j) / dx*_jp + sum_i alpha_i dk(x*_j, x_i) / dx*_jp
+ *   dvar_j / dx*_jp = -2 sum_i beta_ij dk(x*_j, x_i) / dx*_jp
+ * dvar is the gradient of the unclamped K** - T'T: the floor of the variance at 0 is not differentiated, and it is the
+ * same for sigma^2_f and sigma^2_y.
+ *   Xstar, xstar_stride, mstar   as for gprb_predict
+ *   dmstar  d x m x B  in, the prior mean's Jacobian (added like mstar), or NULL for none
+ *   mu, var m x B      out, bit-identical to gprb_predict's tiled path on the same state; var may be NULL
+ *   dmu     d x m x B  out, dmu[p + d*(j + m*b)]
+ *   dvar    d x m x B  out, or NULL: mean only, no triangular substitution runs at all
+ * A GP without an evaluated state gets NaN rows and blocks nobody.  gprb_last_predict_ms(batch, 0) reports the device
+ * time (without the copy of the Jacobians).  The workspace holds one 128-column chunk of right-hand sides per GP. */
+int gprb_predict_grad(gprb_batch* batch, int64_t m, const double* Xstar, int64_t xstar_stride, const double* mstar,
+                      const double* dmstar, double* mu, double* var, double* dmu, double* dvar);
+
 /* ---- parity taps (state after the last gprb_eval of GP b) ------------------------------ */
 int gprb_get_K(gprb_batch* batch, int32_t b, double* out /* n x n, symmetric, noise + jitter included */);
 int gprb_get_chol(gprb_batch* batch, int32_t b, double* out /* n x n upper U with K = U'U, zeros below */);
