@@ -9,6 +9,7 @@
 #include <functional>
 #include <limits>
 #include <new>
+#include <type_traits>
 
 #include "common.cuh"
 #include "kernels.h"
@@ -59,8 +60,28 @@ int make_tensor_map(CUtensorMap* map, const double* base, uint64_t rows, uint64_
   return 0;
 }
 
-static void set_gemm_maps(GemmArgs& ga, const gprb_batch* b) {
-  ga.tm_L132 = b->tm_L132; ga.tm_L68 = b->tm_L68; ga.tm_A68 = b->tm_A68; ga.tm_DT132 = b->tm_DT132; ga.tm_DT68 = b->tm_DT68; ga.tm_D132 = b->tm_D132;
+// Operand tensor maps of the tile GEMM on B factors ga.Lm [B][npad][npad], beside ga.Cin (K) and the inverted diagonal
+// blocks ga.Dinv / ga.DinvT [B][J*128][128]: padded boxes (132 / 68 rows) x KT columns x one GP
+static int encode_factor_maps(GemmArgs& ga, uint64_t B) {
+  const uint64_t np = ga.npad, nd = (uint64_t)ga.J * NB, ms = ga.mat_stride, ds = ga.dinv_stride;
+  int rc;
+  if ((rc = make_tensor_map(&ga.tm_L132, ga.Lm, np, np, B, np, ms, NB + 4, KT)) ||
+      (rc = make_tensor_map(&ga.tm_L68, ga.Lm, np, np, B, np, ms, NB / 2 + 4, KT)) ||
+      (rc = make_tensor_map(&ga.tm_A68, ga.Cin, np, np, B, np, ms, NB / 2 + 4, KT)) ||
+      (rc = make_tensor_map(&ga.tm_DT132, ga.DinvT, NB, nd, B, NB, ds, NB + 4, KT)) ||
+      (rc = make_tensor_map(&ga.tm_DT68, ga.DinvT, NB, nd, B, NB, ds, NB / 2 + 4, KT)) ||
+      (rc = make_tensor_map(&ga.tm_D132, ga.Dinv, NB, nd, B, NB, ds, NB + 4, KT)))
+    return rc;
+  return 0;
+}
+
+// make_posdef! after one factorisation attempt with status f (LAPACK info; < 0: no state or non-finite input): either one
+// more jitter is due (tries counts it, returns true) or info gets the final outcome - the jitter count, -2, or -1 when
+// the matrix is still indefinite after MAX_JITTER jitters.
+static bool posdef_retry(int32_t f, int32_t& tries, int32_t& info) {
+  if (f > 0 && tries < MAX_JITTER) { ++tries; return true; }
+  info = f == 0 ? tries : f < 0 ? -2 : -1;
+  return false;
 }
 
 template <typename T>
@@ -182,9 +203,8 @@ static int enqueue_pipeline(gprb_batch* b, int off, int count, int ngrad, int nr
   };
   if (prof) { b->gemm_ev_used = 0; cudaEventRecord(b->ev[0], st); }
   const int nv = (int)((b->n + KT - 1) / KT * KT);
-  GemmArgs ga{b->Lm, b->DinvT, b->Dinv, b->A, b->Lm, b->KinvD, list, ms, dstride, (int)b->npad, J, 0, GEMM_CHOL_DIAG, nv};
-  ga.fail = b->fail;
-  set_gemm_maps(ga, b);
+  GemmArgs ga = b->gemm;
+  ga.list = list;
   { static const int pf = getenv("GPRB200_PF_CIN") ? atoi(getenv("GPRB200_PF_CIN")) : 1; ga.pf_cin = (!right_looking && pf) ? 1 : 0; }
   if (count > 0) {
   // Small passes are latency bound (one dependent chain of 3 J launches): they use the right-looking factorisation,
@@ -388,12 +408,11 @@ static int eval_pass(gprb_batch* b, const double* theta_host, const uint8_t* mod
   for (int gp : reuse_gps) { info[gp] = b->info_last[gp]; b->inv_ok[gp] = 1; b->v_ok[gp] = 1; }
   for (int pass = 0; pass < 2; ++pass)
     for (int gp : (pass == 0 ? grad_gps : val_gps)) {
-      const int f = b->fail_host[gp];
       b->theta_valid[gp] = 0;
-      if (f == 0) info[gp] = b->tries[gp];
-      else if (f < 0) info[gp] = -2;
-      else if (b->tries[gp] >= MAX_JITTER) info[gp] = -1;
-      else { b->tries[gp]++; pending[gp] = 1; b->state_ok[gp] = 0; b->inv_ok[gp] = 0; b->v_ok[gp] = 0; continue; }
+      if (posdef_retry(b->fail_host[gp], b->tries[gp], info[gp])) {
+        pending[gp] = 1; b->state_ok[gp] = 0; b->inv_ok[gp] = 0; b->v_ok[gp] = 0;
+        continue;
+      }
       b->state_ok[gp] = info[gp] >= 0;
       b->inv_ok[gp] = pass == 0 && info[gp] >= 0;
       b->v_ok[gp] = b->inv_ok[gp];
@@ -764,14 +783,11 @@ int gprb_batch_create(gprb_ctx* ctx, int32_t B, gprb_dataset* const* ds, const d
       rc = cuda_fail(e, "cudaMallocHost", __FILE__, __LINE__);
       break;
     }
-    // operand tensor maps of the tile GEMM: padded boxes (132 / 68 rows) x KT columns x one GP
-    if ((rc = make_tensor_map(&b->tm_L132, b->Lm, (uint64_t)b->npad, (uint64_t)b->npad, B, (uint64_t)b->npad, mat, NB + 4, KT)) ||
-        (rc = make_tensor_map(&b->tm_L68, b->Lm, (uint64_t)b->npad, (uint64_t)b->npad, B, (uint64_t)b->npad, mat, NB / 2 + 4, KT)) ||
-        (rc = make_tensor_map(&b->tm_A68, b->A, (uint64_t)b->npad, (uint64_t)b->npad, B, (uint64_t)b->npad, mat, NB / 2 + 4, KT)) ||
-        (rc = make_tensor_map(&b->tm_DT132, b->DinvT, NB, (uint64_t)b->J * NB, B, NB, dinv, NB + 4, KT)) ||
-        (rc = make_tensor_map(&b->tm_DT68, b->DinvT, NB, (uint64_t)b->J * NB, B, NB, dinv, NB / 2 + 4, KT)) ||
-        (rc = make_tensor_map(&b->tm_D132, b->Dinv, NB, (uint64_t)b->J * NB, B, NB, dinv, NB + 4, KT)) ||
-        (rc = make_tensor_map(&b->tm_LT, b->Lm, (uint64_t)b->npad, (uint64_t)b->npad, B, (uint64_t)b->npad, mat, KT, NB)))
+    b->gemm = GemmArgs{b->Lm, b->DinvT, b->Dinv, b->A, b->Lm, b->KinvD, nullptr, (int64_t)mat, (int64_t)dinv, (int)b->npad, b->J,
+                       0, GEMM_CHOL_DIAG, (int)((b->n + KT - 1) / KT * KT)};
+    b->gemm.fail = b->fail;
+    if ((rc = encode_factor_maps(b->gemm, B)) ||
+        (rc = make_tensor_map(&b->gemm.tm_LT, b->Lm, (uint64_t)b->npad, (uint64_t)b->npad, B, (uint64_t)b->npad, mat, KT, NB)))
       break;
     b->nstreams = 4;
     b->rl_max = 24;
@@ -938,14 +954,14 @@ static int ensure_pinned(double** p, size_t* cap, size_t need) {
   return 0;
 }
 
-// Enqueue the prediction of the GPs gp0 .. gp1-1 on pipeline `slot` (streams 4 slot .. 4 slot + 3): inputs are copied to
-// the slot's pinned staging, everything else is asynchronous; predict_collect waits and hands the results out.
-static int predict_enqueue(gprb_batch* b, int slot, int gp0, int gp1, int64_t m, const double* Xstar, int64_t xstar_stride,
-                           const double* mstar, bool want_var, int gpb = 1) {
+// Stage a prediction of the GPs gp0 .. gp1-1 (one Xstar block per gpb consecutive GPs) on pipeline `slot`: the slot's
+// events and mask on first use, grow-only scratch (h_out: h_out_doubles), the per-GP mask, the inputs through the pinned
+// staging; then t0 and the uploads on the slot's first stream.
+static int predict_stage(gprb_batch* b, int slot, int gp0, int gp1, int gpb, int64_t m, const double* Xstar,
+                         int64_t xstar_stride, const double* mstar, size_t h_out_doubles) {
   gprb_predict_slot& sl = b->ps[slot];
-  const int B = b->B, J = b->J, count = gp1 - gp0;
-  cudaStream_t* str = b->stream + 4 * slot;
-  cudaStream_t st = str[0];
+  const int B = b->B, count = gp1 - gp0;
+  cudaStream_t st = b->stream[4 * slot];
   const int nblocks = (count + gpb - 1) / gpb;  // Xstar blocks: one per gpb consecutive GPs (the outputs of a trial)
   const size_t nx = (size_t)(xstar_stride ? xstar_stride * (nblocks - 1) + m * b->d : m * b->d);
   const size_t nout = (size_t)count * m;
@@ -958,21 +974,135 @@ static int predict_enqueue(gprb_batch* b, int slot, int gp0, int gp1, int64_t m,
   }
   if ((rc = ensure_dev(&sl.pX, &sl.pX_cap, nx)) || (rc = ensure_dev(&sl.pmu, &sl.pmu_cap, nout)) ||
       (rc = ensure_pinned(&sl.h_in, &sl.h_in_cap, nx + (mstar ? nout : 0))) ||
-      (rc = ensure_pinned(&sl.h_out, &sl.h_out_cap, 2 * nout)))
+      (rc = ensure_pinned(&sl.h_out, &sl.h_out_cap, h_out_doubles)))
     return rc;
   if (mstar && (rc = ensure_dev(&sl.pms, &sl.pms_cap, nout))) return rc;
-  if (want_var && (rc = ensure_dev(&sl.pvar, &sl.pvar_cap, nout))) return rc;
   // per-GP mask: a GP without an evaluated state gets NaN rows and blocks nobody (examples/parallel/core.jl:41-46)
-  bool all_v = true, any_ok = false;
   for (int i = 0; i < B; ++i) sl.h_mask[i] = b->state_ok[i] ? 0 : 1;
-  for (int i = gp0; i < gp1; ++i)
-    if (b->state_ok[i]) { any_ok = true; all_v = all_v && b->v_ok[i]; }
   memcpy(sl.h_in, Xstar, sizeof(double) * nx);
   if (mstar) memcpy(sl.h_in + nx, mstar, sizeof(double) * nout);
   GPRB_CUDA(cudaEventRecord(sl.t0, st));
   GPRB_CUDA(cudaMemcpyAsync(sl.mask, sl.h_mask, sizeof(int32_t) * B, cudaMemcpyHostToDevice, st));
   GPRB_CUDA(cudaMemcpyAsync(sl.pX, sl.h_in, sizeof(double) * nx, cudaMemcpyHostToDevice, st));
   if (mstar) GPRB_CUDA(cudaMemcpyAsync(sl.pms, sl.h_in + nx, sizeof(double) * nout, cudaMemcpyHostToDevice, st));
+  return 0;
+}
+
+// The slot's right-hand-side block pT [count][npad][PT] and its tensor map (row r = k, box = 68 columns x KT rows),
+// re-encoded whenever pT is (re)allocated.
+static int slot_rhs(gprb_batch* b, gprb_predict_slot& sl, int count) {
+  int rc;
+  if ((rc = ensure_dev(&sl.pT, &sl.pT_cap, (size_t)count * b->npad * PT))) return rc;
+  if (sl.tm_T_cap != sl.pT_cap) {
+    if ((rc = make_tensor_map(&sl.tm_T68, sl.pT, PT, (uint64_t)b->npad, sl.pT_cap / ((size_t)b->npad * PT), PT, (uint64_t)b->npad * PT,
+                              NB / 2 + 4, KT)))
+      return rc;
+    sl.tm_T_cap = sl.pT_cap;
+  }
+  return 0;
+}
+
+// One dependent chain of J tile-GEMM launches, one per block row: GEMM_FWD_ROW top-down, GEMM_BWD_ROW bottom-up.
+static int row_chain(gprb_batch* b, GemmArgs& ga, int mode, int ntl, int count, cudaStream_t st) {
+  ga.mode = mode;
+  for (int k = 0; k < ga.J; ++k) {
+    ga.step = mode == GEMM_BWD_ROW ? ga.J - 1 - k : k;
+    if (int rc = launch_tile_gemm(ga, ntl, count, st)) return rc;
+    b->ctx->launches++;
+  }
+  return 0;
+}
+
+// The tiled path of a prediction staged on `slot` (predict_stage), one chunk of PT test columns at a time:
+// k_predict_cross on the slot's first stream; the GPs dealt over stream groups (the slot's streams and join events),
+// each of which runs the FWD_ROW chain T = L^-1 K* when T != nullptr and then hook(ta, ga, ntl, g0, g1, stream) on its
+// stream; with `finish`, k_predict_finish of the whole range on the slot's first stream.  T is [count][npad][PT] behind
+// tm_T, or with keep_T one such block per chunk (chunk c of local GP g is block c * count + g).  hook = nullptr: no
+// per-group work besides the chain.
+template <typename Hook>
+static int predict_tiles(gprb_batch* b, int slot, int gp0, int gp1, int gpb, int64_t m, int64_t xstar_stride, bool mstar,
+                         double* var, double* T, const CUtensorMap& tm_T, bool keep_T, bool finish, Hook&& hook) {
+  constexpr bool has_hook = !std::is_same<Hook, std::nullptr_t>::value;
+  static const char* zmax = getenv("GPRB200_PC_ZMAX");
+  gprb_predict_slot& sl = b->ps[slot];
+  const int J = b->J, count = gp1 - gp0;
+  const int64_t npad = b->npad;
+  cudaStream_t* str = b->stream + 4 * slot;
+  cudaEvent_t* join = b->join + 4 * slot;
+  int rc;
+  if ((rc = ensure_dev(&sl.pmupart, &sl.pmupart_cap, (size_t)count * J * PT))) return rc;
+  // L^-1 K*: one launch per block row, `count` tiles of 128 x 128 each (PDMats whiten! as a blocked substitution)
+  GemmArgs ga = b->gemm;
+  ga.Cin = nullptr;
+  ga.Tm = T; ga.t_stride = npad * PT; ga.ldt = PT;
+  ga.tm_T68 = tm_T;
+  ga.fail = sl.mask;  // tiles of a GP without state exit at once
+  // the GPs are dealt over the stream groups: the dependent chain of J launches of one group fills the wave
+  // tails of the others (`count` tiles per launch are not a multiple of the SM count); with no work per group (a
+  // mean-only gprb_predict) there is one group and no event
+  const int ns = std::min(4, b->nstreams);
+  const int S = (T || has_hook) && count >= 8 * ns ? ns : 1;
+  for (int c = 0; (int64_t)c * PT < m; ++c) {
+    const int64_t s0 = (int64_t)c * PT;
+    const int tblk = keep_T ? c * count : 0;  // T block of the chunk's first GP
+    PredictTileArgs ta{b->Xtptr, b->theta, b->alpha, sl.pX, mstar ? sl.pms : nullptr, T ? T + (size_t)tblk * npad * PT : nullptr,
+                       sl.pmupart, sl.pmu, var, xstar_stride, (int)b->n, (int)npad, b->d, J, (int)m, b->kind, (int)s0,
+                       (int)std::min<int64_t>(PT, m - s0)};
+    ta.gp_off = gp0;
+    ta.mask = sl.mask;
+    ta.gpb = gpb;
+    if (zmax) ta.zmax = atof(zmax);
+    if ((rc = launch_predict_cross(ta, count, str[0]))) return rc;
+    b->ctx->launches++;
+    ga.t_gp_off = gp0 - tblk;
+    ga.ncols = ta.mc;
+    // right-hand-side tiles are 64 test columns wide (two CTAs per SM); few GPs (large n, or the reference's single-GP
+    // call pattern): 32-column tiles, so that a launch still puts a CTA on every SM
+    ga.colw = (int64_t)count * ((ta.mc + 63) / 64) >= b->ctx->sm_count ? 64 : 32;
+    const int ntl = (ta.mc + ga.colw - 1) / ga.colw;
+    if (S > 1) GPRB_CUDA(cudaEventRecord(join[0], str[0]));
+    for (int s = 0; s < S; ++s) {
+      const int g0 = (int)((int64_t)count * s / S), g1 = (int)((int64_t)count * (s + 1) / S);
+      if (s > 0) GPRB_CUDA(cudaStreamWaitEvent(str[s], join[0], 0));
+      ga.gp_off = gp0 + g0;
+      if (T && (rc = row_chain(b, ga, GEMM_FWD_ROW, ntl, g1 - g0, str[s]))) return rc;
+      if constexpr (has_hook)
+        if ((rc = hook(ta, ga, ntl, g0, g1, str[s]))) return rc;
+      if (s > 0) {
+        GPRB_CUDA(cudaEventRecord(join[s], str[s]));
+        GPRB_CUDA(cudaStreamWaitEvent(str[0], join[s], 0));
+      }
+    }
+    if (finish) {
+      if ((rc = launch_predict_finish(ta, count, str[0]))) return rc;
+      b->ctx->launches++;
+    }
+  }
+  return 0;
+}
+
+// Wait for the slot's t1 and keep the device time t0 .. t1 of its last call (gprb_last_predict_ms).
+static int slot_wait(gprb_predict_slot& sl) {
+  GPRB_CUDA(cudaEventSynchronize(sl.t1));
+  float ms = 0.f;
+  if (cudaEventElapsedTime(&ms, sl.t0, sl.t1) == cudaSuccess) sl.last_ms = ms;
+  return 0;
+}
+
+// Enqueue the prediction of the GPs gp0 .. gp1-1 on pipeline `slot` (streams 4 slot .. 4 slot + 3): inputs are copied to
+// the slot's pinned staging, everything else is asynchronous; predict_collect waits and hands the results out.
+static int predict_enqueue(gprb_batch* b, int slot, int gp0, int gp1, int64_t m, const double* Xstar, int64_t xstar_stride,
+                           const double* mstar, bool want_var, int gpb = 1) {
+  gprb_predict_slot& sl = b->ps[slot];
+  const int J = b->J, count = gp1 - gp0;
+  cudaStream_t st = b->stream[4 * slot];
+  const size_t nout = (size_t)count * m;
+  int rc;
+  if ((rc = predict_stage(b, slot, gp0, gp1, gpb, m, Xstar, xstar_stride, mstar, 2 * nout))) return rc;
+  if (want_var && (rc = ensure_dev(&sl.pvar, &sl.pvar_cap, nout))) return rc;
+  bool all_v = true, any_ok = false;
+  for (int i = gp0; i < gp1; ++i)
+    if (b->state_ok[i]) { any_ok = true; all_v = all_v && b->v_ok[i]; }
 
   // GEMV-like path: few test columns and the triangular inverse already resident (the last evaluation had a gradient)
   const int ps = m <= 1 ? 1 : m <= 2 ? 2 : m <= 4 ? 4 : 8;
@@ -991,64 +1121,10 @@ static int predict_enqueue(gprb_batch* b, int slot, int gp0, int gp1, int64_t m,
     if ((rc = launch_predict(pa, count, st))) return rc;
     b->ctx->launches++;
   } else {
-    if ((rc = ensure_dev(&sl.pmupart, &sl.pmupart_cap, (size_t)count * J * PT))) return rc;
-    if (want_var) {
-      if ((rc = ensure_dev(&sl.pT, &sl.pT_cap, (size_t)count * b->npad * PT))) return rc;
-      if (sl.tm_T_cap != sl.pT_cap) {  // (re)allocated: the right-hand-side block [GP][row r = k][PT test columns], box = 68 columns x KT rows
-        if ((rc = make_tensor_map(&sl.tm_T68, sl.pT, PT, (uint64_t)b->npad, sl.pT_cap / ((size_t)b->npad * PT), PT, (uint64_t)b->npad * PT,
-                                  NB / 2 + 4, KT)))
-          return rc;
-        sl.tm_T_cap = sl.pT_cap;
-      }
-    }
-    const int nv = (int)((b->n + KT - 1) / KT * KT);
-    for (int64_t s0 = 0; s0 < m; s0 += PT) {
-      PredictTileArgs ta{b->Xtptr, b->theta, b->alpha, sl.pX, mstar ? sl.pms : nullptr, want_var ? sl.pT : nullptr, sl.pmupart,
-                         sl.pmu, want_var ? sl.pvar : nullptr, xstar_stride, (int)b->n, (int)b->npad, b->d, J, (int)m, b->kind,
-                         (int)s0, (int)std::min<int64_t>(PT, m - s0)};
-      ta.gp_off = gp0;
-      ta.mask = sl.mask;
-      ta.gpb = gpb;
-      { static const char* ev = getenv("GPRB200_PC_ZMAX"); if (ev) ta.zmax = atof(ev); }
-      if ((rc = launch_predict_cross(ta, count, st))) return rc;
-      b->ctx->launches++;
-      if (want_var) {
-        // L^-1 K*: one launch per block row, `count` tiles of 128 x 128 each (PDMats whiten! as a blocked substitution)
-        GemmArgs ga{b->Lm, b->DinvT, b->Dinv, nullptr, b->Lm, b->KinvD, nullptr, b->npad * b->npad, (int64_t)J * NB * NB,
-                    (int)b->npad, J, 0, GEMM_FWD_ROW, nv};
-        ga.Tm = sl.pT; ga.t_stride = b->npad * PT; ga.ldt = PT; ga.t_gp_off = gp0;
-        set_gemm_maps(ga, b);
-        ga.tm_T68 = sl.tm_T68;
-        ga.ncols = ta.mc;
-        ga.fail = sl.mask;  // tiles of a GP without state exit at once
-        // right-hand-side tiles are 64 test columns wide (two CTAs per SM); few GPs (large n, or the reference's single-GP
-        // call pattern): 32-column tiles, so that a launch still puts a CTA on every SM
-        ga.colw = (int64_t)count * ((ta.mc + 63) / 64) >= b->ctx->sm_count ? 64 : 32;
-        const int ntl = (ta.mc + ga.colw - 1) / ga.colw;
-        // the GPs are dealt over the stream groups: the dependent chain of J launches of one group fills the wave
-        // tails of the others (`count` tiles per launch are not a multiple of the SM count)
-        const int ns = std::min(4, b->nstreams);
-        const int S = (count >= 8 * ns) ? ns : 1;
-        if (S > 1) GPRB_CUDA(cudaEventRecord(b->join[4 * slot], st));
-        for (int s = 0; s < S; ++s) {
-          const int g0 = (int)((int64_t)count * s / S), g1 = (int)((int64_t)count * (s + 1) / S);
-          cudaStream_t ss = str[s];
-          if (s > 0) GPRB_CUDA(cudaStreamWaitEvent(ss, b->join[4 * slot], 0));
-          ga.gp_off = gp0 + g0;
-          for (int i = 0; i < J; ++i) {
-            ga.step = i;
-            if ((rc = launch_tile_gemm(ga, ntl, g1 - g0, ss))) return rc;
-            b->ctx->launches++;
-          }
-          if (s > 0) {
-            GPRB_CUDA(cudaEventRecord(b->join[4 * slot + s], ss));
-            GPRB_CUDA(cudaStreamWaitEvent(st, b->join[4 * slot + s], 0));
-          }
-        }
-      }
-      if ((rc = launch_predict_finish(ta, count, st))) return rc;
-      b->ctx->launches++;
-    }
+    if (want_var && (rc = slot_rhs(b, sl, count))) return rc;
+    if ((rc = predict_tiles(b, slot, gp0, gp1, gpb, m, xstar_stride, mstar != nullptr, want_var ? sl.pvar : nullptr,
+                            want_var ? sl.pT : nullptr, sl.tm_T68, false, true, nullptr)))
+      return rc;
   }
   GPRB_CUDA(cudaMemcpyAsync(sl.h_out, sl.pmu, sizeof(double) * nout, cudaMemcpyDeviceToHost, st));
   if (want_var) GPRB_CUDA(cudaMemcpyAsync(sl.h_out + nout, sl.pvar, sizeof(double) * nout, cudaMemcpyDeviceToHost, st));
@@ -1059,10 +1135,9 @@ static int predict_enqueue(gprb_batch* b, int slot, int gp0, int gp1, int64_t m,
 
 static int predict_collect(gprb_batch* b, int slot, double* mu, double* var) {
   gprb_predict_slot& sl = b->ps[slot];
-  GPRB_CUDA(cudaEventSynchronize(sl.t1));
+  int rc = slot_wait(sl);
+  if (rc) return rc;
   sl.pending = false;
-  float ms = 0.f;
-  if (cudaEventElapsedTime(&ms, sl.t0, sl.t1) == cudaSuccess) sl.last_ms = ms;
   const size_t nout = (size_t)(sl.gp1 - sl.gp0) * sl.m;
   memcpy(mu, sl.h_out, sizeof(double) * nout);
   if (var && sl.want_var) memcpy(var, sl.h_out + nout, sizeof(double) * nout);
@@ -1182,93 +1257,33 @@ int gprb_get_Kinv(gprb_batch* b, int32_t gp, double* out) {
 // ------------------------------------------------------------------------------------------------
 // Full posterior covariance and posterior draws (gprb_predict_cov, gprb_sample_posterior) on prediction slot 0.
 // The right-hand sides T = L^-1 K* of every 128-column chunk are kept (one [B][npad][PT] block per chunk behind one tensor
-// map), computed by the launches gprb_predict uses (k_predict_cross, GEMM_FWD_ROW chains on the four stream groups,
-// k_predict_finish for mu) - always the tiled path, the GEMV path never materialises T.  The covariance tiles of a stream
-// group follow its last FWD_ROW chain on the group's stream.  Leaves Sigma in pc.S and mu in the slot's pmu; t0 recorded.
+// map), computed by gprb_predict's tiled path (predict_tiles) - the GEMV path never materialises T.  The covariance
+// tiles of a stream group follow its last FWD_ROW chain on the group's stream.  Leaves Sigma in pc.S and mu in the slot's
+// pmu; t0 recorded.
 static int postcov_enqueue(gprb_batch* b, int64_t m, const double* Xstar, int64_t xstar_stride, const double* mstar, bool add_noise) {
   gprb_predict_slot& sl = b->ps[0];
   gprb_postcov_ws& w = b->pc;
-  const int B = b->B, J = b->J, count = B, gp0 = 0;
-  cudaStream_t* str = b->stream;
-  cudaStream_t st = str[0];
+  const int count = b->B;
   const int64_t npad = b->npad, mpad = (m + NB - 1) / NB * NB;
   const int nchunk = (int)(mpad / NB);
-  const size_t nx = (size_t)(xstar_stride ? xstar_stride * (B - 1) + m * b->d : m * b->d);
-  const size_t nout = (size_t)count * m;
   int rc;
-  if (!sl.t0) {
-    GPRB_CUDA(cudaEventCreate(&sl.t0));
-    GPRB_CUDA(cudaEventCreate(&sl.t1));
-    GPRB_CUDA(cudaMallocHost((void**)&sl.h_mask, sizeof(int32_t) * B));
-    if ((rc = dev_alloc(&sl.mask, (size_t)B))) return rc;
-  }
-  if ((rc = ensure_dev(&sl.pX, &sl.pX_cap, nx)) || (rc = ensure_dev(&sl.pmu, &sl.pmu_cap, nout)) ||
-      (rc = ensure_dev(&sl.pmupart, &sl.pmupart_cap, (size_t)count * J * PT)) ||
-      (rc = ensure_pinned(&sl.h_in, &sl.h_in_cap, nx + (mstar ? nout : 0))) || (rc = ensure_pinned(&sl.h_out, &sl.h_out_cap, nout)) ||
-      (rc = ensure_dev(&w.T, &w.T_cap, (size_t)nchunk * count * npad * PT)) ||
-      (rc = ensure_dev(&w.S, &w.S_cap, (size_t)count * mpad * mpad)) || (rc = ensure_dev(&w.bad, &w.bad_cap, (size_t)count)))
+  if ((rc = ensure_dev(&w.T, &w.T_cap, (size_t)nchunk * count * npad * PT)) ||
+      (rc = ensure_dev(&w.S, &w.S_cap, (size_t)count * mpad * mpad)) || (rc = ensure_dev(&w.bad, &w.bad_cap, (size_t)count)) ||
+      // T of chunk c, GP g is block c * count + g of the map
+      (rc = make_tensor_map(&w.tm_T68, w.T, PT, (uint64_t)npad, (uint64_t)nchunk * count, PT, (uint64_t)npad * PT, NB / 2 + 4, KT)) ||
+      (rc = predict_stage(b, 0, 0, count, 1, m, Xstar, xstar_stride, mstar, (size_t)count * m)))
     return rc;
-  if (mstar && (rc = ensure_dev(&sl.pms, &sl.pms_cap, nout))) return rc;
-  // T of chunk c, GP g is block c * count + g of the map (GEMM_FWD_ROW reads it through t_gp_off = gp0 - c * count)
-  if ((rc = make_tensor_map(&w.tm_T68, w.T, PT, (uint64_t)npad, (uint64_t)nchunk * count, PT, (uint64_t)npad * PT, NB / 2 + 4, KT)))
-    return rc;
-  for (int i = 0; i < B; ++i) sl.h_mask[i] = b->state_ok[i] ? 0 : 1;
-  memcpy(sl.h_in, Xstar, sizeof(double) * nx);
-  if (mstar) memcpy(sl.h_in + nx, mstar, sizeof(double) * nout);
-  GPRB_CUDA(cudaEventRecord(sl.t0, st));
-  GPRB_CUDA(cudaMemcpyAsync(sl.mask, sl.h_mask, sizeof(int32_t) * B, cudaMemcpyHostToDevice, st));
-  GPRB_CUDA(cudaMemcpyAsync(sl.pX, sl.h_in, sizeof(double) * nx, cudaMemcpyHostToDevice, st));
-  if (mstar) GPRB_CUDA(cudaMemcpyAsync(sl.pms, sl.h_in + nx, sizeof(double) * nout, cudaMemcpyHostToDevice, st));
-  GPRB_CUDA(cudaMemsetAsync(w.bad, 0, sizeof(int32_t) * count, st));
-
-  const int nv = (int)((b->n + KT - 1) / KT * KT);
-  PostCovArgs pa{sl.pX, b->theta, sl.mask, w.S, w.bad, xstar_stride, nv, b->d, (int)m, (int)mpad, b->kind, gp0, count, 0,
+  GPRB_CUDA(cudaMemsetAsync(w.bad, 0, sizeof(int32_t) * count, b->stream[0]));
+  PostCovArgs pa{sl.pX, b->theta, sl.mask, w.S, w.bad, xstar_stride, b->gemm.nv, b->d, (int)m, (int)mpad, b->kind, 0, count, 0,
                  add_noise ? 1 : 0, w.tm_T68};
-  const int ns = std::min(4, b->nstreams);
-  const int S = (count >= 8 * ns) ? ns : 1;
-  for (int c = 0; c < nchunk; ++c) {
-    const int64_t s0 = (int64_t)c * PT;
-    PredictTileArgs ta{b->Xtptr, b->theta, b->alpha, sl.pX, mstar ? sl.pms : nullptr, w.T + (size_t)c * count * npad * PT,
-                       sl.pmupart, sl.pmu, nullptr, xstar_stride, (int)b->n, (int)b->npad, b->d, J, (int)m, b->kind,
-                       (int)s0, (int)std::min<int64_t>(PT, m - s0)};
-    ta.gp_off = gp0;
-    ta.mask = sl.mask;
-    if ((rc = launch_predict_cross(ta, count, st))) return rc;
+  auto cov = [&](const PredictTileArgs& ta, GemmArgs&, int, int g0, int g1, cudaStream_t ss) {
+    if (ta.s0 + ta.mc < m) return 0;  // the covariance tiles wait until every chunk of the group's GPs is solved
+    pa.g0 = g0;
+    if (int rc = launch_post_cov(pa, g1 - g0, ss)) return rc;
     b->ctx->launches++;
-    GemmArgs ga{b->Lm, b->DinvT, b->Dinv, nullptr, b->Lm, b->KinvD, nullptr, b->npad * b->npad, (int64_t)J * NB * NB,
-                (int)b->npad, J, 0, GEMM_FWD_ROW, nv};
-    ga.Tm = w.T; ga.t_stride = npad * PT; ga.ldt = PT; ga.t_gp_off = gp0 - c * count;
-    set_gemm_maps(ga, b);
-    ga.tm_T68 = w.tm_T68;
-    ga.ncols = ta.mc;
-    ga.fail = sl.mask;
-    ga.colw = (int64_t)count * ((ta.mc + 63) / 64) >= b->ctx->sm_count ? 64 : 32;
-    const int ntl = (ta.mc + ga.colw - 1) / ga.colw;
-    if (S > 1) GPRB_CUDA(cudaEventRecord(b->join[0], st));
-    for (int s = 0; s < S; ++s) {
-      const int g0 = (int)((int64_t)count * s / S), g1 = (int)((int64_t)count * (s + 1) / S);
-      cudaStream_t ss = str[s];
-      if (s > 0) GPRB_CUDA(cudaStreamWaitEvent(ss, b->join[0], 0));
-      ga.gp_off = gp0 + g0;
-      for (int i = 0; i < J; ++i) {
-        ga.step = i;
-        if ((rc = launch_tile_gemm(ga, ntl, g1 - g0, ss))) return rc;
-        b->ctx->launches++;
-      }
-      if (c == nchunk - 1) {  // every chunk of this group's GPs is solved: its covariance tiles
-        pa.g0 = g0;
-        if ((rc = launch_post_cov(pa, g1 - g0, ss))) return rc;
-        b->ctx->launches++;
-      }
-      if (s > 0) {
-        GPRB_CUDA(cudaEventRecord(b->join[s], ss));
-        GPRB_CUDA(cudaStreamWaitEvent(st, b->join[s], 0));
-      }
-    }
-    if ((rc = launch_predict_finish(ta, count, st))) return rc;
-    b->ctx->launches++;
-  }
-  return 0;
+    return 0;
+  };
+  return predict_tiles(b, 0, 0, count, 1, m, xstar_stride, mstar != nullptr, nullptr, w.T, w.tm_T68, true, true, cov);
 }
 
 static int postcov_check(gprb_batch* b, int64_t m, const double* Xstar, int64_t xstar_stride) {
@@ -1289,14 +1304,7 @@ static int postcov_factor(gprb_batch* b, int64_t m, const int32_t* list, int cnt
   GemmArgs ga{w.L, w.DinvT, w.Dinv, w.S, w.L, nullptr, list, ms, dstride, (int)mpad, Jm, 0, GEMM_CHOL_DIAG, nvm};
   ga.fail = w.fail;
   if (Jm > 1) {
-    const uint64_t B = (uint64_t)b->B;
-    if ((rc = make_tensor_map(&ga.tm_L132, w.L, mpad, mpad, B, mpad, ms, NB + 4, KT)) ||
-        (rc = make_tensor_map(&ga.tm_L68, w.L, mpad, mpad, B, mpad, ms, NB / 2 + 4, KT)) ||
-        (rc = make_tensor_map(&ga.tm_A68, w.S, mpad, mpad, B, mpad, ms, NB / 2 + 4, KT)) ||
-        (rc = make_tensor_map(&ga.tm_DT132, w.DinvT, NB, (uint64_t)Jm * NB, B, NB, dstride, NB + 4, KT)) ||
-        (rc = make_tensor_map(&ga.tm_DT68, w.DinvT, NB, (uint64_t)Jm * NB, B, NB, dstride, NB / 2 + 4, KT)) ||
-        (rc = make_tensor_map(&ga.tm_D132, w.Dinv, NB, (uint64_t)Jm * NB, B, NB, dstride, NB + 4, KT)))
-      return rc;
+    if ((rc = encode_factor_maps(ga, (uint64_t)b->B))) return rc;
     ga.tm_T68 = w.tm_T68;
   }
   DiagArgs da{w.S, w.L, w.Dinv, w.DinvT, w.logdet, w.fail, list, ms, dstride, (int)mpad, Jm, 0, nvm};
@@ -1317,14 +1325,6 @@ static int postcov_factor(gprb_batch* b, int64_t m, const int32_t* list, int cnt
       b->ctx->launches++;
     }
   }
-  return 0;
-}
-
-static int postcov_finish_time(gprb_batch* b) {
-  gprb_predict_slot& sl = b->ps[0];
-  GPRB_CUDA(cudaEventSynchronize(sl.t1));
-  float ms = 0.f;
-  if (cudaEventElapsedTime(&ms, sl.t0, sl.t1) == cudaSuccess) sl.last_ms = ms;
   return 0;
 }
 
@@ -1354,7 +1354,7 @@ int gprb_predict_cov(gprb_batch* b, int64_t m, const double* Xstar, int64_t xsta
   GPRB_CUDA(cudaMemcpyAsync(sl.h_out, sl.pmu, sizeof(double) * B * m, cudaMemcpyDeviceToHost, st));
   GPRB_CUDA(cudaMemcpyAsync(cov, w.O, sizeof(double) * B * m * m, cudaMemcpyDeviceToHost, st));
   GPRB_CUDA(cudaStreamSynchronize(st));
-  if ((rc = postcov_finish_time(b))) return rc;
+  if ((rc = slot_wait(sl))) return rc;
   memcpy(mu, sl.h_out, sizeof(double) * B * m);
   return GPRB_OK;
 }
@@ -1407,11 +1407,7 @@ int gprb_sample_posterior(gprb_batch* b, int64_t m, const double* Xstar, int64_t
     std::vector<int32_t> retry;
     for (int k = 0; k < cnt; ++k) {
       const int g = list ? pend[k] : k;
-      const int f = w.fail_host[g];
-      if (f == 0) info[g] = tries[g];
-      else if (f < 0) info[g] = -2;
-      else if (tries[g] >= MAX_JITTER) info[g] = -1;
-      else { ++tries[g]; retry.push_back(g); }
+      if (posdef_retry(w.fail_host[g], tries[g], info[g])) retry.push_back(g);
     }
     if (retry.empty()) break;
     pend = retry;
@@ -1429,7 +1425,7 @@ int gprb_sample_posterior(gprb_batch* b, int64_t m, const double* Xstar, int64_t
   GPRB_CUDA(cudaEventRecord(sl.t1, st));
   GPRB_CUDA(cudaMemcpyAsync(out, w.O, sizeof(double) * nz, cudaMemcpyDeviceToHost, st));
   GPRB_CUDA(cudaStreamSynchronize(st));
-  return postcov_finish_time(b);
+  return slot_wait(sl);
 }
 
 }  // extern "C"
@@ -1587,119 +1583,50 @@ int gprb_eval_loo(gprb_batch* b, const double* theta, const uint8_t* active, dou
 }  // extern "C"
 
 // ------------------------------------------------------------------------------------------------
-// Predictive gradients (gprb_predict_grad) on prediction slot 0, chunk by chunk (128 test columns).  Per chunk:
-// k_predict_cross on the slot's stream, then per stream group of GPs: the FWD_ROW chain (T = L^-1 K*, when a variance is
-// asked for), k_predict_finish for the group's mu / var (the launches gprb_predict's tiled path issues, so mu and var are
-// bit-identical to it), the BWD_ROW chain (beta = L^-T T in place, only with dvar) and k_predict_jac.
+// Predictive gradients (gprb_predict_grad) on prediction slot 0, chunk by chunk (128 test columns): gprb_predict's tiled
+// path (predict_tiles; the FWD_ROW chain T = L^-1 K* only when a variance is asked for), where each stream group then
+// runs k_predict_finish for its own mu / var (the launches gprb_predict issues, so mu and var are bit-identical to it),
+// the BWD_ROW chain (beta = L^-T T in place, only with dvar) and k_predict_jac.
 static int predgrad_enqueue(gprb_batch* b, int64_t m, const double* Xstar, int64_t xstar_stride, const double* mstar,
                             const double* dmstar, bool want_var, bool want_dvar) {
   gprb_predict_slot& sl = b->ps[0];
   gprb_predgrad_ws& w = b->pg;
-  const int B = b->B, J = b->J, count = B, d = b->d;
+  const int J = b->J, count = b->B, d = b->d;
   const int64_t npad = b->npad;
-  cudaStream_t* str = b->stream;
-  cudaStream_t st = str[0];
+  cudaStream_t st = b->stream[0];
   const bool want_T = want_var || want_dvar;
-  const size_t nx = (size_t)(xstar_stride ? xstar_stride * (B - 1) + m * d : m * d);
   const size_t nout = (size_t)count * m, njac = nout * d;
   int rc;
-  if (!sl.t0) {
-    GPRB_CUDA(cudaEventCreate(&sl.t0));
-    GPRB_CUDA(cudaEventCreate(&sl.t1));
-    GPRB_CUDA(cudaMallocHost((void**)&sl.h_mask, sizeof(int32_t) * B));
-    if ((rc = dev_alloc(&sl.mask, (size_t)B))) return rc;
-  }
-  if ((rc = ensure_dev(&sl.pX, &sl.pX_cap, nx)) || (rc = ensure_dev(&sl.pmu, &sl.pmu_cap, nout)) ||
-      (rc = ensure_dev(&sl.pmupart, &sl.pmupart_cap, (size_t)count * J * PT)) ||
-      (rc = ensure_pinned(&sl.h_in, &sl.h_in_cap, nx + (mstar ? nout : 0))) || (rc = ensure_pinned(&sl.h_out, &sl.h_out_cap, 2 * nout)) ||
-      (rc = ensure_dev(&w.jac, &w.jac_cap, (want_dvar ? 2 : 1) * njac)))
-    return rc;
-  if (mstar && (rc = ensure_dev(&sl.pms, &sl.pms_cap, nout))) return rc;
+  if ((rc = ensure_dev(&w.jac, &w.jac_cap, (want_dvar ? 2 : 1) * njac))) return rc;
   if (dmstar && (rc = ensure_dev(&w.dms, &w.dms_cap, njac))) return rc;
   if (want_var && (rc = ensure_dev(&sl.pvar, &sl.pvar_cap, nout))) return rc;
-  if (want_T) {
-    if ((rc = ensure_dev(&sl.pT, &sl.pT_cap, (size_t)count * npad * PT))) return rc;
-    if (sl.tm_T_cap != sl.pT_cap) {
-      if ((rc = make_tensor_map(&sl.tm_T68, sl.pT, PT, (uint64_t)npad, sl.pT_cap / ((size_t)npad * PT), PT, (uint64_t)npad * PT,
-                                NB / 2 + 4, KT)))
-        return rc;
-      sl.tm_T_cap = sl.pT_cap;
-    }
-  }
-  for (int i = 0; i < B; ++i) sl.h_mask[i] = b->state_ok[i] ? 0 : 1;
-  memcpy(sl.h_in, Xstar, sizeof(double) * nx);
-  if (mstar) memcpy(sl.h_in + nx, mstar, sizeof(double) * nout);
-  GPRB_CUDA(cudaEventRecord(sl.t0, st));
-  GPRB_CUDA(cudaMemcpyAsync(sl.mask, sl.h_mask, sizeof(int32_t) * B, cudaMemcpyHostToDevice, st));
-  GPRB_CUDA(cudaMemcpyAsync(sl.pX, sl.h_in, sizeof(double) * nx, cudaMemcpyHostToDevice, st));
-  if (mstar) GPRB_CUDA(cudaMemcpyAsync(sl.pms, sl.h_in + nx, sizeof(double) * nout, cudaMemcpyHostToDevice, st));
+  if (want_T && (rc = slot_rhs(b, sl, count))) return rc;
+  if ((rc = predict_stage(b, 0, 0, count, 1, m, Xstar, xstar_stride, mstar, 2 * nout))) return rc;
   if (dmstar) GPRB_CUDA(cudaMemcpyAsync(w.dms, dmstar, sizeof(double) * njac, cudaMemcpyHostToDevice, st));
-
-  const int nv = (int)((b->n + KT - 1) / KT * KT);
-  const int ns = std::min(4, b->nstreams);
-  const int S = (count >= 8 * ns) ? ns : 1;
-  for (int64_t s0 = 0; s0 < m; s0 += PT) {
-    PredictTileArgs ta{b->Xtptr, b->theta, b->alpha, sl.pX, mstar ? sl.pms : nullptr, want_T ? sl.pT : nullptr, sl.pmupart,
-                       sl.pmu, want_var ? sl.pvar : nullptr, xstar_stride, (int)b->n, (int)npad, d, J, (int)m, b->kind,
-                       (int)s0, (int)std::min<int64_t>(PT, m - s0)};
-    ta.gp_off = 0;
-    ta.mask = sl.mask;
-    if ((rc = launch_predict_cross(ta, count, st))) return rc;
+  auto jac = [&](const PredictTileArgs& ta, GemmArgs& ga, int ntl, int g0, int g1, cudaStream_t ss) {
+    // the group's mu / var: k_predict_finish indexes its outputs and T by blockIdx, so the group's GPs start at g0
+    PredictTileArgs tg = ta;
+    tg.gp_off = g0;
+    if (tg.T) tg.T += (size_t)g0 * npad * PT;
+    tg.mupart += (size_t)g0 * J * PT;
+    tg.mu += (size_t)g0 * m;
+    if (tg.var) tg.var += (size_t)g0 * m;
+    if (tg.mstar) tg.mstar += (size_t)g0 * m;
+    int rc;
+    if ((rc = launch_predict_finish(tg, g1 - g0, ss))) return rc;
     b->ctx->launches++;
-    GemmArgs ga{b->Lm, b->DinvT, b->Dinv, nullptr, b->Lm, b->KinvD, nullptr, npad * npad, (int64_t)J * NB * NB,
-                (int)npad, J, 0, GEMM_FWD_ROW, nv};
-    ga.Tm = sl.pT; ga.t_stride = npad * PT; ga.ldt = PT; ga.t_gp_off = 0;
-    set_gemm_maps(ga, b);
-    ga.tm_T68 = sl.tm_T68;
-    ga.tm_LT = b->tm_LT;
-    ga.ncols = ta.mc;
-    ga.fail = sl.mask;
-    ga.colw = (int64_t)count * ((ta.mc + 63) / 64) >= b->ctx->sm_count ? 64 : 32;
-    const int ntl = (ta.mc + ga.colw - 1) / ga.colw;
-    if (S > 1) GPRB_CUDA(cudaEventRecord(b->join[0], st));
-    for (int s = 0; s < S; ++s) {
-      const int g0 = (int)((int64_t)count * s / S), g1 = (int)((int64_t)count * (s + 1) / S);
-      cudaStream_t ss = str[s];
-      if (s > 0) GPRB_CUDA(cudaStreamWaitEvent(ss, b->join[0], 0));
-      ga.gp_off = g0;
-      if (want_T) {
-        ga.mode = GEMM_FWD_ROW;
-        for (int i = 0; i < J; ++i) {
-          ga.step = i;
-          if ((rc = launch_tile_gemm(ga, ntl, g1 - g0, ss))) return rc;
-          b->ctx->launches++;
-        }
-      }
-      // the group's mu / var: k_predict_finish indexes its outputs and T by blockIdx, so the group's GPs start at g0
-      PredictTileArgs tg = ta;
-      tg.gp_off = g0;
-      if (tg.T) tg.T += (size_t)g0 * npad * PT;
-      tg.mupart += (size_t)g0 * J * PT;
-      tg.mu += (size_t)g0 * m;
-      if (tg.var) tg.var += (size_t)g0 * m;
-      if (tg.mstar) tg.mstar += (size_t)g0 * m;
-      if ((rc = launch_predict_finish(tg, g1 - g0, ss))) return rc;
-      b->ctx->launches++;
-      if (want_dvar) {
-        ga.mode = GEMM_BWD_ROW;
-        for (int i = J - 1; i >= 0; --i) {
-          ga.step = i;
-          if ((rc = launch_tile_gemm(ga, ntl, g1 - g0, ss))) return rc;
-          b->ctx->launches++;
-        }
-      }
-      PredictJacArgs ja{b->Xtptr, b->theta, b->alpha, want_dvar ? sl.pT + (size_t)g0 * npad * PT : nullptr,
-                        sl.pX + (size_t)g0 * xstar_stride, dmstar ? w.dms + (size_t)g0 * m * d : nullptr,
-                        w.jac + (size_t)g0 * m * d, want_dvar ? w.jac + njac + (size_t)g0 * m * d : nullptr, sl.mask,
-                        xstar_stride, (int)b->n, (int)npad, d, (int)m, b->kind, (int)s0, ta.mc, g0};
-      if ((rc = launch_predict_jac(ja, g1 - g0, ss))) return rc;
-      b->ctx->launches++;
-      if (s > 0) {
-        GPRB_CUDA(cudaEventRecord(b->join[s], ss));
-        GPRB_CUDA(cudaStreamWaitEvent(st, b->join[s], 0));
-      }
-    }
-  }
+    if (want_dvar && (rc = row_chain(b, ga, GEMM_BWD_ROW, ntl, g1 - g0, ss))) return rc;
+    PredictJacArgs ja{b->Xtptr, b->theta, b->alpha, want_dvar ? sl.pT + (size_t)g0 * npad * PT : nullptr,
+                      sl.pX + (size_t)g0 * xstar_stride, dmstar ? w.dms + (size_t)g0 * m * d : nullptr,
+                      w.jac + (size_t)g0 * m * d, want_dvar ? w.jac + njac + (size_t)g0 * m * d : nullptr, sl.mask,
+                      xstar_stride, (int)b->n, (int)npad, d, (int)m, b->kind, ta.s0, ta.mc, g0};
+    if ((rc = launch_predict_jac(ja, g1 - g0, ss))) return rc;
+    b->ctx->launches++;
+    return 0;
+  };
+  if ((rc = predict_tiles(b, 0, 0, count, 1, m, xstar_stride, mstar != nullptr, want_var ? sl.pvar : nullptr,
+                          want_T ? sl.pT : nullptr, sl.tm_T68, false, false, jac)))
+    return rc;
   GPRB_CUDA(cudaMemcpyAsync(sl.h_out, sl.pmu, sizeof(double) * nout, cudaMemcpyDeviceToHost, st));
   if (want_var) GPRB_CUDA(cudaMemcpyAsync(sl.h_out + nout, sl.pvar, sizeof(double) * nout, cudaMemcpyDeviceToHost, st));
   GPRB_CUDA(cudaEventRecord(sl.t1, st));
@@ -1722,7 +1649,7 @@ int gprb_predict_grad(gprb_batch* b, int64_t m, const double* Xstar, int64_t xst
   GPRB_CUDA(cudaMemcpyAsync(dmu, b->pg.jac, sizeof(double) * njac, cudaMemcpyDeviceToHost, st));
   if (dvar) GPRB_CUDA(cudaMemcpyAsync(dvar, b->pg.jac + njac, sizeof(double) * njac, cudaMemcpyDeviceToHost, st));
   GPRB_CUDA(cudaStreamSynchronize(st));
-  if ((rc = postcov_finish_time(b))) return rc;
+  if ((rc = slot_wait(sl))) return rc;
   memcpy(mu, sl.h_out, sizeof(double) * nout);
   if (var) memcpy(var, sl.h_out + nout, sizeof(double) * nout);
   return GPRB_OK;

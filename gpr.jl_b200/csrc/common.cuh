@@ -8,6 +8,7 @@
 #include <vector>
 
 #include "../../include/gprb200.h"
+#include "kernels.h"
 
 namespace gprb {
 
@@ -186,7 +187,6 @@ struct gprb_batch {
   double* diag_off = nullptr;     // [B] fixed per-GP diagonal offset (gprb_batch_set_diag_offset), default 0
   double* logdet_part = nullptr;  // [B][J]
   int32_t* fail = nullptr;        // [B] 0 ok / first failing column+1 (LAPACK info)
-  int32_t* info = nullptr;        // [B] device copy of the per-GP info
   double* mll = nullptr;          // [B]
   double* grad = nullptr;         // [B][P]
   double* grad_part = nullptr;    // [B][ntiles][P+1] per-tile partial sums (deterministic 2-pass reduction)
@@ -218,12 +218,10 @@ struct gprb_batch {
   gprb_postcov_ws pc;             // full covariance / posterior draws (gprb_predict_cov, gprb_sample_posterior)
   gprb_loo_ws loo;                // leave-one-out cross-validation (gprb_eval_loo)
   gprb_predgrad_ws pg;            // predictive gradients (gprb_predict_grad)
-  // TMA tensor maps of the tile GEMM's operands (encoded once per batch; box = padded rows x KT columns x 1 GP)
-  CUtensorMap tm_L132, tm_L68;     // Lm  [B][npad][npad]
-  CUtensorMap tm_A68;              // A   [B][npad][npad] (L2 prefetch of the K tiles the Cholesky modes start from)
-  CUtensorMap tm_DT132, tm_DT68;   // DinvT [B][J*128][128]
-  CUtensorMap tm_D132;             // Dinv  [B][J*128][128]
-  CUtensorMap tm_LT;               // Lm with box = KT rows x 128 columns (GEMM_BWD_ROW reads L's lower tiles transposed)
+  // The tile GEMM's arguments on the batch's factor, which every tile-GEMM launch on it starts from: Lm, A (Cin), Dinv,
+  // DinvT, KinvD, fail, their strides and the TMA tensor maps of the operands, encoded once per batch (box = padded rows
+  // x KT columns x 1 GP; tm_LT: Lm with box = KT rows x 128 columns, GEMM_BWD_ROW reads L's lower tiles transposed)
+  gprb::GemmArgs gemm{};
   std::vector<cudaEvent_t> gemm_ev;  // profiling: start/stop pairs around every tile-GEMM launch
   int gemm_ev_used = 0;
   std::vector<double> gemm_ms;  // per tile-GEMM launch time of the last profiled evaluation, launch order
