@@ -153,11 +153,15 @@ __global__ void __launch_bounds__(PW_THREADS, 1) k_assemble(AssembleArgs g) {
 //   z_ip = sqrt(w_p) (x_ip - x_0p)         scaled inputs, centred at the dataset's first sample (constant input
 //                                          dimensions become exact zeros), built in shared memory per tile
 //   r2_ij = |z_i|^2 + |z_j|^2 - 2 z_i.z_j  the d-long contraction z_i.z_j runs as DMMA.8x8x4 tiles (SASS DMMA)
-// The expansion loses accuracy by ~ (d/4 + 2) eps (|z_i|^2 + |z_j|^2) in r2, i.e. half of that relative in K.
+// The expansion loses accuracy by an absolute delta ~ (d/4 + 2) eps (|z_i|^2 + |z_j|^2) in r2.  SEArd and Matern-3/2, 5/2
+// are smooth in r2, so that is a relative error of about delta / 2 in K.  Matern-1/2, k = s_f^2 exp(-r), is not: its
+// relative error is delta / (2 r), and sqrt(delta) for a duplicated sample (r = 0).
 // Parity with the reference's direct differences (1e-12 relative on K) is kept by a guard: pairs whose norm sum
 // exceeds GRAM_SMAX and whose K is not an underflow (r2 below the per-kernel cut-off) are recomputed with direct differences of the
-// raw inputs.  With trajectory data and sane length-scales the guard never fires (|z|^2 << 1); extreme
-// length-scales (config.json has l down to 1e-4) take the slow exact path per element.
+// raw inputs.  With trajectory data and sane length-scales that part never fires (|z|^2 << 1); extreme
+// length-scales (config.json has l down to 1e-4) take the slow exact path per element.  Matern-1/2 also recomputes the
+// off-diagonal pairs that are close relative to their norm sum (GRAM_CLOSE12): with delta <= 4e-15 ssum, r >= 0.02 ssum
+// keeps delta / (2 r) <= 1e-13.  Consecutive states of a trajectory and repeated samples are such pairs.
 // One CTA (256 threads, 8 warps of 32 x 32 register tiles) = 128 rows x 64 columns of a lower tile; two CTAs per SM.
 // ---------------------------------------------------------------------------------------------------------------
 constexpr int GA_THREADS = 256;
@@ -166,6 +170,7 @@ constexpr int GA_LDJ = GA_CW + 4;     // padded row of the column-input tile (co
 constexpr int GA_LDC = NB + 2;        // column stride of the cross-term tile: the accumulator stores of a half-warp hit
                                       // (2 t) GA_LDC + g, distinct modulo 16 only for a stride = 2 mod 8 (132 gave 2-way conflicts)
 constexpr double GRAM_SMAX = 16.0;    // (d/4 + 2) eps * 16 < 4e-14 for d <= 62
+constexpr double GRAM_CLOSE12 = 4e-4; // Matern-1/2: exact path while r2 < GRAM_CLOSE12 ssum^2, i.e. r < 0.02 ssum
 // Pairs whose kernel value underflows to zero are exact zeros either way and skip the exact path.  SEArd: exp(-r2/2)
 // underflows beyond r2 = 1500.  Matern: k ~ exp(-c r) with c = 1, sqrt 3, sqrt 5 only underflows beyond r = 750 / c.
 // The test is made on a LOWER bound of r2 (the expansion errs by <= (d/4 + 2) eps (|z_i|^2 + |z_j|^2) < 4e-15 ssum), so
@@ -176,8 +181,8 @@ __device__ __forceinline__ double gram_r2cut() {
 }
 
 // CTAS = resident CTAs per SM the kernel is compiled for: 3 (80 registers, a few spilled words in the prologue) whenever
-// three 71 KB input/cross-term regions fit (d <= 28: 5.7 -> 5.15 ms per 400 GPs, the phases of three CTAs interleave
-// better than those of two), else 2.
+// three CTAs' shared memory fits an SM (d <= 44, up to 72 KB each:5.7 -> 5.15 ms per 400 GPs at d = 26, the phases of
+// three CTAs interleave better than those of two), else 2.
 template <int KIND, int CTAS>
 __global__ void __launch_bounds__(GA_THREADS, CTAS) k_assemble_gram(AssembleArgs g) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -292,7 +297,10 @@ __global__ void __launch_bounds__(GA_THREADS, CTAS) k_assemble_gram(AssembleArgs
     const int c = c0 + cl;
     const double ssum = nr + nj[cl];
     double r2 = fmax(ssum - 2.0 * Cs[cl * GA_LDC + rl], 0.0);
-    if (ssum > GRAM_SMAX && r2 - 4e-15 * ssum < gram_r2cut<KIND>() && rr < n && c < n) {  // exact path: direct differences of the raw inputs
+    // r2 - 4e-15 ssum is a lower bound of the true r2: a pair is never misclassified as far apart
+    const bool far_out = ssum > GRAM_SMAX;
+    const bool close12 = KIND == GPRB_KERNEL_MAT12_ARD && rr != c && r2 - 4e-15 * ssum < GRAM_CLOSE12 * ssum * ssum;
+    if ((far_out || close12) && r2 - 4e-15 * ssum < gram_r2cut<KIND>() && rr < n && c < n) {  // exact path: direct differences of the raw inputs
       r2 = 0.0;
       for (int p = 0; p < d; ++p) {
         const double df = Xt[(int64_t)p * g.npad + rr] - Xt[(int64_t)p * g.npad + c];
