@@ -10,6 +10,7 @@
 #include <limits>
 #include <new>
 #include <type_traits>
+#include <unordered_set>
 
 #include "common.cuh"
 #include "kernels.h"
@@ -75,6 +76,20 @@ static int encode_factor_maps(GemmArgs& ga, uint64_t B) {
   return 0;
 }
 
+// The batch's tile-GEMM prototype (gprb_batch::gemm) on its current buffers, n and npad, tensor maps included.
+static int set_batch_gemm(gprb_batch* b) {
+  const int64_t mat = b->npad * b->npad, dinv = (int64_t)b->J * NB * NB;
+  b->gemm = GemmArgs{b->Lm, b->DinvT, b->Dinv, b->A, b->Lm, b->KinvD, nullptr, mat, dinv, (int)b->npad, b->J, 0, GEMM_CHOL_DIAG,
+                     (int)((b->n + KT - 1) / KT * KT)};
+  b->gemm.fail = b->fail;
+  int rc;
+  if ((rc = encode_factor_maps(b->gemm, (uint64_t)b->B)) ||
+      (rc = make_tensor_map(&b->gemm.tm_LT, b->Lm, (uint64_t)b->npad, (uint64_t)b->npad, (uint64_t)b->B, (uint64_t)b->npad,
+                            (uint64_t)mat, KT, NB)))
+    return rc;
+  return 0;
+}
+
 // make_posdef! after one factorisation attempt with status f (LAPACK info; < 0: no state or non-finite input): either one
 // more jitter is due (tries counts it, returns true) or info gets the final outcome - the jitter count, -2, or -1 when
 // the matrix is still indefinite after MAX_JITTER jitters.
@@ -91,6 +106,15 @@ static int dev_alloc(T** p, size_t count) {
   cudaError_t e = cudaMalloc((void**)p, count * sizeof(T));
   if (e != cudaSuccess) return cuda_fail(e, "cudaMalloc", __FILE__, __LINE__);
   return 0;
+}
+
+// The datasets of a batch, each once, in order of first use by GP index.
+static std::vector<gprb_dataset*> distinct_datasets(const gprb_batch* b) {
+  std::vector<gprb_dataset*> out;
+  std::unordered_set<gprb_dataset*> seen;
+  for (gprb_dataset* d : b->ds)
+    if (seen.insert(d).second) out.push_back(d);
+  return out;
 }
 
 static void free_batch(gprb_batch* b) {
@@ -142,9 +166,12 @@ static void free_batch(gprb_batch* b) {
 // `ops` != nullptr: the launches are not issued but appended (as closures) to `ops`, so that run_pipeline can issue the
 // launches of all stream groups interleaved - every group then starts at once instead of one enqueue time (0.3 ms of host
 // work per group) after the previous one, which matters for short passes (50 GPs per GPU in the 8-GPU strong split).
+// j0 > 0 (gprb_batch_append, left-looking, value only): the block rows < j0 of K, L, Dinv and the logdet partials are
+// resident and final - only the lower tiles in block rows >= j0 are assembled, block columns j < j0 get their CHOL_COL
+// tiles in those rows, block columns >= j0 the whole left-looking step, and the solve runs over the whole factor.
 using LaunchOps = std::vector<std::function<int()>>;
 static int enqueue_pipeline(gprb_batch* b, int off, int count, int ngrad, int nreuse, bool right_looking, cudaStream_t st,
-                            bool prof, LaunchOps* ops = nullptr) {
+                            bool prof, LaunchOps* ops = nullptr, int j0 = 0) {
   if (count <= 0) return 0;
   const bool with_grad = ngrad > 0;
   const int32_t* glist = b->list + off;     // inverse + gradient: glist[0 .. ngrad)
@@ -210,6 +237,7 @@ static int enqueue_pipeline(gprb_batch* b, int off, int count, int ngrad, int nr
   // Small passes are latency bound (one dependent chain of 3 J launches): they use the right-looking factorisation,
   // whose launches are short and wide, instead of the left-looking one, whose k-loops grow with the column index.
   AssembleArgs aa{b->Xtptr, b->theta, b->jitter, b->A, nullptr, b->fail, list, ms, (int)b->n, (int)b->npad, b->d, J, b->kind};
+  aa.tile0 = j0 * (j0 + 1) / 2;
   if (right_looking) aa.A2 = b->Lm;
   if ((rc = run([aa, count, st] { return launch_assemble(aa, count, st); }))) return rc;
   ++launches;
@@ -218,6 +246,13 @@ static int enqueue_pipeline(gprb_batch* b, int off, int count, int ngrad, int nr
   if (right_looking) ga.Cin = b->Lm;  // S lives (and is updated in place) in the lower tiles of Lm
   for (int j = 0; j < J; ++j) {
     ga.step = j;
+    if (j < j0) {
+      ga.mode = GEMM_CHOL_COL; ga.row0 = j0;
+      if ((rc = gemm(ga, J - j0))) return rc;
+      ++launches;
+      ga.row0 = 0;
+      continue;
+    }
     if (!right_looking && j > 0) {  // S(0,0) = K(0,0): k_diag_factor reads block column 0 straight from A
       ga.mode = GEMM_CHOL_DIAG;
       if ((rc = gemm(ga, 1))) return rc;
@@ -270,7 +305,7 @@ static int enqueue_pipeline(gprb_batch* b, int off, int count, int ngrad, int nr
 
 // One stream group of an evaluation pass: list[off .. off+count), the first ngrad of them with gradient, the first
 // nreuse of those on the resident factorisation.
-struct Group { int off, count, ngrad, nreuse; bool rl; };
+struct Group { int off, count, ngrad, nreuse; bool rl; int j0 = 0; };
 
 // Order the active GPs of a pass into stream groups inside list_host: the value+gradient GPs and the value-only GPs
 // are each dealt evenly over the groups (equal work per stream), gradient GPs first inside every group.
@@ -290,7 +325,7 @@ static std::vector<Group> build_groups(gprb_batch* b, const std::vector<int32_t>
     const int r0 = cut(reuse_gps.size(), s), r1 = cut(reuse_gps.size(), s + 1);
     const int g0 = cut(grad_gps.size(), s), g1 = cut(grad_gps.size(), s + 1);
     const int v0 = cut(val_gps.size(), s), v1 = cut(val_gps.size(), s + 1);
-    Group g{off, (r1 - r0) + (g1 - g0) + (v1 - v0), (r1 - r0) + (g1 - g0), r1 - r0, !b->profiling && total <= b->rl_max};
+    Group g{off, (r1 - r0) + (g1 - g0) + (v1 - v0), (r1 - r0) + (g1 - g0), r1 - r0, !b->profiling && total <= b->rl_max, 0};
     for (int k = r0; k < r1; ++k) b->list_host[off++] = reuse_gps[k];
     for (int k = g0; k < g1; ++k) b->list_host[off++] = grad_gps[k];
     for (int k = v0; k < v1; ++k) b->list_host[off++] = val_gps[k];
@@ -306,7 +341,7 @@ static int run_pipeline(gprb_batch* b, const std::vector<Group>& groups) {
   if (groups.empty()) return 0;
   if (b->profiling) {
     const Group& g = groups[0];
-    if ((rc = enqueue_pipeline(b, g.off, g.count, g.ngrad, g.nreuse, g.rl, b->stream[0], true))) return rc;
+    if ((rc = enqueue_pipeline(b, g.off, g.count, g.ngrad, g.nreuse, g.rl, b->stream[0], true, nullptr, g.j0))) return rc;
     GPRB_CUDA(cudaStreamSynchronize(b->stream[0]));
     float ms = 0.f;
     const int last = g.ngrad > 0 ? 5 : 3;
@@ -334,7 +369,8 @@ static int run_pipeline(gprb_batch* b, const std::vector<Group>& groups) {
   for (size_t s = 0; s < groups.size(); ++s) {
     const Group& g = groups[s];
     if (s > 0) GPRB_CUDA(cudaStreamWaitEvent(b->stream[s], b->join[0], 0));
-    if ((rc = enqueue_pipeline(b, g.off, g.count, g.ngrad, g.nreuse, g.rl, b->stream[s], false, groups.size() > 1 ? &ops[s] : nullptr)))
+    if ((rc = enqueue_pipeline(b, g.off, g.count, g.ngrad, g.nreuse, g.rl, b->stream[s], false, groups.size() > 1 ? &ops[s] : nullptr,
+                               g.j0)))
       return rc;
     longest = std::max(longest, ops[s].size());
   }
@@ -416,10 +452,10 @@ static int eval_pass(gprb_batch* b, const double* theta_host, const uint8_t* mod
       b->state_ok[gp] = info[gp] >= 0;
       b->inv_ok[gp] = pass == 0 && info[gp] >= 0;
       b->v_ok[gp] = b->inv_ok[gp];
+      if (info[gp] >= 0) b->info_last[gp] = info[gp];  // the jitter rung of the resident state (gprb_batch_append reads it)
       if (theta_host && info[gp] >= 0) {  // remember what is resident now
         memcpy(b->theta_last.data() + (size_t)gp * P, theta_host + (size_t)gp * P, sizeof(double) * P);
         b->theta_valid[gp] = 1;
-        b->info_last[gp] = info[gp];
         b->ds_ver[gp] = b->ds[gp]->version;
       }
     }
@@ -503,7 +539,7 @@ using namespace gprb;
 
 extern "C" {
 
-int gprb_version(void) { return 302; }
+int gprb_version(void) { return 303; }
 const char* gprb_last_error(void) { return g_err.c_str(); }
 
 int gprb_init(gprb_ctx** out, int device) {
@@ -763,6 +799,7 @@ int gprb_batch_create(gprb_ctx* ctx, int32_t B, gprb_dataset* const* ds, const d
   b->ctx = ctx; b->B = B; b->n = ds[0]->n; b->d = ds[0]->d; b->P = b->d + 2; b->kind = kernel_kind;
   b->npad = ds[0]->npad; b->J = (int)(b->npad / NB);
   b->ds.assign(ds, ds + B);
+  for (gprb_dataset* u : distinct_datasets(b)) u->users++;
   const size_t mat = (size_t)b->npad * b->npad, dinv = (size_t)b->J * NB * NB;
   const size_t ntiles = (size_t)b->J * (b->J + 1) / 2;
   int rc = 0;
@@ -783,12 +820,7 @@ int gprb_batch_create(gprb_ctx* ctx, int32_t B, gprb_dataset* const* ds, const d
       rc = cuda_fail(e, "cudaMallocHost", __FILE__, __LINE__);
       break;
     }
-    b->gemm = GemmArgs{b->Lm, b->DinvT, b->Dinv, b->A, b->Lm, b->KinvD, nullptr, (int64_t)mat, (int64_t)dinv, (int)b->npad, b->J,
-                       0, GEMM_CHOL_DIAG, (int)((b->n + KT - 1) / KT * KT)};
-    b->gemm.fail = b->fail;
-    if ((rc = encode_factor_maps(b->gemm, B)) ||
-        (rc = make_tensor_map(&b->gemm.tm_LT, b->Lm, (uint64_t)b->npad, (uint64_t)b->npad, B, (uint64_t)b->npad, mat, KT, NB)))
-      break;
+    if ((rc = set_batch_gemm(b))) break;
     b->nstreams = 4;
     b->rl_max = 24;
     if (const char* ev = getenv("GPRB200_RL_MAX")) b->rl_max = atoi(ev);
@@ -826,7 +858,11 @@ int gprb_batch_create(gprb_ctx* ctx, int32_t B, gprb_dataset* const* ds, const d
     }
     rc = upload_targets(b, ymm);
   } while (0);
-  if (rc) { free_batch(b); return rc; }
+  if (rc) {
+    for (gprb_dataset* u : distinct_datasets(b)) u->users--;
+    free_batch(b);
+    return rc;
+  }
   *out = b;
   return GPRB_OK;
 }
@@ -853,7 +889,11 @@ int gprb_batch_set_diag_offset(gprb_batch* b, const double* offset) {
 }
 
 int gprb_batch_destroy(gprb_batch* b) {
-  if (b) { cudaSetDevice(b->ctx->device); cudaDeviceSynchronize(); }
+  if (b) {
+    cudaSetDevice(b->ctx->device);
+    cudaDeviceSynchronize();
+    for (gprb_dataset* u : distinct_datasets(b)) u->users--;
+  }
   free_batch(b);
   return GPRB_OK;
 }
@@ -1653,6 +1693,220 @@ int gprb_predict_grad(gprb_batch* b, int64_t m, const double* Xstar, int64_t xst
   memcpy(mu, sl.h_out, sizeof(double) * nout);
   if (var) memcpy(var, sl.h_out + nout, sizeof(double) * nout);
   return GPRB_OK;
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------------
+// Appending samples (gprb_batch_append; GaussianProcesses ElasticGPE append!).  The left-looking factorisation computes
+// the tiles of block row i from K's block rows i and j and from L(., k < j) only, and the assembly centres at the
+// dataset's first sample: with j0 = floor(n_old / 128), the block rows < j0 of K, L, the inverted diagonal blocks and the
+// logdet partials on n_old + k samples are bit for bit the resident ones.  The incremental pass (enqueue_pipeline with j0)
+// recomputes the rest, so a GP ends in exactly the state gprb_eval(theta, value only) leaves on the enlarged data.
+
+// The leading rows x cols of every GP's column-major block, from leading dimension lds (blocks of lds x scols) to ldd
+// (blocks of ldd x dcols), all GPs in one 3-D copy.
+static int restride(double* dst, int64_t ldd, int64_t dcols, const double* src, int64_t lds, int64_t scols, int64_t rows,
+                    int64_t cols, int B, cudaStream_t st) {
+  cudaMemcpy3DParms p = {};
+  p.srcPtr = make_cudaPitchedPtr(const_cast<double*>(src), sizeof(double) * lds, sizeof(double) * lds, scols);
+  p.dstPtr = make_cudaPitchedPtr(dst, sizeof(double) * ldd, sizeof(double) * ldd, dcols);
+  p.extent = make_cudaExtent(sizeof(double) * rows, cols, B);
+  p.kind = cudaMemcpyDeviceToDevice;
+  GPRB_CUDA(cudaMemcpy3DAsync(&p, st));
+  return 0;
+}
+
+// Move one [B][ld][ld] matrix to a new allocation of leading dimension ld1, keeping its leading keep x keep block; the
+// old allocation is freed only after the copy, so a failed allocation leaves *p as it was.
+static int move_matrix(gprb_batch* b, double** p, int64_t ld0, int64_t ld1, int64_t keep) {
+  double* q = nullptr;
+  int rc = dev_alloc(&q, (size_t)b->B * ld1 * ld1);
+  if (rc) return rc;
+  if (!(rc = restride(q, ld1, ld1, *p, ld0, ld0, keep, keep, b->B, b->stream[0]))) {
+    cudaError_t e = cudaStreamSynchronize(b->stream[0]);
+    if (e != cudaSuccess) rc = cuda_fail(e, "cudaStreamSynchronize(move_matrix)", __FILE__, __LINE__);
+  }
+  if (rc) { cudaFree(q); return rc; }
+  cudaFree(*p);
+  *p = q;
+  return 0;
+}
+
+// The [B][npad] / [B][J] buffers of a batch at a new npad, J (allocated all or none).
+struct GrownBuffers {
+  double *Dinv = nullptr, *DinvT = nullptr, *KinvD = nullptr, *logdet = nullptr, *gpart = nullptr, *ymm = nullptr,
+         *alpha = nullptr, *zbuf = nullptr;
+  void release() {
+    for (double* p : {Dinv, DinvT, KinvD, logdet, gpart, ymm, alpha, zbuf}) cudaFree(p);
+    *this = GrownBuffers{};
+  }
+};
+
+static int grow_alloc(gprb_batch* b, GrownBuffers& g, int64_t np1, int J1) {
+  const size_t B = (size_t)b->B, dinv = (size_t)J1 * NB * NB, ntiles = (size_t)J1 * (J1 + 1) / 2;
+  int rc;
+  if ((rc = dev_alloc(&g.Dinv, dinv * B)) || (rc = dev_alloc(&g.DinvT, dinv * B)) || (rc = dev_alloc(&g.KinvD, dinv * B)) ||
+      (rc = dev_alloc(&g.logdet, B * J1)) || (rc = dev_alloc(&g.gpart, B * ntiles * GRAD_PARTS_PER_TILE * b->P)) ||
+      (rc = dev_alloc(&g.ymm, B * np1)) || (rc = dev_alloc(&g.alpha, B * np1)) || (rc = dev_alloc(&g.zbuf, B * np1)))
+    g.release();
+  return rc;
+}
+
+// Grow-only workspaces whose shape or tensor maps derive from npad or J: released, the next call allocates them again.
+// (gprb_predgrad_ws is sized by m and d only.)
+static void release_npad_workspaces(gprb_batch* b) {
+  for (gprb_predict_slot& sl : b->ps) {
+    cudaFree(sl.pT); sl.pT = nullptr; sl.pT_cap = 0; sl.tm_T_cap = 0;
+    cudaFree(sl.pmupart); sl.pmupart = nullptr; sl.pmupart_cap = 0;
+  }
+  cudaFree(b->pc.T); b->pc.T = nullptr; b->pc.T_cap = 0;
+  loo_free_groups(b->loo);
+}
+
+extern "C" {
+
+int gprb_batch_append(gprb_batch* b, int64_t k, const double* const* Xnew, int64_t ldx, const double* ymm_new, double* mll,
+                      int32_t* info) {
+  GPRB_REQUIRE(b && Xnew && ymm_new, "gprb_batch_append: NULL argument");
+  GPRB_REQUIRE(k >= 1, "gprb_batch_append: k must be >= 1");
+  GPRB_REQUIRE(ldx >= b->d, "gprb_batch_append: ldx < d");
+  GPRB_REQUIRE(b->n + k <= (1 << 20), "gprb_batch_append: n + k out of range");
+  GPRB_REQUIRE(!b->ps[0].pending && !b->ps[1].pending,
+               "gprb_batch_append: a prediction is in flight - call gprb_predict_wait first");
+  const std::vector<gprb_dataset*> uds = distinct_datasets(b);
+  const int T = (int)uds.size();
+  for (int t = 0; t < T; ++t) {
+    GPRB_REQUIRE(Xnew[t] != nullptr, "gprb_batch_append: NULL input block");
+    GPRB_REQUIRE(uds[t]->users == 1, "gprb_batch_append: a dataset of the batch is also used by another live batch");
+  }
+  GPRB_CUDA(cudaSetDevice(b->ctx->device));
+  const int B = b->B, P = b->P, d = b->d;
+  cudaStream_t st = b->stream[0];
+  const int64_t n0 = b->n, np0 = b->npad, n1 = n0 + k, np1 = (n1 + NB - 1) / NB * NB;
+  const int J0 = b->J, J1 = (int)(np1 / NB), j0 = (int)(n0 / NB);
+  if ((int)b->theta_valid.size() != B) {
+    b->theta_valid.assign(B, 0); b->theta_last.assign((size_t)B * P, 0.0); b->info_last.assign(B, 0); b->ds_ver.assign(B, 0);
+  }
+  // theta of every resident state (gprb_eval_device states included: the device copy is the one that was evaluated)
+  std::vector<double> theta((size_t)B * P);
+  GPRB_CUDA(cudaStreamSynchronize(st));
+  GPRB_CUDA(cudaMemcpy(theta.data(), b->theta, sizeof(double) * B * P, cudaMemcpyDeviceToHost));
+  // incremental: a state factorised without jitter (the jitter 1e-6 tr(K)/n changes with n) that keeps whole block rows
+  std::vector<uint8_t> mode(B, 0);
+  std::vector<int32_t> inc, fall;
+  for (int i = 0; i < B; ++i) {
+    if (!b->state_ok[i]) continue;
+    mode[i] = 1;
+    (b->info_last[i] == 0 && j0 >= 1 ? inc : fall).push_back(i);
+  }
+
+  // ---- device memory: every allocation before anything is freed or overwritten
+  gprb_slab* sl = new (std::nothrow) gprb_slab();
+  GPRB_REQUIRE(sl != nullptr, "gprb_batch_append: out of host memory");
+  int rc;
+  if ((rc = dev_alloc(&sl->X, (size_t)T * d * n1)) || (rc = dev_alloc(&sl->Xt, (size_t)T * d * np1))) {
+    cudaFree(sl->X); cudaFree(sl->Xt); delete sl;
+    return rc;
+  }
+  if (np1 > np0) {
+    release_npad_workspaces(b);
+    GrownBuffers g;
+    // one large matrix at a time: the peak is the resident buffers plus one new [B][npad][npad] copy
+    if ((rc = grow_alloc(b, g, np1, J1)) || (rc = move_matrix(b, &b->A, np0, np1, np0))) {
+      g.release(); cudaFree(sl->X); cudaFree(sl->Xt); delete sl;
+      return rc;
+    }
+    if ((rc = move_matrix(b, &b->Lm, np0, np1, np0))) {
+      if (move_matrix(b, &b->A, np1, np0, np0) == 0) set_batch_gemm(b);  // back to the old stride (its memory was just freed)
+      else set_error("gprb_batch_append: out of device memory, and the batch could not be restored");
+      g.release(); cudaFree(sl->X); cudaFree(sl->Xt); delete sl;
+      return rc;
+    }
+    const size_t dn0 = (size_t)J0 * NB * NB, dn1 = (size_t)J1 * NB * NB;
+    // k_diag_factor writes only the triangular halves of the inverted diagonal blocks: the other halves stay zero
+    GPRB_CUDA(cudaMemsetAsync(g.Dinv, 0, sizeof(double) * dn1 * B, st));
+    GPRB_CUDA(cudaMemsetAsync(g.DinvT, 0, sizeof(double) * dn1 * B, st));
+    GPRB_CUDA(cudaMemsetAsync(g.ymm, 0, sizeof(double) * np1 * B, st));  // zero padding
+    GPRB_CUDA(cudaMemcpy2DAsync(g.Dinv, sizeof(double) * dn1, b->Dinv, sizeof(double) * dn0, sizeof(double) * dn0, B,
+                                cudaMemcpyDeviceToDevice, st));
+    GPRB_CUDA(cudaMemcpy2DAsync(g.DinvT, sizeof(double) * dn1, b->DinvT, sizeof(double) * dn0, sizeof(double) * dn0, B,
+                                cudaMemcpyDeviceToDevice, st));
+    GPRB_CUDA(cudaMemcpy2DAsync(g.logdet, sizeof(double) * J1, b->logdet_part, sizeof(double) * J0, sizeof(double) * J0, B,
+                                cudaMemcpyDeviceToDevice, st));
+    GPRB_CUDA(cudaMemcpy2DAsync(g.ymm, sizeof(double) * np1, b->ymm, sizeof(double) * np0, sizeof(double) * n0, B,
+                                cudaMemcpyDeviceToDevice, st));
+    GPRB_CUDA(cudaStreamSynchronize(st));
+    for (double* p : {b->Dinv, b->DinvT, b->KinvD, b->logdet_part, b->grad_part, b->ymm, b->alpha, b->zbuf}) cudaFree(p);
+    b->Dinv = g.Dinv; b->DinvT = g.DinvT; b->KinvD = g.KinvD; b->logdet_part = g.logdet; b->grad_part = g.gpart;
+    b->ymm = g.ymm; b->alpha = g.alpha; b->zbuf = g.zbuf;
+  }
+
+  // ---- the grown data: old samples, then the new ones, into the new slab; y - m(X) of the new samples
+  for (int t = 0; t < T; ++t) {
+    double* x = sl->X + (size_t)t * d * n1;
+    GPRB_CUDA(cudaMemcpyAsync(x, uds[t]->X, sizeof(double) * d * n0, cudaMemcpyDeviceToDevice, st));
+    GPRB_CUDA(cudaMemcpy2DAsync(x + (size_t)d * n0, sizeof(double) * d, Xnew[t], sizeof(double) * ldx, sizeof(double) * d, k,
+                                cudaMemcpyHostToDevice, st));
+  }
+  if ((rc = launch_transpose_inputs_batched(sl->X, sl->Xt, (int)n1, (int)np1, d, T, st))) return rc;
+  b->ctx->launches++;
+  GPRB_CUDA(cudaMemcpy2DAsync(b->ymm + n0, sizeof(double) * np1, ymm_new, sizeof(double) * k, sizeof(double) * k, B,
+                              cudaMemcpyHostToDevice, st));
+  GPRB_CUDA(cudaStreamSynchronize(st));
+  sl->count = T; sl->refs = T;
+  for (int t = 0; t < T; ++t) {
+    gprb_dataset* ds = uds[t];
+    if (ds->slab) {
+      if (--ds->slab->refs == 0) { cudaFree(ds->slab->X); cudaFree(ds->slab->Xt); delete ds->slab; }
+    } else {
+      cudaFree(ds->X); cudaFree(ds->Xt);
+    }
+    ds->n = n1; ds->npad = np1;
+    ds->X = sl->X + (size_t)t * d * n1;
+    ds->Xt = sl->Xt + (size_t)t * d * np1;
+    ds->slab = sl; ds->slab_index = t;
+    ds->version++;
+  }
+  {
+    std::vector<const double*> xp(B), xtp(B);
+    for (int i = 0; i < B; ++i) { xp[i] = b->ds[i]->X; xtp[i] = b->ds[i]->Xt; }
+    GPRB_CUDA(cudaMemcpy(b->Xptr, xp.data(), sizeof(double*) * B, cudaMemcpyHostToDevice));
+    GPRB_CUDA(cudaMemcpy(b->Xtptr, xtp.data(), sizeof(double*) * B, cudaMemcpyHostToDevice));
+  }
+  b->n = n1; b->npad = np1; b->J = J1;
+  if ((rc = set_batch_gemm(b))) return rc;
+  std::fill(b->inv_ok.begin(), b->inv_ok.end(), (uint8_t)0);
+  std::fill(b->v_ok.begin(), b->v_ok.end(), (uint8_t)0);
+
+  // ---- incremental pass over the stream groups; a GP whose new diagonal blocks fail a pivot joins the fallback
+  std::vector<int32_t> inf(B, 0);
+  if (!inc.empty()) {
+    std::vector<Group> groups = build_groups(b, {}, {}, inc);
+    for (Group& g : groups) { g.rl = false; g.j0 = j0; }
+    GPRB_CUDA(cudaMemcpyAsync(b->list, b->list_host, sizeof(int32_t) * B, cudaMemcpyHostToDevice, st));
+    if ((rc = run_pipeline(b, groups))) return rc;
+    GPRB_CUDA(cudaMemcpyAsync(b->fail_host, b->fail, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, st));
+    GPRB_CUDA(cudaStreamSynchronize(st));
+    for (int gp : inc) {
+      if (b->fail_host[gp] != 0) { fall.push_back(gp); continue; }
+      memcpy(b->theta_last.data() + (size_t)gp * P, theta.data() + (size_t)gp * P, sizeof(double) * P);
+      b->theta_valid[gp] = 1; b->info_last[gp] = 0; b->ds_ver[gp] = b->ds[gp]->version;
+    }
+  }
+  // ---- fallback: an ordinary value-only evaluation with the whole make_posdef! ladder at the resident theta
+  if (!fall.empty()) {
+    std::vector<uint8_t> fm(B, 0);
+    for (int gp : fall) fm[gp] = 1;
+    std::vector<int32_t> finf;
+    if ((rc = evaluate_modes(b, theta.data(), fm.data(), finf))) return rc;
+    for (int gp : fall) inf[gp] = finf[gp];
+  }
+  std::vector<double> tmll;
+  std::vector<int32_t> tinfo;
+  if (!mll) { tmll.resize(B); mll = tmll.data(); }
+  if (!info) { tinfo.resize(B); info = tinfo.data(); }
+  return download_results(b, mode.data(), inf, nullptr, mll, nullptr, info);
 }
 
 }  // extern "C"

@@ -15,5 +15,5 @@ for f in api tilegemm covgrad factor predict postcov loo predgrad lbfgs comm; do
   fi
 done
 for p in "${pids[@]:-}"; do [ -n "$p" ] && wait "$p"; done
-"$NVCC" -shared -o "$OUT" build/*.o -lcudart -ldl
+"$NVCC" -gencode arch=compute_100a,code=sm_100a -shared -o "$OUT" build/*.o -lcudart -ldl
 echo "built $OUT"

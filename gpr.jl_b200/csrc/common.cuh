@@ -94,6 +94,7 @@ struct gprb_dataset {
   uint64_t version = 0;  // bumped by every upload (state reuse compares it)
   gprb_slab* slab = nullptr;  // non-null: X / Xt point into the slab (member `slab_index`)
   int32_t slab_index = 0;
+  int32_t users = 0;     // live batches that use the dataset (gprb_batch_append grows only a dataset no other batch reads)
 };
 
 // One prediction pipeline of a batch (gprb_predict_async slot): own streams, staging and scratch, so that two groups

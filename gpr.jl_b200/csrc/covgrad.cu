@@ -108,7 +108,7 @@ __global__ void __launch_bounds__(PW_THREADS, 1) k_assemble(AssembleArgs g) {
   uint64_t* bar = reinterpret_cast<uint64_t*>(w + MAX_D);
   const int gp = g.list ? g.list[blockIdx.y] : blockIdx.y;
   int ti, tj;
-  lower_tile(blockIdx.x, ti, tj);
+  lower_tile(blockIdx.x + g.tile0, ti, tj);
   const double* th = g.theta + (int64_t)gp * (g.d + 2);
   if (threadIdx.x < g.d) w[threadIdx.x] = exp(-2.0 * th[1 + threadIdx.x]);
   stage_inputs(g.Xt[gp], g.npad, g.d, ti, tj, Xi, Xj, bar);
@@ -197,7 +197,7 @@ __global__ void __launch_bounds__(GA_THREADS, CTAS) k_assemble_gram(AssembleArgs
   double* nj = ni + NB;                                // [GA_CW]  |z_j|^2
   uint64_t* bar = reinterpret_cast<uint64_t*>(nj + GA_CW);
   const int gp = g.list ? g.list[blockIdx.y] : blockIdx.y;
-  const int tile = blockIdx.x >> 1, half = blockIdx.x & 1;
+  const int tile = (blockIdx.x >> 1) + g.tile0, half = blockIdx.x & 1;
   int ti, tj;
   lower_tile(tile, ti, tj);
   const double* th = g.theta + (int64_t)gp * (d + 2);
@@ -616,7 +616,7 @@ int launch_assemble(const AssembleArgs& a, int count, cudaStream_t stream) {
     const int dpad = (a.d + 3) & ~3;
     const size_t zreg = std::max((size_t)dpad * (LDS_T + GA_LDJ), (size_t)GA_CW * GA_LDC);  // input tiles, later the cross-term tile
     const size_t smem = (zreg + 3 * (MAX_D + 2) + NB + GA_CW) * sizeof(double) + 16;
-    dim3 grid(a.J * (a.J + 1) / 2 * (NB / GA_CW), count);
+    dim3 grid((a.J * (a.J + 1) / 2 - a.tile0) * (NB / GA_CW), count);
     const bool three = 3 * (smem + 1024) <= 227 * 1024;  // three CTAs per SM fit (1 KB per CTA is reserved by the driver)
 #define GPRB_GA_CASE(K)                                                                  \
   if (three) {                                                                           \
@@ -635,7 +635,7 @@ int launch_assemble(const AssembleArgs& a, int count, cudaStream_t stream) {
 #undef GPRB_GA_CASE
   } else {
     const size_t smem = pw_smem(a.d, false);
-    dim3 grid(a.J * (a.J + 1) / 2, count);
+    dim3 grid(a.J * (a.J + 1) / 2 - a.tile0, count);
     switch (a.kind) {
       case GPRB_KERNEL_SE_ARD: rc = set_smem(k_assemble<0>, smem); if (!rc) k_assemble<0><<<grid, PW_THREADS, smem, stream>>>(a); break;
       case GPRB_KERNEL_MAT12_ARD: rc = set_smem(k_assemble<1>, smem); if (!rc) k_assemble<1><<<grid, PW_THREADS, smem, stream>>>(a); break;

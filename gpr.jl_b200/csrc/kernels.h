@@ -21,6 +21,8 @@ struct GemmArgs {
   int64_t mat_stride, dinv_stride;
   int npad, J, step, mode;
   int nv;               // n rounded up to 16: rows / k beyond it are padding that is neither computed nor read
+  int row0 = 0;         // GEMM_CHOL_COL: first block row of the launch, i = max(step + 1, row0) + blockIdx (gprb_batch_append
+                        // refactorises only the block rows its new samples reach)
   // GEMM_FWD_ROW only: the right-hand-side block T [B][npad][ldt] (row r of T contiguous over the test columns);
   // it is the B operand, the Cin source and the output at once (block row `step` is solved in place)
   double* Tm = nullptr;
@@ -52,6 +54,7 @@ struct AssembleArgs {
   const int32_t* list;
   int64_t mat_stride;
   int n, npad, d, J, kind;
+  int tile0 = 0;            // first lower tile (row-by-row order) of the launch: j0 (j0 + 1) / 2 assembles block rows >= j0 only
 };
 int launch_assemble(const AssembleArgs& a, int count, cudaStream_t stream);
 

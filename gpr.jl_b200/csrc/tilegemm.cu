@@ -28,7 +28,7 @@
 //
 // Modes (tile coordinates and k-range derive from `mode`, `step` and blockIdx.x):
 //   CHOL_DIAG  S(j,j)   = K(j,j) - sum_{k<j} L(j,k) L(j,k)^T                      -> Lm(j,j)   (potf2 follows)
-//   CHOL_COL   L(i,j)   = [K(i,j) - sum_{k<j} L(i,k) L(j,k)^T] * inv(L_jj)^T      -> Lm(i,j)   i > j = step
+//   CHOL_COL   L(i,j)   = [K(i,j) - sum_{k<j} L(i,k) L(j,k)^T] * inv(L_jj)^T      -> Lm(i,j)   i > j = step, i >= row0
 //   TRTRI_ROW  W(i,j)   = -inv(L_ii) * sum_{k=j}^{i-1} L(i,k) W(k,j)   stored as V(j,i) = W(i,j)^T, i = step
 //   LAUUM      Kinv(i,j) = sum_{k>=i} V(i,k) V(j,k)^T  (i >= j)  -> upper tile (j,i) of A (un-transposed) / KinvD(i)
 //   CHOL_PANEL L(i,j)   = S(i,j) * inv(L_jj)^T                       in place in Lm, i > j = step      } right-looking
@@ -88,7 +88,7 @@ __device__ __forceinline__ void lower_index(int bx, int& i, int& j) {
   j = bx - i * (i + 1) / 2;
 }
 
-__device__ __forceinline__ TileCoord tile_coord(int mode, int step, int J, int bx) {
+__device__ __forceinline__ TileCoord tile_coord(int mode, int step, int J, int row0, int bx) {
   TileCoord tc;
   tc.a_diag_kb = tc.b_diag_kb = -1;
   tc.post = 0;
@@ -97,7 +97,7 @@ __device__ __forceinline__ TileCoord tile_coord(int mode, int step, int J, int b
   if (mode == GEMM_CHOL_DIAG) {
     tc.i = tc.j = step; tc.kb0 = 0; tc.kb1 = step; tc.use_cin = true;
   } else if (mode == GEMM_CHOL_COL) {
-    tc.i = step + 1 + bx; tc.j = step; tc.kb0 = 0; tc.kb1 = step; tc.use_cin = true; tc.post = 1; tc.rblk = step;
+    tc.i = max(step + 1, row0) + bx; tc.j = step; tc.kb0 = 0; tc.kb1 = step; tc.use_cin = true; tc.post = 1; tc.rblk = step;
   } else if (mode == GEMM_TRTRI_ROW) {
     tc.i = step; tc.j = bx; tc.kb0 = bx; tc.kb1 = step; tc.b_diag_kb = bx; tc.post = 2; tc.rblk = step;
   } else if (mode == GEMM_CHOL_PANEL) {
@@ -475,10 +475,8 @@ __device__ __forceinline__ void tile_gemm_body(const GemmArgs& g) {
   uint64_t* empty = bars + NSTAGE;  // [NSTAGE]
   uint64_t* rfull = bars + 2 * NSTAGE;            // [NRBUF]
   uint64_t* rempty = bars + 2 * NSTAGE + NRBUF;   // [NRBUF]
-  constexpr int LDA = COLSPLIT ? LDS_T : LDS_H;  // padded rows of the A-operand chunk (the B chunk follows it in the stage)
 
   GPRB_TL(0);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int gp = g.list ? g.list[blockIdx.y] : g.gp_off + blockIdx.y;
   // A GP whose factorisation already hit a non-positive pivot (make_posdef! will retry it with more jitter) skips the
   // rest of the failed attempt, like dpotrf stopping at the failing column.  The load overlaps the setup below.
@@ -491,7 +489,7 @@ __device__ __forceinline__ void tile_gemm_body(const GemmArgs& g) {
     tc.i = g.step; tc.j = blockIdx.x; tc.kb0 = g.step + 1; tc.kb1 = g.J; tc.a_diag_kb = tc.b_diag_kb = -1;
     tc.use_cin = true; tc.post = 2; tc.rblk = g.step;
   } else {
-    tc = tile_coord(g.mode, g.step, g.J, fwd ? (int)blockIdx.x : (int)(blockIdx.x >> 1));
+    tc = tile_coord(g.mode, g.step, g.J, g.row0, fwd ? (int)blockIdx.x : (int)(blockIdx.x >> 1));
   }
   HalfGeom hg;
   hg.r0h = COLSPLIT ? 0 : half * HB;

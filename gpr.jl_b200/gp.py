@@ -515,6 +515,46 @@ class GPBatch:
             self.lib.check(self.lib.dll.gprb_batch_set_targets(self.handle, _d(ymm)))
             self.ymm = ymm
 
+    def append(self, trials_X_new, Y_new):
+        """``append!`` for every GP of the batch (gprb_batch_append): ``trials_X_new`` holds one d x k array per distinct
+        dataset in creation order (as for ``update_data``), ``Y_new`` (B, k) the raw targets of the new samples.  The batch
+        subtracts m(X_new) itself.  Every GP with a resident state is conditioned on its enlarged data at the theta of
+        that state, bit-identical to a fresh value-only evaluation there -> (mll (B,), info (B,)); GPs without a state
+        get NaN / 0 and stay without one."""
+        keys = list(self._ds)
+        if len(trials_X_new) != len(keys):
+            raise ValueError(f"expected {len(keys)} input blocks, got {len(trials_X_new)}")
+        blocks = [np.asarray(x, dtype=np.float64) for x in trials_X_new]
+        k = blocks[0].shape[1] if blocks[0].ndim == 2 else 0
+        for x in blocks:
+            if x.ndim != 2 or x.shape != (self.d, k):
+                raise ValueError(f"every input block must be d x k = {self.d} x {k}, got {x.shape}")
+        if k < 1:
+            raise ValueError("append needs at least one new sample")
+        Y_new = np.asarray(Y_new, dtype=np.float64).reshape(self.B, k)
+        trial = {key: t for t, key in enumerate(keys)}
+        gp_blocks = [blocks[trial[id(g.x)]] for g in self.gps]
+        ymm_new = as_f64(Y_new - np.stack(self._means(gp_blocks)))
+        keep = [as_f64(x.T) for x in blocks]  # k x d C-order = d x k column-major
+        parr = (C.POINTER(C.c_double) * len(keep))(*[_d(x) for x in keep])
+        mll = np.full(self.B, np.nan)
+        info = np.zeros(self.B, dtype=np.int32)
+        self.lib.check(self.lib.dll.gprb_batch_append(self.handle, k, parr, self.d, _d(ymm_new), _d(mll),
+                                                      info.ctypes.data_as(C.POINTER(C.c_int32))))
+        # one new x per trial, still shared by the trial's GPs (the dataset key is the array's identity)
+        grown = {key: np.concatenate([self._keep[t], blocks[t]], axis=1) for t, key in enumerate(keys)}
+        for b, g in enumerate(self.gps):
+            g.x = grown[id(g.x)]
+            g.y = np.concatenate([g.y, Y_new[b]])
+            g.nobs += k
+        self._ds = {id(grown[key]): self._ds[key] for key in keys}
+        self._keep = [grown[key] for key in keys]
+        self.n += k
+        self.ymm = np.concatenate([self.ymm, ymm_new], axis=1)
+        sel = ~np.isnan(mll)
+        self._mll[sel], self._info[sel], self._has_grad[sel] = mll[sel], info[sel], False
+        return mll, info
+
     def set_diag_offset(self, offset=None):
         """gprb_batch_set_diag_offset: fixed per-GP nugget added to the diagonal of K (None resets it)."""
         off = None if offset is None else as_f64(np.broadcast_to(np.asarray(offset, dtype=np.float64), (self.B,)).copy())
@@ -755,6 +795,20 @@ def optimize(gp, method: LBFGS | None = None, options: Options | None = None):
 
 
 optimize_b = optimize  # ``optimize!`` (the bang is not a Python identifier character)
+
+
+def append(gp, x, y):
+    """``append!(gp, x, y)`` (ElasticGPE): add the samples x (d x k) with targets y (k,) to one GPE and condition it on
+    them at its current parameters.  A GP that shares its batch moves to a batch of its own first (like ``optimize``).
+    For a GPBatch, x is the list of per-dataset blocks and y (B, k), see ``GPBatch.append``.  Returns ``gp``."""
+    if isinstance(gp, GPBatch):
+        gp.append(x, y)
+        return gp
+    if gp._batch is None or gp._batch.B != 1:
+        GPBatch([gp]).update_mll()
+    x = np.asarray(x, dtype=np.float64)
+    gp._batch.append([x.reshape(gp.dim, -1)], np.asarray(y, dtype=np.float64).reshape(1, -1))
+    return gp
 
 
 def predict_y(gp, Xstar, var=True):

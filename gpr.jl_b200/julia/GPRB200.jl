@@ -502,6 +502,63 @@ function predict_grad(gp::B200GPE, x::AbstractMatrix; var::Bool = true, mean_jac
     μ[:, slot], var ? σ2[:, slot] : nothing, ∂μ[:, :, slot], var ? ∂σ2[:, :, slot] : nothing
 end
 
+# ---- append! (ElasticGPE): new samples on resident GPs, only the block rows they reach refactorised ---------------------
+# Base.append! is extended, nothing is exported.  The other GPs of the batch read the same device datasets, so a GPE that
+# shares its batch moves to a batch of its own first (like optimize!).
+"""
+    append!(batch::GPBatch, xs::Vector{<:AbstractMatrix}, ys::AbstractMatrix) -> (mll::Vector{Float64}, info::Vector{Int32})
+
+`xs`: one d × k block per distinct training set of the batch, in order of first use by GP index; `ys`: k × B raw targets
+(m(x) is subtracted here).  Every GP with a resident state is conditioned on its enlarged data at the θ of that state;
+GPs without a state get NaN and stay without one.
+"""
+function Base.append!(batch::GPBatch, xs::AbstractVector{<:AbstractMatrix}, ys::AbstractMatrix)
+    uniq = IdDict{Any,Int}()
+    for gp in batch.gps
+        get!(uniq, gp.x, length(uniq) + 1)
+    end
+    length(xs) == length(uniq) || throw(ArgumentError("append!: expected $(length(uniq)) input blocks, got $(length(xs))"))
+    d, k = batch.d, size(xs[1], 2)
+    all(x -> size(x) == (d, k), xs) || throw(DimensionMismatch("append!: every input block must be $d × $k"))
+    size(ys) == (k, batch.B) || throw(DimensionMismatch("append!: ys must be $k × $(batch.B)"))
+    blocks = [Matrix{Float64}(x) for x in xs]
+    ymm = Matrix{Float64}(undef, k, batch.B)
+    for (x, t) in uniq
+        members = [b for b in 1:batch.B if batch.gps[b].x === x]
+        for j in 1:k, b in members
+            ymm[j, b] = ys[j, b] - GaussianProcesses.mean(batch.gps[b].mean, blocks[t][:, j])
+        end
+    end
+    mll = fill(NaN, batch.B)
+    info = zeros(Int32, batch.B)
+    ptrs = [pointer(x) for x in blocks]
+    GC.@preserve blocks ymm mll info begin
+        check(ccall((:gprb_batch_append, LIB), Cint, (Ptr{Cvoid}, Int64, Ptr{Ptr{Float64}}, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}),
+                    batch.handle, k, ptrs, d, ymm, mll, info))
+    end
+    grown = IdDict{Any,Matrix{Float64}}(x => hcat(x, blocks[t]) for (x, t) in uniq)
+    for (b, gp) in enumerate(batch.gps)
+        gp.x = grown[gp.x]
+        gp.y = vcat(gp.y, ys[:, b])
+        gp.nobs += k
+        isnan(mll[b]) || (gp.mll = mll[b]; gp.target = mll[b])
+    end
+    batch.n += k
+    batch.cache_key = zeros(0, 0)
+    mll, info
+end
+
+"`append!(gp, x::d×k, y::k)`: ElasticGPE's append! on a B200-resident GPE; the GP ends evaluated at its current parameters."
+function Base.append!(gp::B200GPE, x::AbstractMatrix, y::AbstractVector)
+    batch, _ = residence(gp)
+    if batch.B != 1
+        batch = GPBatch(GPE[gp])
+        evaluate!(batch; grad = false)
+    end
+    append!(batch, [x], reshape(Vector{Float64}(y), :, 1))
+    gp
+end
+
 # ---- asynchronous rollout step (two trial groups alternate: device predict of one under the host projectv! of the other) -----
 "Enqueue the mean prediction of GPs gp0:gp1 (1-based, inclusive) at the per-trial state blocks `states` (d × m × trials) on pipeline `slot`."
 function predict_async!(batch::GPBatch, slot::Integer, gp0::Integer, gp1::Integer, states::Array{Float64,3}, G::Integer; var::Bool = false)

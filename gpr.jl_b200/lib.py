@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 EXPORTS = [
     "gprb_version", "gprb_last_error", "gprb_init", "gprb_init_multi", "gprb_destroy", "gprb_device_info",
     "gprb_dataset_create", "gprb_datasets_create", "gprb_dataset_update", "gprb_datasets_update", "gprb_dataset_destroy",
-    "gprb_batch_create", "gprb_batch_set_targets", "gprb_batch_set_diag_offset", "gprb_batch_destroy",
+    "gprb_batch_create", "gprb_batch_set_targets", "gprb_batch_set_diag_offset", "gprb_batch_destroy", "gprb_batch_append",
     "gprb_eval", "gprb_eval_mixed", "gprb_eval_device", "gprb_lbfgs_default_opts", "gprb_optimize", "gprb_lbfgs_selftest",
     "gprb_predict", "gprb_predict_async", "gprb_predict_wait", "gprb_last_predict_ms",
     "gprb_predict_cov", "gprb_sample_posterior", "gprb_eval_loo", "gprb_predict_grad",
@@ -78,6 +78,7 @@ class Library:
         L.gprb_batch_set_targets.argtypes = [_vp, _dp]
         L.gprb_batch_set_diag_offset.argtypes = [_vp, _dp]
         L.gprb_batch_destroy.argtypes = [_vp]
+        L.gprb_batch_append.argtypes = [_vp, C.c_int64, C.POINTER(_dp), C.c_int64, _dp, _dp, C.POINTER(C.c_int32)]
         L.gprb_eval.argtypes = [_vp, _dp, C.POINTER(C.c_uint8), _dp, _dp, C.POINTER(C.c_int32)]
         L.gprb_eval_mixed.argtypes = [_vp, _dp, C.POINTER(C.c_uint8), _dp, _dp, C.POINTER(C.c_int32)]
         L.gprb_eval_device.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp]

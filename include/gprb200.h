@@ -17,6 +17,7 @@
  *       -> gprb_predict_cov, gprb_sample_posterior
  *   predict_LOO(gp), logp_CVLOO(gp), dlogpdtheta_CVLOO(gp)   (GaussianProcesses 0.12 crossvalidation.jl)
  *       -> gprb_eval_loo
+ *   append!(gp, x, y)  (ElasticGPE, GaussianProcesses 0.12 GP.jl)   -> gprb_batch_append
  *   gp.cK / gp.alpha inspection (parity taps)              -> gprb_get_K / _chol / _alpha / _Kinv
  *
  * Conventions
@@ -102,6 +103,22 @@ int gprb_batch_set_targets(gprb_batch* batch, const double* ymm); /* n x B */
  * positive-semidefinite kernels never produce by rounding alone. */
 int gprb_batch_set_diag_offset(gprb_batch* batch, const double* offset /* B or NULL */);
 int gprb_batch_destroy(gprb_batch* batch);
+/* Append k samples to every dataset of the batch and condition every GP that has a resident state on them, at the theta
+ * of that state (GaussianProcesses ElasticGPE append!).
+ *   Xnew     one d x k block per distinct dataset of the batch, in order of first use by GP index, leading dimension ldx
+ *   ymm_new  k x B    y - m(Xnew) per GP (the prior mean stays on the host, as everywhere)
+ *   mll      B  out   (NULL allowed)
+ *   info     B  out   (NULL allowed)
+ * GPs without a resident state have their data grown, but their outputs are not written and they stay without a state.
+ * Afterwards every GP that had a state is in the state gprb_eval(theta, grad = NULL) leaves on the enlarged data, bit for
+ * bit (same info, mll, K, factor, alpha and predictions).  A state factorised without jitter keeps the block rows
+ * < floor(n / 128) of its factor and refactorises only the rest; a state that carried jitter (1e-6 tr(K)/n depends on n),
+ * one with n < 128, and one whose new diagonal blocks fail a pivot get an ordinary value-only evaluation with the
+ * make_posdef! ladder.  A following gprb_eval at the same theta with a gradient runs only the inverse and the gradient.
+ * Refused with GPRB_ERR_ARG, the batch unchanged: k < 1, a NULL pointer, a prediction in flight on either slot, a dataset
+ * that another live batch also uses.  GPRB_ERR_NOMEM leaves the batch unchanged as well. */
+int gprb_batch_append(gprb_batch* batch, int64_t k, const double* const* Xnew, int64_t ldx, const double* ymm_new,
+                      double* mll, int32_t* info);
 
 /* One objective evaluation per active GP (rows a5-a9 of SURVEY.md section 8a).
  *   theta  P x B    in
