@@ -517,6 +517,12 @@ static int download_results(gprb_batch* b, const uint8_t* mode, const std::vecto
   return 0;
 }
 
+int refuse_while_predicting(const gprb_batch* b, const char* fn) {
+  GPRB_REQUIRE(!b->ps[0].pending && !b->ps[1].pending,
+               std::string(fn) + ": a prediction is in flight - call gprb_predict_wait first");
+  return 0;
+}
+
 int eval_pass_host(gprb_batch* b, const double* theta, const uint8_t* mode, const uint8_t* retry, double* mll, double* grad,
                    int32_t* info_out, uint8_t* pending_out) {
   GPRB_REQUIRE(b && theta && mode && mll && grad && info_out && pending_out, "eval_pass_host: NULL argument");
@@ -656,6 +662,8 @@ int gprb_dataset_create(gprb_ctx* ctx, int64_t n, int32_t d, const double* X, in
 int gprb_dataset_update(gprb_dataset* ds, const double* X, int64_t ldx) {
   GPRB_REQUIRE(ds && X, "gprb_dataset_update: NULL argument");
   GPRB_REQUIRE(ldx >= ds->d, "gprb_dataset_update: ldx < d");
+  GPRB_REQUIRE(ds->predicting == 0,
+               "gprb_dataset_update: a prediction that reads the dataset is in flight - call gprb_predict_wait first");
   return dataset_upload(ds, X, ldx);
 }
 
@@ -729,6 +737,8 @@ int gprb_datasets_update(gprb_ctx* ctx, int32_t count, gprb_dataset* const* ds, 
     GPRB_REQUIRE(ds[i] && X[i], "gprb_datasets_update: NULL dataset or matrix");
     GPRB_REQUIRE(ds[i]->ctx == ctx, "gprb_datasets_update: dataset belongs to another context");
     GPRB_REQUIRE(ldx >= ds[i]->d, "gprb_datasets_update: ldx < d");
+    GPRB_REQUIRE(ds[i]->predicting == 0,
+                 "gprb_datasets_update: a prediction that reads one of the datasets is in flight - call gprb_predict_wait first");
   }
   GPRB_CUDA(cudaSetDevice(ctx->device));
   if (slab_contiguous(count, ds, X, ldx)) return slab_upload(ctx, count, ds, X[0]);
@@ -869,12 +879,14 @@ int gprb_batch_create(gprb_ctx* ctx, int32_t B, gprb_dataset* const* ds, const d
 
 int gprb_batch_set_targets(gprb_batch* b, const double* ymm) {
   GPRB_REQUIRE(b && ymm, "gprb_batch_set_targets: NULL argument");
+  if (int rc = refuse_while_predicting(b, "gprb_batch_set_targets")) return rc;
   GPRB_CUDA(cudaSetDevice(b->ctx->device));
   return upload_targets(b, ymm);
 }
 
 int gprb_batch_set_diag_offset(gprb_batch* b, const double* offset) {
   GPRB_REQUIRE(b, "gprb_batch_set_diag_offset: NULL batch");
+  if (int rc = refuse_while_predicting(b, "gprb_batch_set_diag_offset")) return rc;
   GPRB_CUDA(cudaSetDevice(b->ctx->device));
   if (offset) {
     for (int i = 0; i < b->B; ++i) GPRB_REQUIRE(isfinite(offset[i]), "gprb_batch_set_diag_offset: non-finite offset");
@@ -893,6 +905,8 @@ int gprb_batch_destroy(gprb_batch* b) {
     cudaSetDevice(b->ctx->device);
     cudaDeviceSynchronize();
     for (gprb_dataset* u : distinct_datasets(b)) u->users--;
+    for (gprb_predict_slot& sl : b->ps)  // a prediction never waited for no longer reads its datasets
+      for (gprb_dataset* u : sl.reads) u->predicting--;
   }
   free_batch(b);
   return GPRB_OK;
@@ -920,6 +934,7 @@ int gprb_last_stage_ms(gprb_batch* b, double out[8]) {
 // ------------------------------------------------------------------------------------------------
 int gprb_eval_mixed(gprb_batch* b, const double* theta, const uint8_t* mode, double* mll, double* grad, int32_t* info) {
   GPRB_REQUIRE(b && theta && mode && mll && info, "gprb_eval_mixed: NULL argument");
+  if (int rc = refuse_while_predicting(b, "gprb_eval_mixed")) return rc;
   GPRB_CUDA(cudaSetDevice(b->ctx->device));
   bool any_grad = false;
   std::vector<int32_t> act;
@@ -938,6 +953,7 @@ int gprb_eval_mixed(gprb_batch* b, const double* theta, const uint8_t* mode, dou
 
 int gprb_eval(gprb_batch* b, const double* theta, const uint8_t* active, double* mll, double* grad, int32_t* info) {
   GPRB_REQUIRE(b && theta && mll && info, "gprb_eval: NULL argument");
+  if (int rc = refuse_while_predicting(b, "gprb_eval")) return rc;
   std::vector<uint8_t> mode(b->B);
   for (int i = 0; i < b->B; ++i) mode[i] = (!active || active[i]) ? (grad ? 2 : 1) : 0;
   return gprb_eval_mixed(b, theta, mode.data(), mll, grad, info);
@@ -946,6 +962,7 @@ int gprb_eval(gprb_batch* b, const double* theta, const uint8_t* active, double*
 int gprb_eval_device(gprb_batch* b, const double* theta_dev, double* mll_dev, double* grad_dev, int32_t* info_dev,
                      void* stream) {
   GPRB_REQUIRE(b && theta_dev && mll_dev, "gprb_eval_device: NULL argument");
+  if (int rc = refuse_while_predicting(b, "gprb_eval_device")) return rc;
   GPRB_CUDA(cudaSetDevice(b->ctx->device));
   cudaStream_t user = (cudaStream_t)stream;
   const int B = b->B, P = b->P;
@@ -1170,6 +1187,10 @@ static int predict_enqueue(gprb_batch* b, int slot, int gp0, int gp1, int64_t m,
   if (want_var) GPRB_CUDA(cudaMemcpyAsync(sl.h_out + nout, sl.pvar, sizeof(double) * nout, cudaMemcpyDeviceToHost, st));
   GPRB_CUDA(cudaEventRecord(sl.t1, st));
   sl.pending = true; sl.gp0 = gp0; sl.gp1 = gp1; sl.m = m; sl.want_var = want_var;
+  sl.reads.clear();
+  std::unordered_set<gprb_dataset*> seen;
+  for (int i = gp0; i < gp1; ++i)
+    if (seen.insert(b->ds[i]).second) { sl.reads.push_back(b->ds[i]); b->ds[i]->predicting++; }
   return 0;
 }
 
@@ -1178,6 +1199,8 @@ static int predict_collect(gprb_batch* b, int slot, double* mu, double* var) {
   int rc = slot_wait(sl);
   if (rc) return rc;
   sl.pending = false;
+  for (gprb_dataset* u : sl.reads) u->predicting--;
+  sl.reads.clear();
   const size_t nout = (size_t)(sl.gp1 - sl.gp0) * sl.m;
   memcpy(mu, sl.h_out, sizeof(double) * nout);
   if (var && sl.want_var) memcpy(var, sl.h_out + nout, sizeof(double) * nout);
@@ -1600,6 +1623,7 @@ extern "C" {
 int gprb_eval_loo(gprb_batch* b, const double* theta, const uint8_t* active, double* mll, double* grad, double* logp_loo,
                   double* grad_loo, double* mu_loo, double* var_loo, int32_t* info) {
   GPRB_REQUIRE(b && theta && logp_loo && info, "gprb_eval_loo: NULL argument");
+  if (int rc = refuse_while_predicting(b, "gprb_eval_loo")) return rc;
   GPRB_CUDA(cudaSetDevice(b->ctx->device));
   const int B = b->B;
   // the evaluation of gprb_eval with a gradient (the LOO terms need K^-1), with its state reuse
@@ -1772,8 +1796,7 @@ int gprb_batch_append(gprb_batch* b, int64_t k, const double* const* Xnew, int64
   GPRB_REQUIRE(k >= 1, "gprb_batch_append: k must be >= 1");
   GPRB_REQUIRE(ldx >= b->d, "gprb_batch_append: ldx < d");
   GPRB_REQUIRE(b->n + k <= (1 << 20), "gprb_batch_append: n + k out of range");
-  GPRB_REQUIRE(!b->ps[0].pending && !b->ps[1].pending,
-               "gprb_batch_append: a prediction is in flight - call gprb_predict_wait first");
+  if (int rc = refuse_while_predicting(b, "gprb_batch_append")) return rc;
   const std::vector<gprb_dataset*> uds = distinct_datasets(b);
   const int T = (int)uds.size();
   for (int t = 0; t < T; ++t) {

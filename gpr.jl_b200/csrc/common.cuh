@@ -52,6 +52,11 @@ int make_tensor_map(CUtensorMap* map, const double* base, uint64_t rows, uint64_
 int eval_pass_host(gprb_batch* b, const double* theta, const uint8_t* mode, const uint8_t* retry, double* mll, double* grad,
                    int32_t* info, uint8_t* pending);
 
+// GPRB_ERR_ARG with "<fn>: a prediction is in flight - call gprb_predict_wait first" while either prediction slot of b
+// is pending, 0 otherwise: the calls that write a batch's resident state (theta, K, factor, alpha, targets, offsets)
+// refuse then, because the slots' streams are not ordered with the evaluation streams.
+int refuse_while_predicting(const gprb_batch* b, const char* fn);
+
 }  // namespace gprb
 
 struct gprb_ctx;
@@ -95,6 +100,7 @@ struct gprb_dataset {
   gprb_slab* slab = nullptr;  // non-null: X / Xt point into the slab (member `slab_index`)
   int32_t slab_index = 0;
   int32_t users = 0;     // live batches that use the dataset (gprb_batch_append grows only a dataset no other batch reads)
+  int32_t predicting = 0;  // predictions in flight (gprb_predict_async, not yet waited for) that read X / Xt: uploads refuse
 };
 
 // One prediction pipeline of a batch (gprb_predict_async slot): own streams, staging and scratch, so that two groups
@@ -112,6 +118,7 @@ struct gprb_predict_slot {
   size_t h_in_cap = 0, h_out_cap = 0;
   cudaEvent_t t0 = nullptr, t1 = nullptr;           // device time of the last prediction
   bool pending = false;
+  std::vector<gprb_dataset*> reads;  // distinct datasets of GPs gp0 .. gp1-1 while pending (their `predicting` is raised)
   int gp0 = 0, gp1 = 0;
   int64_t m = 0;
   bool want_var = false;

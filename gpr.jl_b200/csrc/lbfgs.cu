@@ -312,6 +312,7 @@ void gprb_lbfgs_default_opts(gprb_lbfgs_opts* o) {
 
 int gprb_optimize(gprb_batch* b, double* theta_inout, const gprb_lbfgs_opts* opts, gprb_opt_result* results) {
   GPRB_REQUIRE(b && theta_inout && results, "gprb_optimize: NULL argument");
+  if (int rc = refuse_while_predicting(b, "gprb_optimize")) return rc;
   gprb_lbfgs_opts o;
   if (opts) o = *opts; else gprb_lbfgs_default_opts(&o);
   const int B = b->B, P = b->P;

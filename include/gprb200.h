@@ -202,7 +202,13 @@ int gprb_predict(gprb_batch* batch, int64_t m, const double* Xstar, int64_t xsta
  * Xstar + (k / gps_per_block)*xstar_stride - gps_per_block consecutive GPs (the G outputs of a trial, which all predict
  * from the trial's own states) share one block, so a step uploads each trial's states once, not G times - and the prior
  * means mstar + k*m.  Both are copied to pinned staging before the call returns, so the caller may overwrite them.  gprb_predict_wait blocks until
- * the slot's prediction is complete and writes mu / var ((gp1-gp0) x m each; var may be NULL when want_var was 0). */
+ * the slot's prediction is complete and writes mu / var ((gp1-gp0) x m each; var may be NULL when want_var was 0).
+ * While a prediction is in flight it reads the batch's resident state and the datasets of its GPs on the slot's own
+ * streams, which nothing orders with evaluations or uploads.  So until gprb_predict_wait, the calls that write that state
+ * are refused with GPRB_ERR_ARG and leave everything unchanged: gprb_eval, gprb_eval_mixed, gprb_eval_device,
+ * gprb_eval_loo, gprb_optimize, gprb_batch_set_targets, gprb_batch_set_diag_offset and gprb_batch_append while either
+ * slot of the batch is pending, and gprb_dataset_update / gprb_datasets_update of a dataset that a pending prediction
+ * of any batch reads. */
 int gprb_predict_async(gprb_batch* batch, int32_t slot, int32_t gp0, int32_t gp1, int64_t m, const double* Xstar,
                        int64_t xstar_stride, int32_t gps_per_block, const double* mstar, int32_t want_var);
 int gprb_predict_wait(gprb_batch* batch, int32_t slot, double* mu, double* var);
