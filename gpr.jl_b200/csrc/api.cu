@@ -99,12 +99,19 @@ static bool posdef_retry(int32_t f, int32_t& tries, int32_t& info) {
   return false;
 }
 
+// GPRB200_POISON_ALLOC=1 (a test knob) fills every floating-point allocation with 0xFF bytes, a quiet NaN in fp64, so that a
+// stage that reads memory nothing wrote turns results into NaN instead of silently multiplying fresh zero pages.  Integer and
+// pointer buffers (lists, fail flags, masks, counters, dataset pointers) are left alone: an index read before it is
+// written must not become an out-of-bounds address.
 template <typename T>
 static int dev_alloc(T** p, size_t count) {
+  static const bool poison = [] { const char* e = getenv("GPRB200_POISON_ALLOC"); return e && e[0] == '1'; }();
   *p = nullptr;
   if (count == 0) count = 1;
   cudaError_t e = cudaMalloc((void**)p, count * sizeof(T));
   if (e != cudaSuccess) return cuda_fail(e, "cudaMalloc", __FILE__, __LINE__);
+  if (std::is_floating_point<T>::value && poison && (e = cudaMemset(*p, 0xFF, count * sizeof(T))) != cudaSuccess)
+    return cuda_fail(e, "cudaMemset(poison)", __FILE__, __LINE__);
   return 0;
 }
 

@@ -6,43 +6,74 @@ diagonal blocks) independently of the GPU."""
 import numpy as np
 
 
-def blocked_pipeline(K, nb):
-    n = K.shape[0]
-    J = n // nb
-    blk = lambda M, i, j: M[i * nb:(i + 1) * nb, j * nb:(j + 1) * nb]
-    Lm = np.zeros_like(K)
+def blocked_pipeline(K, nb, nv=None, kt=16, mutation=None):
+    """K (npad x npad, npad = J nb) -> (L, Kinv, Dinv).  Rows / columns at or beyond ``nv`` (n rounded up to kt, default
+    npad) are padding, handled as the kernels handle it: no stage reads or writes them (fill them with NaN to check),
+    the valid rows of the last block row are nvl = nv - (J - 1) nb, the k-range of k-block J - 1 stops at its last valid
+    kt-chunk, and the diagonal factor of the last block treats its rows >= nvl as the identity.  The padding of L and
+    Kinv comes back as NaN (never written).
+
+    ``mutation`` emulates one plausible error of the ragged paths (tests/test_ragged_reference.py):
+      "lauum_chunk"  LAUUM drops the last valid kt-chunk of k-block J - 1 (nchunks off by one)
+      "slab_col"     the last valid 8-row slab of each CHOL_COL tile of the last block row keeps its parked input T
+                     (mi_valid off by one: the post-multiply by inv(L_jj)^T skips it)
+      "slab_trtri"   the same for the TRTRI_ROW tiles of the last block row (the left-multiply by -inv(L_ii) skips it)
+      "half_skip"    ROWSPLIT tiles (CHOL_COL, LAUUM) of the last block row skip their second half at nvl = 80 (the early
+                     exit one chunk too soon): rows 64 .. 79 stay at zero
+      "col_krange"   the CHOL_COL tiles of the last block row sum over k < j - 1 (the previous step's k-range)"""
+    npad = K.shape[0]
+    J = npad // nb
+    nv = npad if nv is None else nv
+    nvl = nv - (J - 1) * nb
+    rv = lambda i: nvl if i == J - 1 else nb  # valid rows / columns of block i
+    blk = lambda M, i, j: M[i * nb:i * nb + rv(i), j * nb:j * nb + rv(j)]
+    Lm = np.full_like(K, np.nan)
     Dinv = [None] * J
+    last = J - 1
     # --- Cholesky: CHOL_DIAG -> diag_factor -> CHOL_COL
     for j in range(J):
         S = blk(K, j, j).copy()
         for k in range(j):
             S -= blk(Lm, j, k) @ blk(Lm, j, k).T
         Ljj = np.linalg.cholesky(S)
-        blk(Lm, j, j)[:] = Ljj
+        blk(Lm, j, j)[:] = np.tril(Ljj)
         Dinv[j] = np.linalg.inv(Ljj)
         for i in range(j + 1, J):
+            kb1 = j - 1 if (mutation == "col_krange" and i == last) else j
             T = blk(K, i, j).copy()
-            for k in range(j):
+            for k in range(max(kb1, 0)):
                 T -= blk(Lm, i, k) @ blk(Lm, j, k).T
-            blk(Lm, i, j)[:] = T @ Dinv[j].T
-    L = np.tril(Lm).copy()
+            out = T @ Dinv[j].T
+            if i == last and mutation == "slab_col" and nvl < nb:
+                out[nvl - 8:] = T[nvl - 8:]
+            if i == last and mutation == "half_skip" and nvl == 80:
+                out[64:] = 0.0
+            blk(Lm, i, j)[:] = out
+    L = np.tril(Lm)
     # --- TRTRI_ROW: W(i,j) = -Dinv_i * sum_{k=j}^{i-1} L(i,k) W(k,j), stored as V(j,i) = W(i,j)^T (upper tiles of Lm)
     for i in range(1, J):
         for j in range(i):
-            T = np.zeros((nb, nb))
+            T = np.zeros((rv(i), nb))
             for k in range(j, i):
                 Vjk = Dinv[j].T if k == j else blk(Lm, j, k)  # B operand: V(j,k), diagonal block from DinvT
                 T += blk(Lm, i, k) @ Vjk.T
-            blk(Lm, j, i)[:] = (-(Dinv[i] @ T)).T
+            W = -(Dinv[i] @ T)
+            if i == last and mutation == "slab_trtri" and nvl < nb:
+                W[nvl - 8:] = T[nvl - 8:]
+            blk(Lm, j, i)[:] = W.T
     # --- LAUUM: Kinv(i,j) = sum_{k>=i} V(i,k) V(j,k)^T
-    Kinv = np.zeros_like(K)
+    Kinv = np.full_like(K, np.nan)
     for i in range(J):
         for j in range(i + 1):
-            acc = np.zeros((nb, nb))
+            acc = np.zeros((rv(i), rv(j)))
             for k in range(i, J):
                 Vik = Dinv[i].T if k == i else blk(Lm, i, k)
                 Vjk = Dinv[j].T if k == j else blk(Lm, j, k)
+                if k == last and mutation == "lauum_chunk":
+                    Vik, Vjk = Vik[:, :nvl - kt], Vjk[:, :nvl - kt]
                 acc += Vik @ Vjk.T
+            if i == last and mutation == "half_skip" and nvl == 80:
+                acc[64:] = 0.0
             blk(Kinv, i, j)[:] = acc
             blk(Kinv, j, i)[:] = acc.T
     return L, Kinv, Dinv

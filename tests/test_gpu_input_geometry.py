@@ -48,6 +48,7 @@ import pytest
 
 import gpr_jl_b200  # noqa: F401
 from oracle import gp_oracle as go
+from oracle.ld_oracle import k_reference  # noqa: F401  (also read by tests/test_geometry_reference.py)
 from oracle import loo_oracle as lo
 from oracle import postcov_oracle as pco
 from oracle import predgrad_oracle as pgo
@@ -175,37 +176,6 @@ def make_rollout(n, seed, m=12, traj_len=50):
 # ------------------------------------------------------------------------------------------------------------------
 # high-precision reference
 # ------------------------------------------------------------------------------------------------------------------
-def _kfun_ld(r2, sf2, kind):
-    ld = np.longdouble
-    r = np.sqrt(r2)
-    if kind == "se":
-        return sf2 * np.exp(-r2 / 2)
-    if kind == "mat12":
-        return sf2 * np.exp(-r)
-    if kind == "mat32":
-        s = np.sqrt(ld(3)) * r
-        return sf2 * (1 + s) * np.exp(-s)
-    s = np.sqrt(ld(5)) * r
-    return sf2 * (1 + s + 5 * r2 / 3) * np.exp(-s)
-
-
-def k_reference(X, theta, kind, with_r2=False):
-    """K = K_f + (exp(2 logNoise) + eps) I in numpy.longdouble by direct differences of the raw inputs; w_p, s_f^2 and
-    the noise are the float64 values both implementations start from.  X (d, n).  with_r2: -> (K, r2)."""
-    ld = np.longdouble
-    d, n = X.shape
-    w = np.exp(-2.0 * np.asarray(theta[1:-1], dtype=np.float64)).astype(ld)
-    sf2 = ld(math.exp(2.0 * theta[-1]))
-    r2 = np.zeros((n, n), dtype=ld)
-    for p in range(d):
-        x = X[p].astype(ld)
-        df = x[:, None] - x[None, :]
-        r2 += w[p] * df * df
-    K = _kfun_ld(r2, sf2, kind)
-    K[np.diag_indices(n)] = sf2 + (ld(math.exp(2.0 * theta[0])) + ld(EPS))
-    return (K, r2) if with_r2 else K
-
-
 def k_pairs_mpmath(X, theta, kind, pairs, dps=40):
     """K_f(x_i, x_j) at the given pairs in mpmath (dps digits)."""
     import mpmath as mp
